@@ -26,6 +26,11 @@ One JSON line on rank 0.  What is measured (definitions in DESIGN.md, "Measureme
   kernel time / HBM fraction, train steps/s and the CPU training-loop baseline beside it.
 
 ``--impl reference`` runs only the CPU formulation of the loss (rank 0, no GPU, no native library), K timed steps.
+
+``--dump-outputs DIR`` writes, after the timed steps, what the last timed step returned as ``DIR/<name>.npy`` (f32 / f64
+as computed): ``loss_moments`` and ``loss_grad`` of the loss step, and ``train_total`` / ``train_moments`` of the last
+training step when that leg runs (reference arm: ``loss`` and ``loss_grad``).  The inputs are pure functions of fixed
+seeds, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -93,7 +98,22 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-sample-pairs", type=float, default=1e8, help="ordered pairs per CPU-baseline loss step")
     ap.add_argument("--cpu-train-budget", type=float, default=1.0, help="scale of the CPU training-loop baseline's work (1 = default samples)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    """``DIR/<name>.npy`` for every (host) array, in the f32 / f64 it was computed in."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(path, f"{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------ clocks
@@ -194,7 +214,8 @@ def cpu_sample_step(coords, truth_rows, sample_rows):
     return float(l.detach())
 
 
-def time_cpu_sample(n, truth_rows_f64, sample_rows, warmup, steps):
+def time_cpu_sample(n, truth_rows_f64, sample_rows, warmup, steps, outputs=None):
+    """``outputs``: a dict that receives the loss and the coordinate gradient of the last timed step."""
     import torch
 
     torch.set_num_threads(os.cpu_count() or 1)
@@ -205,8 +226,10 @@ def time_cpu_sample(n, truth_rows_f64, sample_rows, warmup, steps):
         cpu_sample_step(coords, truth, sample_rows)
     t0 = time.perf_counter()
     for _ in range(steps):
-        cpu_sample_step(coords, truth, sample_rows)
+        loss = cpu_sample_step(coords, truth, sample_rows)
     dt = time.perf_counter() - t0
+    if outputs is not None:
+        outputs.update(loss=torch.tensor([loss], dtype=torch.float64), loss_grad=coords.grad.clone())
     return sample_rows * n * steps / dt / 1e9, dt / steps, torch.get_num_threads()
 
 
@@ -251,7 +274,10 @@ def run_reference(args):
     n = w["n"]
     sample_rows = sample_rows_for(n, args.cpu_sample_pairs)
     truth = cpu_truth_rows(args.workload, sample_rows)
-    gps, sec_per_step, threads = time_cpu_sample(n, truth, sample_rows, max(args.warmup, 1), args.steps)
+    outputs = {}
+    gps, sec_per_step, threads = time_cpu_sample(n, truth, sample_rows, max(args.warmup, 1), args.steps, outputs)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     sample = f"oracle torch.cdist+MSELoss+autograd on rows [0,{sample_rows}) x {n} cols ({sample_rows * n:.3g} ordered pairs) per step"
     line = {
         "impl": "reference", "metric": METRIC, "value": gps, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -708,6 +734,8 @@ def measure_workload(env: Env, name: str, primary: bool):
         stalled = max_over_ranks(1.0 if elapsed_ms / K > 1.25 * kern_ms + 0.1 else 0.0) > 0
         if not stalled or attempts == 2:
             break
+    # copied now: the legs below run the same loss function into the same device buffers
+    outputs = {"loss_moments": moments.cpu(), "loss_grad": grad.reshape(n, 3).cpu()} if primary and args.dump_outputs else None
     value = float(n) * float(n) * K / (elapsed_ms * 1e-3) / 1e9
     mse = float(moments[0]) / (float(n) * float(n))
     env.windows[f"loss_{name}" if not primary else "loss"] = (w0, w1)
@@ -722,7 +750,7 @@ def measure_workload(env: Env, name: str, primary: bool):
     res = {"name": name, "n": n, "K": K, "W": W, "value": value, "ms_per_step": elapsed_ms / K, "kernel_ms": kern_ms, "exchange_ms": exch_ms, "launches": int(launches),
            "attempts": attempts, "kernel_samples": len(sampled), "mse": mse, "nloc": nloc, "target_bytes": target_bytes, "transport": transport, "setup_s": round(t_setup, 1),
            "achieved": achieved, "peak": peak, "peak_src": peak_src, "loss_mode": loss_mode, "upper": upper, "alg_bytes": alg_bytes, "streamed_bytes": streamed,
-           "rows": [r0, r1], "balance": inp["balance"], "rebalance": inp["rebalance"], "cuts": inp["cuts"]}
+           "rows": [r0, r1], "balance": inp["balance"], "rebalance": inp["rebalance"], "cuts": inp["cuts"], "outputs": outputs}
 
     # ---- (1b) the other per-step mode of the training loops (MSE + Pearson moments in the same pass), briefly
     if primary and loss_mode == "mse":
@@ -889,6 +917,8 @@ def measure_workload(env: Env, name: str, primary: bool):
         if primary:
             profile_region("train", False)
         env.windows["train" if primary else f"train_{name}"] = (w0, time.time())
+        if outputs is not None:
+            outputs.update(train_total=total.reshape(1).cpu(), train_moments=_m.cpu())
         t_ms = max_over_ranks(start.elapsed_time(stop))
         train_out = {"steps_per_s": Kt / (t_ms * 1e-3), "ms_per_step": t_ms / Kt, "steps": Kt, "model": model_cls.__name__,
                      "loss": {"mse": "mse", "mse_pearson": "mse + alpha*(1-pearson)"}.get(tmode, tmode), "nnz": graph.nnz, "total_loss": float(total),
@@ -1055,6 +1085,8 @@ def run_native(args):
             "check": {"mse": res["mse"]},
         }
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, res["outputs"])
     if world > 1:
         env.dist.destroy_process_group()
 

@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -21,6 +23,28 @@ def test_reference_arm_prints_contract_line():
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["d2h_bytes_per_step"] == 0
 
 
+def test_reference_arm_dumps_identical_outputs(tmp_path):
+    import numpy as np
+
+    dumps = []
+    for run in range(2):
+        d = tmp_path / f"run{run}"
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "c3", "--steps", "2", "--warmup", "1",
+                              "--cpu-sample-pairs", "2e5", "--dump-outputs", str(d)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        dumps.append({f.stem: np.load(f) for f in sorted(d.glob("*.npy"))})
+    assert sorted(dumps[0]) == ["loss", "loss_grad"]
+    assert dumps[0]["loss_grad"].shape == (2493, 3) and dumps[0]["loss_grad"].dtype == np.float32
+    assert dumps[0]["loss"].dtype == np.float64 and dumps[0]["loss"][0] > 0
+    for name, a in dumps[0].items():
+        assert np.array_equal(a, dumps[1][name]), name
+
+
+def test_steps_below_one_are_refused():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"], capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert out.returncode != 0 and "--steps" in out.stderr
+
+
 def test_reference_arm_other_ranks_exit_quietly():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"], capture_output=True, text=True, timeout=120, cwd=ROOT, env=env)
@@ -34,6 +58,25 @@ def test_native_arm_needs_cuda():
         return
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1"], capture_output=True, text=True, timeout=300, cwd=ROOT)
     assert out.returncode != 0 and "no CPU fallback" in (out.stderr + out.stdout)
+
+
+@pytest.mark.gpu
+def test_native_arm_dumps_the_last_timed_step(tmp_path):
+    import numpy as np
+
+    n = 2493
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "c3", "--steps", "3", "--warmup", "3", "--train-steps", "2",
+                          "--configs", "none", "--no-e2e", "--no-sparse", "--no-cpu-baseline", "--no-measure-copy", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    d = {f.stem: np.load(f) for f in sorted(tmp_path.glob("*.npy"))}
+    assert sorted(d) == ["loss_grad", "loss_moments", "train_moments", "train_total"]
+    assert d["loss_grad"].shape == (n, 3) and d["loss_grad"].dtype == np.float32 and np.isfinite(d["loss_grad"]).all()
+    assert d["loss_moments"].dtype == np.float64 and d["loss_moments"][0] / n**2 == line["check"]["mse"]
+    g = d["loss_grad"].astype(np.float64)
+    assert np.abs(g.sum(0)).max() <= 1e-4 * np.abs(g).sum(0).max()  # translation invariance: sum_i grad_i = 0
+    assert float(d["train_total"][0]) == line["train"]["total_loss"]
 
 
 def test_committed_native_lines_carry_the_contract_keys():
