@@ -14,7 +14,10 @@ The contact lists come from tests/golden (copies of the reference's Data/ fixtur
 embeddings are replaced by seeded stand-ins (node2vec / gensim are not part of the hot path): the 500 kb stand-ins are a
 rotated, noisy interleaving of the 1 Mb ones, so that the alignment has something to recover.
 
-    python examples/chr19_generalize.py [--steps 300] [--out /tmp/chr19_500kb_generalized_structure.pdb]
+    python examples/chr19_generalize.py [--steps 300] [--loss mse_pearson|mse_pearson_grad] [--out /tmp/chr19_500kb_generalized_structure.pdb]
+
+``--loss mse_pearson`` (default) is the reference's loss, whose Pearson term carries no gradient; ``mse_pearson_grad`` trains
+on the same total with the gradient of the (1 - r) term as well.
 """
 import argparse
 import io
@@ -42,6 +45,7 @@ def main():
     ap.add_argument("-lr", type=float, default=1e-3)
     ap.add_argument("-thresh", type=float, default=1e-8)
     ap.add_argument("-conversion", type=float, default=1.0)
+    ap.add_argument("--loss", default="mse_pearson", choices=["mse_pearson", "mse_pearson_grad"])
     ap.add_argument("--out", default="")
     args = ap.parse_args()
     g = np.load(os.path.join(ROOT, "tests", "golden", "reference_golden.npz"))
@@ -60,7 +64,7 @@ def main():
     target = utils.wish_target(data.y, args.conversion)
     torch.manual_seed(42)
     model = models.GATNetSelectiveResidualsUpdated().cuda()
-    hist = train.fit(model, data.x.float(), data.edge_index, target, mode="mse_pearson", lr=args.lr, thresh=args.thresh, max_steps=args.steps,
+    hist = train.fit(model, data.x.float(), data.edge_index, target, mode=args.loss, lr=args.lr, thresh=args.thresh, max_steps=args.steps,
                      use_cuda_graph=True, check_every=10)
     with torch.no_grad():
         dscc_trained = metrics.dscc(model.get_model(data.x.float(), data.edge_index), target)
@@ -80,7 +84,7 @@ def main():
     dscc_generalised = metrics.dscc(coords, target_fit)
     if args.out:
         utils.WritePDB(coords * 100, args.out)
-    print(f"trained on {n1} loci: steps={len(hist)} loss {hist[0]:.5f} -> {hist[-1]:.5f} dSCC={dscc_trained:.4f}; "
+    print(f"loss {args.loss}: trained on {n1} loci: steps={len(hist)} loss {hist[0]:.5f} -> {hist[-1]:.5f} dSCC={dscc_trained:.4f}; "
           f"generalised to {n2} loci: dSCC={dscc_generalised:.4f}" + (f"; wrote {args.out}" if args.out else ""))
     return hist, coords, dscc_trained, dscc_generalised
 

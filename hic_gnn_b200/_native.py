@@ -34,6 +34,8 @@ SIGNATURES = {
     "hicgat_pairloss_describe_schedule_mode": (C.c_int, [_i64, _i64, _i64, _u32, _p, _i32]),
     "hicgat_pairloss_sparse_workspace_bytes": (_sz, [_i64, _i64, _i64]),
     "hicgat_pairloss_sparse_fwd_bwd": (C.c_int, [_p, _p, _p, _p, _f32, _i64, _i64, _i64, _u32, _f32, _f32, _p, _p, _p, _sz, _p]),
+    "hicgat_pairloss_pearson_grad": (C.c_int, [_p, _p, _i64, _i64, _i64, _i64, _u32, _p, _f32, _i32, _p, _p, _sz, _p]),
+    "hicgat_pairloss_sparse_pearson_grad": (C.c_int, [_p, _p, _p, _p, _f32, _i64, _i64, _i64, _u32, _p, _f32, _i32, _p, _p, _sz, _p]),
     "hicgat_asymmetry_f32": (C.c_int, [_p, _i64, _i64, _i64, _i64, _p, _p]),
     "hicgat_asymmetry_f64": (C.c_int, [_p, _i64, _i64, _i64, _i64, _p, _p]),
     "hicgat_pairloss_rowside_add": (C.c_int, [_p, _p, _i64, _i64, _i64, _i64, _f32, _p, _p]),

@@ -94,9 +94,27 @@ __device__ __forceinline__ void acc_zero(Acc& a) {
     a.sabs0 = a.sabs1 = 0.f;
 }
 
+// Second pass of the differentiable Pearson modes (hicgat_pairloss_pearson_grad): the per-pair weight needs the GLOBAL
+// moments, so it is a library-internal mode bit that only those entry points set.
+constexpr uint32_t kPearson = 64u;
+// true when the instantiation produces a gradient (the MSE / L1 bits or the Pearson pass)
+__host__ __device__ constexpr bool has_grad(uint32_t mode) { return (mode & (3u | kPearson)) != 0; }
+
+// Coefficients of the Pearson pass, derived on the device from the global moments (see pearson_coef):
+// w = (c_mse (d - t) + lamA rho) / d,  rho = t - (beta d + kappa)
+struct PearsonCoef {
+    f2 lam_a, beta, kappa, cm;
+};
+
 template <uint32_t MODE>
-__device__ __forceinline__ f2 grad_weight(f2 e, f2 rs, float c_mse, float c_l1) {
-    if constexpr ((MODE & 3u) == HICGAT_PAIR_GRAD_MSE) {
+__device__ __forceinline__ f2 grad_weight(f2 e, f2 rs, float c_mse, float c_l1, f2 d, f2 t, const PearsonCoef& pc) {
+    if constexpr ((MODE & kPearson) != 0) {
+        // the residual of the regression of t on d, formed in f32 as t - fma(beta, d, kappa), and the MSE residual are kept
+        // apart: folding them into one affine a t + b d + c loses the cancellation of t against beta d + kappa near r = 1
+        f2 w = f2_mul(pc.lam_a, f2_sub(t, f2_fma(pc.beta, d, pc.kappa)));
+        if constexpr ((MODE & HICGAT_PAIR_GRAD_MSE) != 0) w = f2_fma(pc.cm, e, w);
+        return f2_mul(w, rs);
+    } else if constexpr ((MODE & 3u) == HICGAT_PAIR_GRAD_MSE) {
         return f2_mul(e, rs);
     } else if constexpr ((MODE & 3u) == HICGAT_PAIR_GRAD_L1) {
         float ea, eb, ra, rb;
@@ -127,7 +145,7 @@ struct RowAcc {
 // accumulators and the strictly-upper sum of squares is kept apart (it counts twice in the full-matrix loss).
 template <uint32_t MODE, bool UPPER, bool ROWS>
 __device__ __forceinline__ void pair_fast(Acc& a, RowAcc& ra, int p, f2 xjx, f2 xjy, f2 xjz, f2 xix, f2 xiy,
-                                          f2 xiz, f2 t, float c_mse, float c_l1) {
+                                          f2 xiz, f2 t, float c_mse, float c_l1, const PearsonCoef& pc) {
     f2 dx = f2_sub(xjx, xix), dy = f2_sub(xjy, xiy), dz = f2_sub(xjz, xiz);
     f2 d2 = f2_fma(dx, dx, f2_fma(dy, dy, f2_fma(dz, dz, HICGAT_TINY2)));
     float d2a, d2b;
@@ -136,10 +154,12 @@ __device__ __forceinline__ void pair_fast(Acc& a, RowAcc& ra, int p, f2 xjx, f2 
     f2 d = f2_mul(d2, rs);
     f2 e = f2_sub(d, t);
     constexpr bool kMom = UPPER && (MODE & (kMomFull | kMomLight));
-    if constexpr (kMom || (UPPER && ROWS)) a.seu = f2_fma(e, e, a.seu);
+    if constexpr ((MODE & kPearson) != 0) {
+        // the Pearson pass produces the gradient only (its moments are an input)
+    } else if constexpr (kMom || (UPPER && ROWS)) a.seu = f2_fma(e, e, a.seu);
     else a.see = f2_fma(e, e, a.see);
-    if constexpr ((MODE & 3u) != 0) {
-        f2 w = grad_weight<MODE>(e, rs, c_mse, c_l1);
+    if constexpr (has_grad(MODE)) {
+        f2 w = grad_weight<MODE>(e, rs, c_mse, c_l1, d, t, pc);
         a.gx[p] = f2_fma(w, dx, a.gx[p]);
         a.gy[p] = f2_fma(w, dy, a.gy[p]);
         a.gz[p] = f2_fma(w, dz, a.gz[p]);
@@ -168,7 +188,7 @@ __device__ __forceinline__ void pair_fast(Acc& a, RowAcc& ra, int p, f2 xjx, f2 
 // mv: 1 for valid (row, column) -- in upper-triangle mode additionally row <= column; mu: 1 where row < col.
 template <uint32_t MODE, bool ROWS>
 __device__ __forceinline__ void pair_masked(Acc& a, RowAcc& ra, int p, f2 xjx, f2 xjy, f2 xjz, f2 xix, f2 xiy,
-                                            f2 xiz, f2 t, f2 mv, f2 mu, float c_mse, float c_l1) {
+                                            f2 xiz, f2 t, f2 mv, f2 mu, float c_mse, float c_l1, const PearsonCoef& pc) {
     f2 dx = f2_sub(xjx, xix), dy = f2_sub(xjy, xiy), dz = f2_sub(xjz, xiz);
     f2 d2 = f2_fma(dx, dx, f2_fma(dy, dy, f2_fma(dz, dz, HICGAT_TINY2)));
     float d2a, d2b;
@@ -177,8 +197,8 @@ __device__ __forceinline__ void pair_masked(Acc& a, RowAcc& ra, int p, f2 xjx, f
     f2 d = f2_mul(d2, rs);
     f2 e = f2_mul(f2_sub(d, t), mv);
     constexpr bool kMom = (MODE & (kMomFull | kMomLight)) != 0;
-    if constexpr ((MODE & 3u) != 0) {
-        f2 w = f2_mul(grad_weight<MODE>(e, rs, c_mse, c_l1), mv);
+    if constexpr (has_grad(MODE)) {
+        f2 w = f2_mul(grad_weight<MODE>(e, rs, c_mse, c_l1, d, t, pc), mv);
         a.gx[p] = f2_fma(w, dx, a.gx[p]);
         a.gy[p] = f2_fma(w, dy, a.gy[p]);
         a.gz[p] = f2_fma(w, dz, a.gz[p]);
@@ -188,7 +208,9 @@ __device__ __forceinline__ void pair_masked(Acc& a, RowAcc& ra, int p, f2 xjx, f
             ra.z = f2_fma(w, dz, ra.z);
         }
     }
-    if constexpr (kMom || ROWS) {
+    if constexpr ((MODE & kPearson) != 0) {
+        // gradient only, as in pair_fast
+    } else if constexpr (kMom || ROWS) {
         f2 eu = f2_mul(e, mu);
         f2 el = f2_sub(e, eu);  // the part of e not under the upper mask
         a.see = f2_fma(el, el, a.see);
@@ -251,7 +273,41 @@ struct Params {
     int rs_first, rs_count, rs_groups;
     double* rs_scratch;       // [rs_count][rs_groups][384] segment sums
     unsigned* rs_ticket;      // [rs_count] arrival counters, zero between calls
+    // Pearson pass: the global f64 moments of the first pass (read on the device only) and whether the Pearson term is
+    // weighted by alpha = min(1, 0.1 + 1 / (MSE + 1e-6)) (mse_pearson_grad) or by 1 (pearson)
+    const double* pmom;
+    int dyn_alpha;
 };
+
+// r, beta, kappa, A and alpha from the global moments (f64), rounded once to f32.  Called after griddepcontrol.wait (the
+// moments are written by the previous kernels of the stream).  Degenerate moments (v_d v_t <= 0 or not finite: n <= 2,
+// coincident loci, a constant target) give a zero Pearson weight: r is NaN there and carries no gradient.
+template <uint32_t MODE>
+__device__ __forceinline__ PearsonCoef pearson_coef(const double* pm, int n, float c_mse, int dyn_alpha) {
+    PearsonCoef pc;
+    pc.lam_a = pc.beta = pc.kappa = pc.cm = 0ull;
+    if constexpr ((MODE & kPearson) != 0) {
+        const double np = 0.5 * (double)n * (double)(n - 1);
+        const double sd = pm[2], sdd = pm[3], st = pm[4], stt = pm[5], sdt = pm[6];
+        const double vd = sdd - sd * sd / np, vt = stt - st * st / np, c = sdt - sd * st / np;
+        const double prod = vd * vt;
+        if (prod > 0.0 && prod < INFINITY) {
+            const double beta = c / vd;
+            const double kappa = st / np - beta * (sd / np);
+            double lam = 1.0;
+            if (dyn_alpha) {  // the loss value's f32 MSE, as MSELoss returns it
+                const double mse = (double)(float)(pm[0] / ((double)n * (double)n));
+                lam = fmin(1.0, 0.1 + 1.0 / (mse + 1e-6));
+            }
+            const float la = (float)(-lam / sqrt(prod)), b = (float)beta, k = (float)kappa;
+            pc.lam_a = f2_pack(la, la);
+            pc.beta = f2_pack(b, b);
+            pc.kappa = f2_pack(k, k);
+        }
+        pc.cm = f2_pack(c_mse, c_mse);
+    }
+    return pc;
+}
 
 struct ColumnRegs {
     f2 xjx[2], xjy[2], xjz[2], mv[2];
@@ -310,9 +366,10 @@ __device__ __forceinline__ int row_butterfly_slot(int lane) {
 template <uint32_t MODE, bool ROWS, typename XI>
 __device__ __forceinline__ void process_group(Acc& a, const ColumnRegs& c, const float4 (&t)[kU], const XI xi,
                                               int rows_here, int rg, int col0, int n, bool edge,
-                                              int strip_lo, int strip_hi, float c_mse, float c_l1, float* __restrict__ rowdst, int lane) {
+                                              int strip_lo, int strip_hi, float c_mse, float c_l1, float* __restrict__ rowdst, int lane,
+                                              const PearsonCoef& pc) {
     const bool fast = !edge && rows_here == kU;
-    constexpr bool kRowGrad = ROWS && (MODE & 3u) != 0;
+    constexpr bool kRowGrad = ROWS && has_grad(MODE);
     float rv[kRowGrad ? 3 * kU : 1];
     if (fast && rg + kU - 1 < strip_lo) {  // strictly above the diagonal
 #pragma unroll
@@ -322,8 +379,8 @@ __device__ __forceinline__ void process_group(Acc& a, const ColumnRegs& c, const
             xi.load(u, xy, zz);
             f2 xix = f2_pack(xy.x, xy.y), xiy = f2_pack(xy.z, xy.w), xiz = f2_pack(zz.x, zz.y);
             RowAcc ra = {0ull, 0ull, 0ull};
-            pair_fast<MODE, true, ROWS>(a, ra, 0, c.xjx[0], c.xjy[0], c.xjz[0], xix, xiy, xiz, f2_pack(t[u].x, t[u].y), c_mse, c_l1);
-            pair_fast<MODE, true, ROWS>(a, ra, 1, c.xjx[1], c.xjy[1], c.xjz[1], xix, xiy, xiz, f2_pack(t[u].z, t[u].w), c_mse, c_l1);
+            pair_fast<MODE, true, ROWS>(a, ra, 0, c.xjx[0], c.xjy[0], c.xjz[0], xix, xiy, xiz, f2_pack(t[u].x, t[u].y), c_mse, c_l1, pc);
+            pair_fast<MODE, true, ROWS>(a, ra, 1, c.xjx[1], c.xjy[1], c.xjz[1], xix, xiy, xiz, f2_pack(t[u].z, t[u].w), c_mse, c_l1, pc);
             if constexpr (kRowGrad) {
                 rv[3 * u] = f2_hsum(ra.x); rv[3 * u + 1] = f2_hsum(ra.y); rv[3 * u + 2] = f2_hsum(ra.z);
             }
@@ -336,8 +393,8 @@ __device__ __forceinline__ void process_group(Acc& a, const ColumnRegs& c, const
             xi.load(u, xy, zz);
             f2 xix = f2_pack(xy.x, xy.y), xiy = f2_pack(xy.z, xy.w), xiz = f2_pack(zz.x, zz.y);
             RowAcc ra = {0ull, 0ull, 0ull};
-            pair_fast<MODE, false, false>(a, ra, 0, c.xjx[0], c.xjy[0], c.xjz[0], xix, xiy, xiz, f2_pack(t[u].x, t[u].y), c_mse, c_l1);
-            pair_fast<MODE, false, false>(a, ra, 1, c.xjx[1], c.xjy[1], c.xjz[1], xix, xiy, xiz, f2_pack(t[u].z, t[u].w), c_mse, c_l1);
+            pair_fast<MODE, false, false>(a, ra, 0, c.xjx[0], c.xjy[0], c.xjz[0], xix, xiy, xiz, f2_pack(t[u].x, t[u].y), c_mse, c_l1, pc);
+            pair_fast<MODE, false, false>(a, ra, 1, c.xjx[1], c.xjy[1], c.xjz[1], xix, xiy, xiz, f2_pack(t[u].z, t[u].w), c_mse, c_l1, pc);
         }
     } else {
 #pragma unroll
@@ -356,8 +413,8 @@ __device__ __forceinline__ void process_group(Acc& a, const ColumnRegs& c, const
                     mv0 = f2_pack((col0 + 0 < n && r <= col0 + 0) ? 1.f : 0.f, (col0 + 1 < n && r <= col0 + 1) ? 1.f : 0.f);
                     mv1 = f2_pack((col0 + 2 < n && r <= col0 + 2) ? 1.f : 0.f, (col0 + 3 < n && r <= col0 + 3) ? 1.f : 0.f);
                 }
-                pair_masked<MODE, ROWS>(a, ra, 0, c.xjx[0], c.xjy[0], c.xjz[0], xix, xiy, xiz, f2_pack(t[u].x, t[u].y), mv0, mu0, c_mse, c_l1);
-                pair_masked<MODE, ROWS>(a, ra, 1, c.xjx[1], c.xjy[1], c.xjz[1], xix, xiy, xiz, f2_pack(t[u].z, t[u].w), mv1, mu1, c_mse, c_l1);
+                pair_masked<MODE, ROWS>(a, ra, 0, c.xjx[0], c.xjy[0], c.xjz[0], xix, xiy, xiz, f2_pack(t[u].x, t[u].y), mv0, mu0, c_mse, c_l1, pc);
+                pair_masked<MODE, ROWS>(a, ra, 1, c.xjx[1], c.xjy[1], c.xjz[1], xix, xiy, xiz, f2_pack(t[u].z, t[u].w), mv1, mu1, c_mse, c_l1, pc);
             }
             if constexpr (kRowGrad) {
                 rv[3 * u] = f2_hsum(ra.x); rv[3 * u + 1] = f2_hsum(ra.y); rv[3 * u + 2] = f2_hsum(ra.z);
@@ -417,7 +474,7 @@ struct CombineSmem {
 // warp-level part of the CTA combine: park this warp's gradients / moments in shared memory
 template <uint32_t MODE, bool ROWS = false>
 __device__ __forceinline__ void park_warp(const Acc& a, CombineSmem& S, int warp, int lane) {
-    if constexpr ((MODE & 3u) != 0) {
+    if constexpr (has_grad(MODE)) {
 #pragma unroll
         for (int p = 0; p < 2; ++p) {
             float x0, x1, y0, y1, z0, z1;
@@ -472,7 +529,7 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 template <uint32_t MODE>
 __device__ __forceinline__ void publish_cta(const Params& P, CombineSmem& S, int strip, int chunk, int tid, int nthreads) {
     const int cta = chunk * P.nstrips + strip;
-    if constexpr ((MODE & 3u) != 0) {
+    if constexpr (has_grad(MODE)) {
         float* gp = P.gpart + (size_t)cta * (kCols * 3);
         for (int i = tid; i < kCols * 3; i += nthreads) {
             float s = 0.f;
@@ -551,7 +608,9 @@ __global__ void __launch_bounds__(kCombineThreads, 2) pairloss_combine_kernel(co
         const bool live = pass == npass - 1;
         if (live) {
             pdl_wait();  // no-op when launched without the programmatic-serialization attribute
-            if (P.work_counter && bid == 0 && tid == 0) *P.work_counter = 0u;  // the persistent kernel's item counter, for the next launch
+            // the persistent kernel's item counter, for the next launch: reset by block 0 (the moment CTA), the one CTA that reaches this
+            // live pass in every mode (strip and row-side CTAs may return in the first pass under programmatic dependent launch)
+            if (P.work_counter && blockIdx.x == 0 && tid == 0) *P.work_counter = 0u;
 #ifdef HICGAT_TRACE
             if (ctr) ctr[1] = gtimer();
 #endif
@@ -606,6 +665,10 @@ __global__ void __launch_bounds__(kCombineThreads, 2) pairloss_combine_kernel(co
                 }
             }
         } else {
+            if (!P.moments) {  // Pearson pass: the moments are an input (P.pmom), nothing to sum; stay for the live pass's counter reset
+                if (live) return;
+                continue;
+            }
             double m[kNM];
 #pragma unroll
             for (int k = 0; k < kNM; ++k) m[k] = 0.0;
@@ -674,6 +737,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_ldg_kernel(cons
     load_columns(c, P.coords, col0, n);
     Acc a;
     acc_zero(a);
+    const PearsonCoef pc = pearson_coef<MODE>(P.pmom, n, P.c_mse, P.dyn_alpha);
     __syncthreads();
 
     const bool can_load = col0 + 3 < P.pitch;  // pitch is a multiple of 4
@@ -694,7 +758,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_ldg_kernel(cons
                 t[u] = (u < rows_here && can_load) ? ldg_stream_f4(tbase + (size_t)(rl + u) * P.pitch)
                                                    : make_float4(0.f, 0.f, 0.f, 0.f);
         }
-        process_group<MODE, false>(a, c, t, XiPtr{s_xy + rl, s_z + rl}, rows_here, row_begin + rl, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1, nullptr, lane);
+        process_group<MODE, false>(a, c, t, XiPtr{s_xy + rl, s_z + rl}, rows_here, row_begin + rl, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1, nullptr, lane, pc);
     }
     park_warp<MODE>(a, S, warp, lane);
     __syncthreads();
@@ -733,6 +797,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_const_kernel(co
     load_columns(c, P.coords, col0, n);
     Acc a;
     acc_zero(a);
+    const PearsonCoef pc = pearson_coef<MODE>(P.pmom, n, P.c_mse, P.dyn_alpha);
     __syncthreads();
     const int strip_lo = strip * kCols, strip_hi = strip_lo + kCols - 1;
     const int ngroups = (nrows + kU - 1) / kU;
@@ -754,7 +819,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_const_kernel(co
             }
         }
         process_group<MODE, ROWS>(a, c, t, XiPtr{s_xy + rl, s_z + rl}, rows_here, rg, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1,
-                                  ROWS ? P.rpart + (size_t)strip * P.rpitch + (size_t)(rg - P.r0) * 3 : nullptr, lane);
+                                  ROWS ? P.rpart + (size_t)strip * P.rpitch + (size_t)(rg - P.r0) * 3 : nullptr, lane, pc);
     }
     park_warp<MODE, ROWS>(a, S, warp, lane);
     __syncthreads();
@@ -772,13 +837,20 @@ __global__ void __launch_bounds__(256) pairloss_csr_fix_kernel(const float* __re
                                                                const int32_t* __restrict__ col, const float* __restrict__ tval, float fill, int n,
                                                                int r0, int r1, float c_mse, float c_l1, double* __restrict__ moments,
                                                                float* __restrict__ grad, double* __restrict__ grad64, double* __restrict__ part,
-                                                               unsigned* __restrict__ counter) {
+                                                               unsigned* __restrict__ counter, const double* __restrict__ pmom, int dyn_alpha) {
     __shared__ double s_m[8][kNM];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int i = r0 + blockIdx.x * 8 + warp;
     double m[kNM];
 #pragma unroll
     for (int k = 0; k < kNM; ++k) m[k] = 0.0;
+    float lam_a = 0.f, cm = 0.f;
+    if constexpr ((MODE & kPearson) != 0) {
+        float u;
+        const PearsonCoef pc = pearson_coef<MODE>(pmom, n, c_mse, dyn_alpha);
+        f2_unpack(pc.lam_a, lam_a, u);
+        if constexpr ((MODE & HICGAT_PAIR_GRAD_MSE) != 0) cm = c_mse;
+    }
     if (i < r1) {
         const float xi = coords[(size_t)i * 3], yi = coords[(size_t)i * 3 + 1], zi = coords[(size_t)i * 3 + 2];
         float gx = 0.f, gy = 0.f, gz = 0.f;
@@ -794,7 +866,9 @@ __global__ void __launch_bounds__(256) pairloss_csr_fix_kernel(const float* __re
             const double dsee = (double)et * et - (double)ef * ef;
             m[0] += dsee;
             float w = 0.f;
-            if constexpr ((MODE & 3u) == HICGAT_PAIR_GRAD_MSE) w = c_mse * (fill - t) * rs;
+            // Pearson pass: [c_mse (d - t) + lamA (t - beta d - kappa)] - [the same at t = fill] = (lamA - c_mse) (t - fill)
+            if constexpr ((MODE & kPearson) != 0) w = (lam_a * (t - fill) + cm * (fill - t)) * rs;
+            else if constexpr ((MODE & 3u) == HICGAT_PAIR_GRAD_MSE) w = c_mse * (fill - t) * rs;
             else if constexpr ((MODE & 3u) == HICGAT_PAIR_GRAD_L1) w = c_l1 * (copysignf(1.f, et) - copysignf(1.f, ef)) * rs;
             else if constexpr ((MODE & 3u) == 3u) w = (c_mse * (fill - t) + c_l1 * (copysignf(1.f, et) - copysignf(1.f, ef))) * rs;
             gx = fmaf(w, dx, gx); gy = fmaf(w, dy, gy); gz = fmaf(w, dz, gz);
@@ -810,7 +884,7 @@ __global__ void __launch_bounds__(256) pairloss_csr_fix_kernel(const float* __re
                 }
             }
         }
-        if constexpr ((MODE & 3u) != 0) {
+        if constexpr (has_grad(MODE)) {
             gx = warp_sum(gx); gy = warp_sum(gy); gz = warp_sum(gz);
             if (lane == 0) {
                 if (grad) { grad[(size_t)i * 3] += gx; grad[(size_t)i * 3 + 1] += gy; grad[(size_t)i * 3 + 2] += gz; }
@@ -859,7 +933,7 @@ __global__ void __launch_bounds__(256) pairloss_csr_fix_kernel(const float* __re
         for (int k = 0; k < kNM; ++k) s_m[warp][k] = m[k];
     }
     __syncthreads();
-    if (threadIdx.x < kNM) {
+    if (threadIdx.x < kNM && moments) {  // no moments in the Pearson pass
         double s = 0.0;
 #pragma unroll
         for (int w = 0; w < 8; ++w) s += s_m[w][threadIdx.x];
@@ -976,6 +1050,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_kernel(cons
     load_columns(c, P.coords, col0, n);
     Acc a;
     acc_zero(a);
+    const PearsonCoef pc = pearson_coef<MODE>(P.pmom, n, P.c_mse, P.dyn_alpha);
     __syncwarp();
 
     for (int t = 0; t < ntiles; ++t) {
@@ -994,7 +1069,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_kernel(cons
         for (int u = 0; u < kU; ++u) tv[u] = lds_f4(slot + lane * 16 + u * (kCols * 4));
         const int rg = row_begin + t * kTileRows + wrow;
         process_group<MODE, ROWS>(a, c, tv, xi, rows_here, rg, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1,
-                                  ROWS ? P.rpart + (size_t)strip * P.rpitch + (size_t)(rg - P.r0) * 3 : nullptr, lane);
+                                  ROWS ? P.rpart + (size_t)strip * P.rpitch + (size_t)(rg - P.r0) * 3 : nullptr, lane, pc);
         __syncwarp();  // every lane is done with slot s
         if (refill) {
             if (lane == 0) issue(t + kStages, s);
@@ -1102,6 +1177,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_persist_ker
         load_columns(c, P.coords, col0, n);
         Acc a;
         acc_zero(a);
+        const PearsonCoef pc = pearson_coef<MODE>(P.pmom, n, P.c_mse, P.dyn_alpha);
         for (int t = 0; t < ntiles; ++t) {
             const unsigned g = gt + t;
             const int s = (int)(g % kStages);
@@ -1116,7 +1192,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_persist_ker
             for (int u = 0; u < kU; ++u) tv[u] = lds_f4(slot + lane * 16 + u * (kCols * 4));
             const int rg = row_begin + t * kTileRows + wrow;
             process_group<MODE, ROWS>(a, c, tv, xi, rows_here, rg, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1,
-                                      ROWS ? P.rpart + (size_t)strip * P.rpitch + (size_t)(rg - P.r0) * 3 : nullptr, lane);
+                                      ROWS ? P.rpart + (size_t)strip * P.rpitch + (size_t)(rg - P.r0) * 3 : nullptr, lane, pc);
             __syncwarp();  // every lane is done with slot s
             if (refill) issue(strip, row_begin, t + kStages, g + kStages, xi_next);
         }
@@ -1151,7 +1227,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_persist_ker
             }
         }
         float gv[2][6];
-        if constexpr ((MODE & 3u) != 0) {
+        if constexpr (has_grad(MODE)) {
 #pragma unroll
             for (int p = 0; p < 2; ++p) {
                 f2_unpack(a.gx[p], gv[p][0], gv[p][3]);
@@ -1168,7 +1244,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_persist_ker
             }
         }
         __syncthreads();
-        if constexpr ((MODE & 3u) != 0) {
+        if constexpr (has_grad(MODE)) {
             if (warp < kWarps / 2) {
 #pragma unroll
                 for (int p = 0; p < 2; ++p) {
@@ -1181,7 +1257,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_persist_ker
         __syncthreads();
         {
             const int cta = chunk * P.nstrips + strip;
-            if constexpr ((MODE & 3u) != 0) {
+            if constexpr (has_grad(MODE)) {
                 float* gp = P.gpart + (size_t)cta * (kCols * 3);
                 for (int i = threadIdx.x; i < kCols * 3; i += kThreads) {
                     float sum = 0.f;
@@ -1303,6 +1379,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_warp_kernel
         load_columns(c, P.coords, col0, n);
         Acc a;
         acc_zero(a);
+        const PearsonCoef pc = pearson_coef<MODE>(P.pmom, n, P.c_mse, P.dyn_alpha);
         __syncwarp();
         for (int t = 0; t < ntiles; ++t) {
             const unsigned g = gt + t;
@@ -1318,7 +1395,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_warp_kernel
             for (int u = 0; u < kU; ++u) tv[u] = lds_f4(slot + lane * 16 + u * (kCols * 4));
             const int rg = row_begin + t * kU;
             process_group<MODE, ROWS>(a, c, tv, xi, rows_here, rg, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1,
-                                      ROWS ? P.rpart + (size_t)strip * P.rpitch + (size_t)(rg - P.r0) * 3 : nullptr, lane);
+                                      ROWS ? P.rpart + (size_t)strip * P.rpitch + (size_t)(rg - P.r0) * 3 : nullptr, lane, pc);
             __syncwarp();
             if (refill) issue(t + kStages, g + kStages, xi_next);
         }
@@ -1326,7 +1403,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_warp_kernel
         // ---- publish this warp's partial of the strip: slot (segment index, strip)
         const int seg = (int)(gw - soff / P.seg_len);
         const size_t slot_id = (size_t)seg * P.nstrips + strip;
-        if constexpr ((MODE & 3u) != 0) {
+        if constexpr (has_grad(MODE)) {
             float* gp = P.gpart + slot_id * (kCols * 3) + lane * 12;
             float x0, x1, y0, y1, z0, z1, x2, x3, y2, y3, z2, z3;
             f2_unpack(a.gx[0], x0, x1); f2_unpack(a.gy[0], y0, y1); f2_unpack(a.gz[0], z0, z1);
@@ -1748,8 +1825,9 @@ bool make_target_map(CUtensorMap* map, const float* target, int64_t pitch, int64
 
 template <uint32_t MODE>
 cudaError_t launch_combine(const Params& P, cudaStream_t stream) {
-    const float scale = ((MODE & 3u) == HICGAT_PAIR_GRAD_MSE) ? P.c_mse : ((MODE & 3u) == HICGAT_PAIR_GRAD_L1) ? P.c_l1 : 1.f;
-    const int want_grad = (MODE & 3u) != 0 ? 1 : 0;
+    // the Pearson pass carries its coefficients in the per-pair weight: no scale
+    const float scale = (MODE & kPearson) ? 1.f : ((MODE & 3u) == HICGAT_PAIR_GRAD_MSE) ? P.c_mse : ((MODE & 3u) == HICGAT_PAIR_GRAD_L1) ? P.c_l1 : 1.f;
+    const int want_grad = has_grad(MODE) ? 1 : 0;
     if (g_pdl) {
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3(P.nstrips + 1 + (P.rs_groups > 1 ? P.rs_groups * P.rs_count : 0));
@@ -1962,11 +2040,11 @@ extern "C" size_t hicgat_pairloss_workspace_bytes_mode(int64_t n, int64_t r0, in
 static int pairloss_impl(const float* coords, const float* target, int64_t pitch, int64_t n,
                          int64_t r0, int64_t r1, uint32_t mode, float c_mse, float c_l1,
                          double* moments, float* grad, double* grad64, void* workspace, size_t workspace_bytes,
-                         hicgat_stream_t stream_) {
+                         hicgat_stream_t stream_, const double* pmom = nullptr, int dyn_alpha = 0) {
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     HICGAT_REQUIRE(n > 0 && n < (1ll << 30) && r0 >= 0 && r1 >= r0 && r1 <= n, "hicgat_pairloss_fwd_bwd: bad n/r0/r1 (%lld,%lld,%lld)", (long long)n, (long long)r0, (long long)r1);
     // an empty row block (r0 == r1, a trailing rank of a sharded run) has no target rows to point at
-    HICGAT_REQUIRE(coords && (target || r0 == r1) && moments && workspace, "hicgat_pairloss_fwd_bwd: null pointer");
+    HICGAT_REQUIRE(coords && (target || r0 == r1) && (moments || pmom) && workspace, "hicgat_pairloss_fwd_bwd: null pointer");
     HICGAT_REQUIRE(pitch >= n && (pitch % 4) == 0, "hicgat_pairloss_fwd_bwd: pitch %lld must be >= n and a multiple of 4", (long long)pitch);
     HICGAT_REQUIRE(aligned16(target), "hicgat_pairloss_fwd_bwd: target must be 16-byte aligned");  // NULL passes
     HICGAT_REQUIRE((mode & ~63u) == 0, "hicgat_pairloss_fwd_bwd: unknown mode bits 0x%x", mode);
@@ -1978,7 +2056,8 @@ static int pairloss_impl(const float* coords, const float* target, int64_t pitch
     if ((mode & HICGAT_PAIR_MOMENTS_D) && (mode & HICGAT_PAIR_GRAD_L1)) {     // the L1 value needs sum |d-t|: full set
         mode = (mode & ~HICGAT_PAIR_MOMENTS_D) | HICGAT_PAIR_MOMENTS;
     }
-    HICGAT_REQUIRE(!(mode & 3u) || grad || grad64, "hicgat_pairloss_fwd_bwd: grad is NULL but a gradient mode is set");
+    if (pmom) mode |= kPearson;  // second pass of the differentiable Pearson modes (hicgat_pairloss_pearson_grad)
+    HICGAT_REQUIRE(!has_grad(mode) || grad || grad64, "hicgat_pairloss_fwd_bwd: grad is NULL but a gradient mode is set");
     int variant = g_variant;
     CUtensorMap map;
     if (variant != 1 && r1 > r0 && !make_target_map(&map, target, pitch, n, r1 - r0)) variant = 1;
@@ -1990,7 +2069,7 @@ static int pairloss_impl(const float* coords, const float* target, int64_t pitch
     }
     unsigned char* ws = static_cast<unsigned char*>(workspace);
     if (r1 == r0) {  // empty row block: contributes nothing
-        HICGAT_CUDA(cudaMemsetAsync(moments, 0, sizeof(double) * kNM, stream));
+        if (moments) HICGAT_CUDA(cudaMemsetAsync(moments, 0, sizeof(double) * kNM, stream));
         if (grad) HICGAT_CUDA(cudaMemsetAsync(grad, 0, sizeof(float) * 3 * (size_t)n, stream));
         if (grad64) HICGAT_CUDA(cudaMemsetAsync(grad64, 0, sizeof(double) * 3 * (size_t)n, stream));
         return HICGAT_OK;
@@ -2000,6 +2079,7 @@ static int pairloss_impl(const float* coords, const float* target, int64_t pitch
     P.n = (int)n; P.r0 = (int)r0; P.r1 = (int)r1; P.rb = L.rb; P.nstrips = L.nstrips; P.nchunks = L.nchunks; P.stagger = L.stagger; P.sch = L.sch;
     P.fill = 0.f;
     P.c_mse = c_mse; P.c_l1 = c_l1; P.moments = moments; P.grad = grad; P.grad64 = grad64;
+    P.pmom = pmom; P.dyn_alpha = dyn_alpha;
     P.mpart = reinterpret_cast<double*>(ws + L.off_mpart);
     P.gpart = reinterpret_cast<float*>(ws + L.off_gpart);
     P.upper = sym ? 1 : 0; P.rpitch = L.rpitch; P.rpart = reinterpret_cast<float*>(ws + L.off_rpart);
@@ -2022,6 +2102,7 @@ static int pairloss_impl(const float* coords, const float* target, int64_t pitch
 #define HICGAT_CASE(M) case M: err = launch_mode<M>(variant, map, P, grid, stream); break;
         HICGAT_CASE(0u) HICGAT_CASE(1u) HICGAT_CASE(2u) HICGAT_CASE(3u) HICGAT_CASE(4u)
         HICGAT_CASE(5u) HICGAT_CASE(6u) HICGAT_CASE(7u) HICGAT_CASE(8u) HICGAT_CASE(9u)
+        HICGAT_CASE(64u) HICGAT_CASE(65u)
 #undef HICGAT_CASE
         default:
             set_error("hicgat_pairloss_fwd_bwd: unsupported mode 0x%x", mode);
@@ -2082,29 +2163,31 @@ cudaError_t launch_sparse(const Params& P, dim3 grid, const int32_t* rowptr, con
     e = launch_combine<MODE>(P, stream);
     if (e != cudaSuccess) return e;
     pairloss_csr_fix_kernel<MODE><<<fix_ctas, 256, 0, stream>>>(P.coords, rowptr, col, tval, P.fill, P.n, P.r0, P.r1, P.c_mse, P.c_l1, P.moments, P.grad,
-                                                                 P.grad64, part, counter);
+                                                                 P.grad64, part, counter, P.pmom, P.dyn_alpha);
     return cudaGetLastError();
 }
 }  // namespace
 
 extern "C" size_t hicgat_pairloss_sparse_workspace_bytes(int64_t n, int64_t r0, int64_t r1) {
     if (n <= 0 || r0 < 0 || r1 < r0 || r1 > n) return 0;
-    return sparse_layout(n, r0, r1, true).total;  // covers both the full-matrix and the upper-triangle (HICGAT_PAIR_SYMMETRIC) pass
+    return std::max(sparse_layout(n, r0, r1, true).total, sparse_layout(n, r0, r1, false).total);  // with or without HICGAT_PAIR_SYMMETRIC
 }
 
 static int pairloss_sparse_impl(const float* coords, const int32_t* rowptr, const int32_t* col, const float* tval, float fill, int64_t n,
                                 int64_t r0, int64_t r1, uint32_t mode, float c_mse, float c_l1, double* moments, float* grad, double* grad64,
-                                void* workspace, size_t workspace_bytes, hicgat_stream_t stream_) {
+                                void* workspace, size_t workspace_bytes, hicgat_stream_t stream_, const double* pmom = nullptr,
+                                int dyn_alpha = 0) {
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     HICGAT_REQUIRE(n > 0 && n < (1ll << 30) && r0 >= 0 && r1 >= r0 && r1 <= n, "hicgat_pairloss_sparse_fwd_bwd: bad n/r0/r1 (%lld,%lld,%lld)", (long long)n, (long long)r0, (long long)r1);
-    HICGAT_REQUIRE(coords && rowptr && (col || r0 == r1) && (tval || r0 == r1) && moments && workspace, "hicgat_pairloss_sparse_fwd_bwd: null pointer");
+    HICGAT_REQUIRE(coords && rowptr && (col || r0 == r1) && (tval || r0 == r1) && (moments || pmom) && workspace, "hicgat_pairloss_sparse_fwd_bwd: null pointer");
     HICGAT_REQUIRE((mode & ~63u) == 0, "hicgat_pairloss_sparse_fwd_bwd: unknown mode bits 0x%x", mode);
     const bool ws_clean = (mode & HICGAT_PAIR_WS_CLEAN) != 0;
     const bool sym = (mode & HICGAT_PAIR_SYMMETRIC) != 0;
     mode &= ~(HICGAT_PAIR_WS_CLEAN | HICGAT_PAIR_SYMMETRIC);
     if (mode & HICGAT_PAIR_MOMENTS) mode &= ~HICGAT_PAIR_MOMENTS_D;
     if ((mode & HICGAT_PAIR_MOMENTS_D) && (mode & HICGAT_PAIR_GRAD_L1)) mode = (mode & ~HICGAT_PAIR_MOMENTS_D) | HICGAT_PAIR_MOMENTS;
-    HICGAT_REQUIRE(!(mode & 3u) || grad || grad64, "hicgat_pairloss_sparse_fwd_bwd: grad is NULL but a gradient mode is set");
+    if (pmom) mode |= kPearson;
+    HICGAT_REQUIRE(!has_grad(mode) || grad || grad64, "hicgat_pairloss_sparse_fwd_bwd: grad is NULL but a gradient mode is set");
     const SparseLayout L = sparse_layout(n, r0, r1, sym);
     if (workspace_bytes < L.total) {
         set_error("hicgat_pairloss_sparse_fwd_bwd: workspace %zu < required %zu", workspace_bytes, L.total);
@@ -2115,7 +2198,7 @@ static int pairloss_sparse_impl(const float* coords, const int32_t* rowptr, cons
         HICGAT_CUDA(cudaMemsetAsync(ws + L.off_counter, 0, sizeof(unsigned), stream));  // ticket of pairloss_csr_fix_kernel
     }
     if (r1 == r0) {
-        HICGAT_CUDA(cudaMemsetAsync(moments, 0, sizeof(double) * kNM, stream));
+        if (moments) HICGAT_CUDA(cudaMemsetAsync(moments, 0, sizeof(double) * kNM, stream));
         if (grad) HICGAT_CUDA(cudaMemsetAsync(grad, 0, sizeof(float) * 3 * (size_t)n, stream));
         if (grad64) HICGAT_CUDA(cudaMemsetAsync(grad64, 0, sizeof(double) * 3 * (size_t)n, stream));
         return HICGAT_OK;
@@ -2125,6 +2208,7 @@ static int pairloss_sparse_impl(const float* coords, const int32_t* rowptr, cons
     P.n = (int)n; P.r0 = (int)r0; P.r1 = (int)r1; P.rb = L.dense.rb; P.nstrips = L.dense.nstrips; P.nchunks = L.dense.nchunks; P.stagger = L.dense.stagger; P.sch = L.dense.sch;
     P.fill = fill;
     P.c_mse = c_mse; P.c_l1 = c_l1; P.moments = moments; P.grad = grad; P.grad64 = grad64;
+    P.pmom = pmom; P.dyn_alpha = dyn_alpha;
     P.mpart = reinterpret_cast<double*>(ws + L.dense.off_mpart);
     P.gpart = reinterpret_cast<float*>(ws + L.dense.off_gpart);
     P.upper = sym ? 1 : 0; P.rpitch = L.dense.rpitch; P.rpart = reinterpret_cast<float*>(ws + L.dense.off_rpart);
@@ -2142,6 +2226,7 @@ static int pairloss_sparse_impl(const float* coords, const int32_t* rowptr, cons
 #define HICGAT_CASE(M) case M: err = launch_sparse<M>(P, grid, rowptr, col, tval, L.fix_ctas, part, counter, stream); break;
         HICGAT_CASE(0u) HICGAT_CASE(1u) HICGAT_CASE(2u) HICGAT_CASE(3u) HICGAT_CASE(4u)
         HICGAT_CASE(5u) HICGAT_CASE(6u) HICGAT_CASE(7u) HICGAT_CASE(8u) HICGAT_CASE(9u)
+        HICGAT_CASE(64u) HICGAT_CASE(65u)
 #undef HICGAT_CASE
         default:
             set_error("hicgat_pairloss_sparse_fwd_bwd: unsupported mode 0x%x", mode);
@@ -2159,6 +2244,40 @@ extern "C" int hicgat_pairloss_sparse_fwd_bwd(const float* coords, const int32_t
                                               int64_t n, int64_t r0, int64_t r1, uint32_t mode, float c_mse, float c_l1, double* moments,
                                               float* grad, void* workspace, size_t workspace_bytes, hicgat_stream_t stream) {
     return pairloss_sparse_impl(coords, rowptr, col, tval, fill, n, r0, r1, mode, c_mse, c_l1, moments, grad, nullptr, workspace, workspace_bytes, stream);
+}
+
+// ------------------------------------------------------------------ differentiable Pearson: second pass
+namespace {
+constexpr uint32_t kPearsonModeBits = HICGAT_PAIR_SYMMETRIC | HICGAT_PAIR_WS_CLEAN | HICGAT_PAIR_GRAD_MSE;
+int check_pearson_args(const char* what, uint32_t mode, const double* moments, const float* grad) {
+    if (!moments || !grad) {
+        set_error("%s: null moments / grad", what);
+        return HICGAT_ERR_INVALID;
+    }
+    if ((mode & ~kPearsonModeBits) != 0) {
+        set_error("%s: mode 0x%x: only HICGAT_PAIR_SYMMETRIC | HICGAT_PAIR_WS_CLEAN | HICGAT_PAIR_GRAD_MSE are accepted", what, mode);
+        return HICGAT_ERR_INVALID;
+    }
+    return HICGAT_OK;
+}
+}  // namespace
+
+extern "C" int hicgat_pairloss_pearson_grad(const float* coords, const float* target, int64_t pitch, int64_t n, int64_t r0, int64_t r1,
+                                            uint32_t mode, const double* moments, float c_mse, int dyn_alpha, float* grad, void* workspace,
+                                            size_t workspace_bytes, hicgat_stream_t stream) {
+    const int rc = check_pearson_args("hicgat_pairloss_pearson_grad", mode, moments, grad);
+    if (rc != HICGAT_OK) return rc;
+    return pairloss_impl(coords, target, pitch, n, r0, r1, mode, c_mse, 0.f, nullptr, grad, nullptr, workspace, workspace_bytes, stream, moments,
+                         dyn_alpha ? 1 : 0);
+}
+
+extern "C" int hicgat_pairloss_sparse_pearson_grad(const float* coords, const int32_t* rowptr, const int32_t* col, const float* tval, float fill,
+                                                   int64_t n, int64_t r0, int64_t r1, uint32_t mode, const double* moments, float c_mse,
+                                                   int dyn_alpha, float* grad, void* workspace, size_t workspace_bytes, hicgat_stream_t stream) {
+    const int rc = check_pearson_args("hicgat_pairloss_sparse_pearson_grad", mode, moments, grad);
+    if (rc != HICGAT_OK) return rc;
+    return pairloss_sparse_impl(coords, rowptr, col, tval, fill, n, r0, r1, mode, c_mse, 0.f, nullptr, grad, nullptr, workspace, workspace_bytes,
+                                stream, moments, dyn_alpha ? 1 : 0);
 }
 
 extern "C" int hicgat_pairdist_fwd(const float* coords, int64_t n, float* dist, int64_t pitch, hicgat_stream_t stream_) {

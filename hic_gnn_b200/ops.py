@@ -209,7 +209,7 @@ def pairloss_raw(coords: torch.Tensor, target: WishTarget, mode: int, c_mse: flo
             moments = torch.empty(N.PAIR_NMOM, dtype=torch.float64, device=coords.device)
         if grad is None and (mode & 3):
             grad = torch.empty(n, 3, dtype=torch.float32, device=coords.device)
-        ws = _PairWorkspace.get(coords.device, n, target.r0, target.r1, sparse=True)
+        ws = _PairWorkspace.get(coords.device, n, target.r0, target.r1, sparse=True, sym=_USE_UPPER)  # the layout depends on the mode
         rc = N.lib().hicgat_pairloss_sparse_fwd_bwd(
             coords.data_ptr(), target.rowptr.data_ptr(), target.col.data_ptr(), target.tval.data_ptr(), target.fill, n, target.r0, target.r1,
             mode | N.PAIR_WS_CLEAN | (N.PAIR_SYMMETRIC if _USE_UPPER else 0), c_mse, c_l1, moments.data_ptr(), _ptr(grad), ws.data_ptr(), ws.numel(), _stream(),
@@ -243,6 +243,43 @@ def pairloss_raw(coords: torch.Tensor, target: WishTarget, mode: int, c_mse: flo
     return moments, grad
 
 
+def pearson_grad_raw(coords: torch.Tensor, target, moments: torch.Tensor, with_mse: bool, grad=None) -> torch.Tensor:
+    """Second pass of the differentiable Pearson modes (``hicgat_pairloss_pearson_grad`` / ``_sparse_pearson_grad``): this row
+    block's contribution to the gradient of ``1 - r`` (``with_mse=False``) or of ``MSE + alpha (1 - r)`` with alpha held
+    constant (``with_mse=True``), from the GLOBAL f64 moments ``moments`` (pass 1 + the target constants), read on the device."""
+    _cuda(coords, moments)
+    n = target.n
+    if coords.dtype != torch.float32 or coords.shape != (n, 3):
+        raise RuntimeError(f"coords must be float32 [n,3] with n={n}, got {coords.dtype} {tuple(coords.shape)}")
+    if moments.dtype != torch.float64 or moments.numel() != N.PAIR_NMOM or not moments.is_contiguous():
+        raise RuntimeError("moments must be a contiguous float64 CUDA tensor of HICGAT_PAIR_NMOM elements")
+    coords = coords.contiguous()
+    if grad is None:
+        grad = torch.empty(n, 3, dtype=torch.float32, device=coords.device)
+    mode = N.PAIR_WS_CLEAN | (N.PAIR_GRAD_MSE if with_mse else 0)
+    c_mse = 4.0 / (float(n) * float(n))
+    if isinstance(target, SparseWishTarget):
+        ws = _PairWorkspace.get(coords.device, n, target.r0, target.r1, sparse=True, sym=_USE_UPPER)
+        rc = N.lib().hicgat_pairloss_sparse_pearson_grad(
+            coords.data_ptr(), target.rowptr.data_ptr(), target.col.data_ptr(), target.tval.data_ptr(), target.fill, n, target.r0, target.r1,
+            mode | (N.PAIR_SYMMETRIC if _USE_UPPER else 0), moments.data_ptr(), c_mse, int(with_mse), grad.data_ptr(), ws.data_ptr(), ws.numel(), _stream(),
+        )
+        N.check(rc, "hicgat_pairloss_sparse_pearson_grad")
+        return grad
+    _cuda(target.data)
+    if target.symmetric is False:
+        raise NotImplementedError("the differentiable Pearson gradient needs a symmetric target: t_ij != t_ji found when the target was built "
+                                  "(symmetrise it, e.g. (T + T.T)/2 or triu(T) + triu(T, 1).T, whichever the experiment means)")
+    sym = uses_upper_triangle(target)
+    ws = _PairWorkspace.get(coords.device, n, target.r0, target.r1, sym=sym)
+    rc = N.lib().hicgat_pairloss_pearson_grad(
+        coords.data_ptr(), target.data.data_ptr(), target.pitch, n, target.r0, target.r1, mode | (N.PAIR_SYMMETRIC if sym else 0),
+        moments.data_ptr(), c_mse, int(with_mse), grad.data_ptr(), ws.data_ptr(), ws.numel(), _stream(),
+    )
+    N.check(rc, "hicgat_pairloss_pearson_grad")
+    return grad
+
+
 def pearson_from_moments(m: torch.Tensor, npairs: float) -> torch.Tensor:
     """Pearson r of (d, t) over i<j from raw f64 moments (scipy.stats.pearsonr's value,
     HiC_GAT_generalize_directly.py:220)."""
@@ -253,11 +290,42 @@ def pearson_from_moments(m: torch.Tensor, npairs: float) -> torch.Tensor:
     return (cov / torch.sqrt(vd * vt)).clamp(-1.0, 1.0)
 
 
+# differentiable Pearson modes of pairwise_loss: pass 1 (moments) -> global moments -> pass 2 (gradient)
+_PEARSON_MODES = ("pearson", "mse_pearson_grad")
+
+
+def pearson_loss_from_moments(m: torch.Tensor, n: int, with_mse: bool) -> torch.Tensor:
+    """f64 value of ``1 - r`` (``with_mse=False``) or of ``MSE + alpha (1 - r)``, ``alpha = min(1, 0.1 + 1/(MSE + 1e-6))`` with
+    the f32 MSE (``with_mse=True``: the value of the ``mse_pearson`` training loss, HiC_GAT_generalize_directly.py:219-225).
+    r is NaN when ``v_d v_t <= 0`` or is not finite (n <= 2, coincident loci, a constant target), as scipy gives."""
+    npairs = n * (n - 1) / 2.0
+    vd = m[3] - m[2] * m[2] / npairs
+    vt = m[5] - m[4] * m[4] / npairs
+    prod = vd * vt
+    r = torch.where((prod > 0) & torch.isfinite(prod), pearson_from_moments(m, npairs), torch.full_like(prod, float("nan")))
+    if not with_mse:
+        return 1.0 - r
+    mse = (m[0] / (float(n) * float(n))).to(torch.float32).double()
+    alpha = torch.clamp(0.1 + 1.0 / (mse + 1e-6), max=1.0)
+    return mse + alpha * (1.0 - r)
+
+
 class _PairLossFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, coords, target, mode_name, reducer):
         n = target.n
         npairs = n * (n - 1) / 2.0
+        if mode_name in _PEARSON_MODES:
+            with_mse = mode_name == "mse_pearson_grad"
+            if reducer is not None:
+                moments, grad = reducer(coords.detach())
+            else:
+                moments, _ = pairloss_raw(coords.detach(), target, N.PAIR_MOMENTS_D, 0.0, 0.0)
+                moments = moments + target.t_moments()
+                grad = pearson_grad_raw(coords.detach(), target, moments, with_mse)
+            ctx.save_for_backward(grad)
+            ctx.mark_non_differentiable(moments)
+            return pearson_loss_from_moments(moments, n, with_mse), moments
         mode = _MODES[mode_name]
         c_mse, c_l1 = 4.0 / (float(n) * float(n)), 0.1 / max(npairs, 1.0)
         if reducer is not None:  # row-sharded: local block + one packed all-reduce (sharding.py)
@@ -286,19 +354,50 @@ def pairwise_loss(coords: torch.Tensor, target: WishTarget, mode: str = "mse", r
     mode ``"mse"``          MSELoss(cdist(coords), truth)            HiC-GNN_main.py:126-127
          ``"mse_moments"``  same + Pearson/L1 moments in one pass    HiC_GAT_generalize_directly.py:206-225
          ``"contrastive"``  0.1*mean_{i<j}|t-d| (f64)                train_and_test_same_res_GAT_node2vec.py:131-134
+         ``"pearson"``      1 - r over i<j (f64), with its gradient
+         ``"mse_pearson_grad"``  MSE + alpha (1 - r) (f64, the value of the mse_pearson training loss), alpha held constant
+                            and the gradient of BOTH terms (the reference's r is a float without one)
+    The two Pearson modes run two passes (moments, then the gradient from the global moments) and need a symmetric target.
     """
-    if mode not in ("mse", "mse_moments", "mse_moments_full", "contrastive"):
+    if mode not in ("mse", "mse_moments", "mse_moments_full", "contrastive") + _PEARSON_MODES:
         raise ValueError(mode)
     return _PairLossFn.apply(coords, target, mode, reducer)
 
 
 def sharded_reducer(target: WishTarget, mode: str, group=None, transport: str = "auto"):
     """``reducer`` for :func:`pairwise_loss` when ``target`` is this rank's row block.
-    ``transport``: see :func:`sharding.make_sharded_pair_loss`."""
+    ``transport``: see :func:`sharding.make_sharded_pair_loss` (the two-pass modes ``pearson`` / ``mse_pearson_grad`` take
+    ``"p2p"``, ``"nccl"`` or ``"auto"``)."""
+    import torch.distributed as dist
+
     from . import sharding
 
     n = target.n
     npairs = n * (n - 1) / 2.0
+    device = target.tval.device if isinstance(target, SparseWishTarget) else target.data.device
+    if mode in _PEARSON_MODES:
+        if transport == "p2p_oneshot":
+            raise NotImplementedError(f"mode {mode!r}: the one-shot p2p exchange is not extended to the two-pass modes (use 'p2p' or 'nccl')")
+        with_mse = mode == "mse_pearson_grad"
+
+        def moments_fn(coords, out):
+            pairloss_raw(coords, target, N.PAIR_MOMENTS_D, 0.0, 0.0, moments=out)
+
+        def grad_fn(coords, moments, grad=None):
+            return pearson_grad_raw(coords, target, moments.contiguous(), with_mse, grad=grad)
+
+        const = sharding.allreduce_packed(target.t_moments().clone(), group)
+        multi = dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
+        if transport == "p2p" or (transport == "auto" and multi and device.type == "cuda"):
+            try:
+                return sharding.P2PTwoPassShardedPairLoss(n, moments_fn, grad_fn, device, group, moment_const=const)
+            except Exception as e:  # no symmetric memory on this system: the NCCL exchange is equivalent
+                if transport == "p2p":
+                    raise
+                import warnings
+
+                warnings.warn(f"symmetric-memory exchange unavailable ({e!r}); using two NCCL all-reduces")
+        return sharding.TwoPassShardedPairLoss(n, moments_fn, grad_fn, device, group, moment_const=const)
     m = _MODES[mode]
     c_mse, c_l1 = 4.0 / (float(n) * float(n)), 0.1 / max(npairs, 1.0)
     fn = sharding.cuda_local_fn(target, m, c_mse, c_l1)
@@ -306,7 +405,6 @@ def sharded_reducer(target: WishTarget, mode: str, group=None, transport: str = 
     const = None
     if m & N.PAIR_MOMENTS_D and not m & N.PAIR_MOMENTS:
         const = sharding.allreduce_packed(target.t_moments().clone(), group)  # global sum t, sum t^2: once
-    device = target.tval.device if isinstance(target, SparseWishTarget) else target.data.device
     return sharding.make_sharded_pair_loss(n, fn, device, group, moment_const=const, transport=transport, local_split_fn=split_fn)
 
 

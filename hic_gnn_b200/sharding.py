@@ -120,6 +120,30 @@ class ShardedPairLoss:
         return moments, grad
 
 
+class TwoPassShardedPairLoss:
+    """Same contract as :class:`ShardedPairLoss` for the differentiable Pearson modes, whose gradient needs the GLOBAL
+    moments: ``moments_fn(coords, moments_f64[8])`` fills this block's pass-1 moments, one ``all_reduce`` sums them (plus
+    ``moment_const``, the target-only sums), ``grad_fn(coords, global_moments) -> grad_f32[n,3]`` is this block's pass-2
+    gradient, and a second ``all_reduce`` (f64) sums that.  Backend-agnostic (NCCL, or gloo with CPU stand-ins in the
+    tests); not capturable in a CUDA graph."""
+
+    capturable = False
+
+    def __init__(self, n: int, moments_fn, grad_fn, device, group=None, moment_const=None):
+        self.n, self.moments_fn, self.grad_fn, self.group = n, moments_fn, grad_fn, group
+        self.moments = torch.zeros(N.PAIR_NMOM, dtype=torch.float64, device=device)
+        self.gbuf = torch.zeros(3 * n, dtype=torch.float64, device=device)
+        self.moment_const = moment_const
+
+    def __call__(self, coords: torch.Tensor):
+        self.moments_fn(coords, self.moments)
+        allreduce_packed(self.moments, self.group)
+        moments = self.moments if self.moment_const is None else self.moments + self.moment_const
+        self.gbuf.copy_(self.grad_fn(coords, moments).reshape(-1))
+        allreduce_packed(self.gbuf, self.group)
+        return moments, self.gbuf.view(self.n, 3).to(torch.float32)
+
+
 class P2PShardedPairLoss:
     """Same contract as :class:`ShardedPairLoss`, but the exchange is the hand-written two-shot all-reduce over
     NVLink peer memory (``hicgat_allreduce_partials_twoshot``, csrc/comm.cu): the fused loss kernel writes its partial
@@ -187,6 +211,67 @@ class P2PShardedPairLoss:
         )
         N.check(rc, "hicgat_allreduce_partials_p2p")
         return m, g
+
+
+class P2PTwoPassShardedPairLoss:
+    """:class:`TwoPassShardedPairLoss` over NVLink peer memory: both exchanges are the two-shot kernel
+    (``hicgat_allreduce_partials_twoshot``), so the whole sharded step -- pass 1, moments exchange, pass 2, gradient exchange --
+    has identical launch arguments every step and can be captured in a CUDA graph (``capturable``).
+    The moments exchange is a two-shot all-reduce of a moments-only partial (``n = 1``: the 16-byte gradient part stays zero);
+    the gradient exchange reduces a partial whose moment part stays zero.  Each has its own state array and signal-slot range.
+    ``moments_fn(coords, moments_f64[8])`` fills this block's pass-1 moments in place, ``grad_fn(coords, global_moments, grad_f32[n,3])``
+    this block's pass-2 gradient in place.  The returned moments / gradient are views of the result buffers: valid until the next call."""
+
+    SLOT_BASE = P2PShardedPairLoss.SLOT_BASE
+    SLOTS_MOMENTS = SLOT_BASE + 64   # two-shot barriers use 2 x 16 slots from their base
+    SLOTS_GRAD = SLOT_BASE + 96
+    capturable = True
+
+    def __init__(self, n: int, moments_fn, grad_fn, device, group=None, moment_const=None):
+        import ctypes as C
+
+        import torch.distributed._symmetric_memory as symm
+
+        group = group if group is not None else dist.group.WORLD
+        self.n, self.moments_fn, self.grad_fn = n, moments_fn, grad_fn
+        grad_bytes = (12 * n + 15) // 16 * 16
+        # layout: [moments partial: 64 + 16 | moments result: 16 | gradient partial: 64 + grad_bytes | gradient result: grad_bytes]
+        self.m_part, self.m_res = 0, 80
+        self.g_part = 96
+        self.g_res = self.g_part + 64 + grad_bytes
+        self.buf = symm.empty(self.g_res + grad_bytes, dtype=torch.uint8, device=device)
+        self.buf.zero_()
+        self.hdl = symm.rendezvous(self.buf, group)
+        self.world, self.rank = self.hdl.world_size, self.hdl.rank
+        if self.hdl.signal_pad_size < 4 * (self.SLOTS_GRAD + 32):
+            raise RuntimeError("symmetric-memory signal pad too small")
+        ptrs = [int(p) for p in self.hdl.buffer_ptrs]
+        table = lambda off: (C.c_uint64 * self.world)(*[p + off for p in ptrs])
+        self._m_bufs, self._m_res = table(self.m_part), table(self.m_res)
+        self._g_bufs, self._g_res = table(self.g_part), table(self.g_res)
+        self._pads = (C.c_uint64 * self.world)(*[int(p) for p in self.hdl.signal_pad_ptrs])
+        self.moment_const = moment_const
+        self.part_m = self.buf[self.m_part: self.m_part + 64].view(torch.float64)
+        self.part_g = self.buf[self.g_part + 64: self.g_part + 64 + 12 * n].view(torch.float32).view(n, 3)
+        self.res_g = self.buf[self.g_res: self.g_res + 12 * n].view(torch.float32).view(n, 3)
+        self.out_m = torch.empty(N.PAIR_NMOM, dtype=torch.float64, device=device)
+        self.scratch_m = torch.empty(N.PAIR_NMOM, dtype=torch.float64, device=device)  # the gradient exchange's (zero) moment sum
+        self.state_m = torch.zeros(4, dtype=torch.int32, device=device)
+        self.state_g = torch.zeros(4, dtype=torch.int32, device=device)
+        torch.cuda.synchronize(device)
+        dist.barrier(group)  # every rank's buffer is zeroed and mapped before the first signal
+
+    def __call__(self, coords: torch.Tensor):
+        lib, stream = N.lib(), torch.cuda.current_stream().cuda_stream
+        self.moments_fn(coords, self.part_m)
+        N.check(lib.hicgat_allreduce_partials_twoshot(self._m_bufs, self._m_res, self._pads, self.rank, self.world, 1, self.SLOTS_MOMENTS,
+                                                      self.state_m.data_ptr(), None if self.moment_const is None else self.moment_const.data_ptr(),
+                                                      self.out_m.data_ptr(), stream), "hicgat_allreduce_partials_twoshot")
+        self.grad_fn(coords, self.out_m, self.part_g)
+        N.check(lib.hicgat_allreduce_partials_twoshot(self._g_bufs, self._g_res, self._pads, self.rank, self.world, self.n, self.SLOTS_GRAD,
+                                                      self.state_g.data_ptr(), None, self.scratch_m.data_ptr(), stream),
+                "hicgat_allreduce_partials_twoshot")
+        return self.out_m, self.res_g
 
 
 def make_sharded_pair_loss(n: int, local_fn, device, group=None, moment_const=None, transport: str = "auto", local_split_fn=None):

@@ -10,6 +10,9 @@ loss+gradient launch over the f32 target, backward through the conv kernels, Ada
   ``"mse"``          total = MSE                                       (HiC-GNN_main.py:127)
   ``"mse_pearson"``  total = MSE + min(1, 0.1 + 1/(MSE+1e-6)) (1 - r)  (HiC_GAT_generalize_directly.py:219-225;
                      r is a constant w.r.t. autograd in the reference, so the gradient is MSE's)
+  ``"mse_pearson_grad"``  the same total as ``"mse_pearson"``, but the (1 - r) term carries its gradient (alpha held
+                     constant): two passes per step (moments, then the gradient from the global moments), no host read,
+                     graph-capturable, also sharded over the p2p exchange (ops.sharded_reducer, transport "p2p" / "auto")
   ``"contrastive"``  total = 0.1 mean_{i<j} |t - d|                    (train_and_test_same_res_GAT_node2vec.py:131-134)
   ``"mse_spearman"`` total = MSE + alpha (1 - dSCC), fixed alpha       (combined_loss_training.py:119-142; the Spearman
                      term is a scipy value in the reference, i.e. a constant for autograd: the gradient is MSE's.  The
@@ -22,7 +25,8 @@ from torch.optim import Adam
 
 from .ops import WishTarget, pairwise_loss, pearson_from_moments
 
-_KERNEL_MODE = {"mse": "mse", "mse_pearson": "mse_moments", "contrastive": "contrastive", "mse_spearman": "mse_moments"}
+_KERNEL_MODE = {"mse": "mse", "mse_pearson": "mse_moments", "mse_pearson_grad": "mse_pearson_grad", "contrastive": "contrastive",
+                "mse_spearman": "mse_moments"}
 
 
 def drmsd_from_moments(moments: torch.Tensor, n: int) -> torch.Tensor:
@@ -34,7 +38,7 @@ def step_loss(model, x, graph, target: WishTarget, mode: str, reducer=None, alph
     """Forward + fused loss; returns (differentiable loss, total value tensor, moments)."""
     coords = model.get_model(x, graph)
     loss, moments = pairwise_loss(coords, target, _KERNEL_MODE[mode], reducer)
-    total = loss.detach()
+    total = loss.detach()  # mse_pearson_grad: the f64 total from the same moments as the gradient
     if mode == "mse_spearman":
         from . import metrics
 

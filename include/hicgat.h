@@ -162,6 +162,32 @@ HICGAT_API int hicgat_pairloss_sparse_fwd_bwd(const float* coords, const int32_t
                                    void* workspace, size_t workspace_bytes, hicgat_stream_t stream);
 
 /* ------------------------------------------------------------------------------------
+ * Differentiable Pearson term (loss 1 - r over the pairs i<j, P = n(n-1)/2), second pass.  The gradient needs the
+ * GLOBAL moments, so one training step is: pass 1 = hicgat_pairloss_fwd_bwd / _sparse_fwd_bwd with HICGAT_PAIR_MOMENTS_D
+ * and no gradient bit, + the target constants sum t / sum t^2 (slots 4, 5 of a HICGAT_PAIR_MOMENTS launch), summed over
+ * ranks when sharded; then this call, which reads that f64[HICGAT_PAIR_NMOM] vector `moments` ON THE DEVICE (no host
+ * read: the step stays capturable in a CUDA graph) and writes this rank's gradient contribution for all n loci:
+ *   v_d = S_dd - S_d^2/P, v_t = S_tt - S_t^2/P, c = S_dt - S_d S_t/P, beta = c/v_d, kappa = S_t/P - beta S_d/P,
+ *   A = -1/sqrt(v_d v_t),  rho_ij = t_ij - (beta d_ij + kappa)  (the residual of the regression of t on d)
+ *   grad_j = sum_{i != j} [ c_mse (d - t) + lambda A rho ] / d * (x_j - x_i)
+ * with c_mse applied only when mode has HICGAT_PAIR_GRAD_MSE, and lambda = 1, or with dyn_alpha != 0
+ * lambda = min(1, 0.1 + 1/(MSE + 1e-6)), MSE = moments[0]/n^2 rounded to f32 (the MSE + alpha (1 - r) loss).
+ * Degenerate moments (v_d v_t <= 0 or not finite: n <= 2, coincident loci, a constant target) give a zero Pearson
+ * weight (r is NaN there); the MSE part is unchanged.
+ * mode: only HICGAT_PAIR_SYMMETRIC, HICGAT_PAIR_WS_CLEAN and HICGAT_PAIR_GRAD_MSE (anything else, or a NULL moments /
+ * grad pointer, is HICGAT_ERR_INVALID).  The target must be symmetric: there is no row-side pass for t_ij != t_ji.
+ * Workspaces as for hicgat_pairloss_fwd_bwd / hicgat_pairloss_sparse_fwd_bwd (the same buffer as pass 1 may be used).
+ * ---------------------------------------------------------------------------------- */
+HICGAT_API int hicgat_pairloss_pearson_grad(const float* coords, const float* target, int64_t pitch, int64_t n, int64_t r0,
+                                 int64_t r1, uint32_t mode, const double* moments, float c_mse, int dyn_alpha,
+                                 float* grad, void* workspace, size_t workspace_bytes, hicgat_stream_t stream);
+HICGAT_API int hicgat_pairloss_sparse_pearson_grad(const float* coords, const int32_t* rowptr, const int32_t* col,
+                                        const float* tval, float fill, int64_t n, int64_t r0, int64_t r1,
+                                        uint32_t mode, const double* moments, float c_mse, int dyn_alpha,
+                                        float* grad, void* workspace, size_t workspace_bytes,
+                                        hicgat_stream_t stream);
+
+/* ------------------------------------------------------------------------------------
  * Non-symmetric targets.  The fused kernels above take the column-side sum as the complete gradient,
  * which needs t_ij = t_ji; the reference does not symmetrise `y` (utils.py:29-35, MSELoss over the full
  * matrix at HiC-GNN_main.py:127; convert_to_matrix's triu + tril(mat.T, 1), utils.py:21, is asymmetric on
