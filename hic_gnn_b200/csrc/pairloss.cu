@@ -20,7 +20,7 @@
 //   waits on a global load it issued itself and 2 CTAs x 8 warps x 3 x 4 KB = 192 KB of target
 //   are in flight per SM.  TMA zero-fills columns >= n and rows >= r1-r0 (no edge address logic).
 // Variant 1 ("ldg"): each lane issues 8 streaming 128-bit ld.global.nc per row group; kept for
-//   A/B measurements and as the path used when a tensor map cannot be encoded.
+//   A/B measurements and as the path used when a tensor map cannot be encoded.  Same triangle modes.
 #include <cuda.h>  // CUtensorMap (types only; the encoder is resolved through cudart at run time)
 
 #include <stdlib.h>
@@ -709,9 +709,17 @@ __global__ void __launch_bounds__(kCombineThreads, 2) pairloss_combine_kernel(co
 #endif
 }
 
-// ------------------------------------------------------------------ variant 1: per-lane streaming loads
-template <uint32_t MODE>
-__global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_ldg_kernel(const Params P) {
+// ------------------------------------------------------------------ variant 1 and the implicit target: per-lane target values
+// One CTA per (strip, row chunk), the chunk's x_i staged in shared memory; every lane takes its 4 target values of a row group
+//   IMPLICIT = false (variant 1): from the target, with streaming 128-bit ld.global.nc loads (8 per group);
+//   IMPLICIT = true  (implicit target, SURVEY.md section 8 row f-4): from nowhere -- on a sparse map every non-edge pair has wish
+//     distance `fill` (1.0 after cont2dist: zero contacts map to max/max, utils.py:78-80) and the diagonal 0, so the N x N target
+//     need not exist.  The loss against that constant background is FP32 / MUFU bound instead of HBM bound;
+//     pairloss_csr_fix_kernel then corrects the nnz pairs that do carry a contact.
+// ROWS: upper-triangle mode (chunk_rows clips every strip at its last column, so no row below the diagonal strip is loaded).
+// Same decomposition, arithmetic and reductions as the TMA kernels.
+template <uint32_t MODE, bool ROWS, bool IMPLICIT>
+__global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_lane_kernel(const Params P) {
     pdl_launch_dependents();
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float4* s_xy = reinterpret_cast<float4*>(smem_raw);                          // [rb] (x,x,y,y)
@@ -726,7 +734,6 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_ldg_kernel(cons
     const int count = chunk_rows(P, strip, chunk, row_begin, nrows);
     if (chunk >= count || nrows <= 0) return;  // unstaggered strips leave the extra chunk slot empty
     const bool edge = (strip + 1) * kCols > n;
-
     for (int r = threadIdx.x; r < nrows; r += kThreads) {
         const float* c = P.coords + (size_t)(row_begin + r) * 3;
         float x = c[0], y = c[1], z = c[2];
@@ -739,66 +746,8 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_ldg_kernel(cons
     acc_zero(a);
     const PearsonCoef pc = pearson_coef<MODE>(P.pmom, n, P.c_mse, P.dyn_alpha);
     __syncthreads();
-
-    const bool can_load = col0 + 3 < P.pitch;  // pitch is a multiple of 4
+    const bool can_load = col0 + 3 < P.pitch;  // pitch is a multiple of 4 (0 for the implicit target)
     const float* tbase = P.target + (size_t)(row_begin - P.r0) * P.pitch + col0;
-    const int strip_lo = strip * kCols, strip_hi = strip_lo + kCols - 1;
-    const int ngroups = (nrows + kU - 1) / kU;
-
-    for (int g = warp; g < ngroups; g += kWarps) {
-        const int rl = g * kU;
-        const int rows_here = min(kU, nrows - rl);
-        float4 t[kU];
-        if (rows_here == kU && can_load) {
-#pragma unroll
-            for (int u = 0; u < kU; ++u) t[u] = ldg_stream_f4(tbase + (size_t)(rl + u) * P.pitch);
-        } else {
-#pragma unroll
-            for (int u = 0; u < kU; ++u)
-                t[u] = (u < rows_here && can_load) ? ldg_stream_f4(tbase + (size_t)(rl + u) * P.pitch)
-                                                   : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-        process_group<MODE, false>(a, c, t, XiPtr{s_xy + rl, s_z + rl}, rows_here, row_begin + rl, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1, nullptr, lane, pc);
-    }
-    park_warp<MODE>(a, S, warp, lane);
-    __syncthreads();
-    publish_cta<MODE>(P, S, strip, chunk, threadIdx.x, kThreads);
-}
-
-// ------------------------------------------------------------------ implicit target, dense part (compute only)
-// SURVEY.md section 8 row f-4: on a sparse map every non-edge pair has wish distance `fill` (1.0 after
-// cont2dist: zero contacts map to max/max, utils.py:78-80) and the diagonal 0, so the N x N target need
-// not exist.  This kernel evaluates the loss against that constant background with no target loads at
-// all (FP32 / MUFU bound instead of HBM bound); pairloss_csr_fix_kernel then corrects the nnz pairs
-// that do carry a contact.  Same decomposition, arithmetic and reductions as the streamed kernels.
-template <uint32_t MODE, bool ROWS>
-__global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_const_kernel(const Params P) {
-    pdl_launch_dependents();
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    float4* s_xy = reinterpret_cast<float4*>(smem_raw);                          // [rb] (x,x,y,y)
-    float2* s_z = reinterpret_cast<float2*>(smem_raw + sizeof(float4) * P.rb);   // [rb] (z,z)
-    __shared__ CombineSmem S;
-
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int strip = blockIdx.x, chunk = blockIdx.y;
-    const int n = P.n;
-    const int col0 = strip * kCols + lane * 4;
-    int row_begin, nrows;
-    const int count = chunk_rows(P, strip, chunk, row_begin, nrows);
-    if (chunk >= count || nrows <= 0) return;
-    const bool edge = (strip + 1) * kCols > n;
-    for (int r = threadIdx.x; r < nrows; r += kThreads) {
-        const float* c = P.coords + (size_t)(row_begin + r) * 3;
-        float x = c[0], y = c[1], z = c[2];
-        s_xy[r] = make_float4(x, x, y, y);
-        s_z[r] = make_float2(z, z);
-    }
-    ColumnRegs c;
-    load_columns(c, P.coords, col0, n);
-    Acc a;
-    acc_zero(a);
-    const PearsonCoef pc = pearson_coef<MODE>(P.pmom, n, P.c_mse, P.dyn_alpha);
-    __syncthreads();
     const int strip_lo = strip * kCols, strip_hi = strip_lo + kCols - 1;
     const int ngroups = (nrows + kU - 1) / kU;
     const float f = P.fill;
@@ -806,16 +755,27 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_const_kernel(co
         const int rl = g * kU, rg = row_begin + rl;
         const int rows_here = min(kU, nrows - rl);
         float4 t[kU];
+        if constexpr (IMPLICIT) {
 #pragma unroll
-        for (int u = 0; u < kU; ++u) t[u] = make_float4(f, f, f, f);
-        if (rg + kU - 1 >= strip_lo && rg <= strip_hi) {  // the group touches the diagonal: t_ii = 0
+            for (int u = 0; u < kU; ++u) t[u] = make_float4(f, f, f, f);
+            if (rg + kU - 1 >= strip_lo && rg <= strip_hi) {  // the group touches the diagonal: t_ii = 0
 #pragma unroll
-            for (int u = 0; u < kU; ++u) {
-                const int dc = rg + u - col0;
-                if (dc == 0) t[u].x = 0.f;
-                if (dc == 1) t[u].y = 0.f;
-                if (dc == 2) t[u].z = 0.f;
-                if (dc == 3) t[u].w = 0.f;
+                for (int u = 0; u < kU; ++u) {
+                    const int dc = rg + u - col0;
+                    if (dc == 0) t[u].x = 0.f;
+                    if (dc == 1) t[u].y = 0.f;
+                    if (dc == 2) t[u].z = 0.f;
+                    if (dc == 3) t[u].w = 0.f;
+                }
+            }
+        } else {
+            if (rows_here == kU && can_load) {
+#pragma unroll
+                for (int u = 0; u < kU; ++u) t[u] = ldg_stream_f4(tbase + (size_t)(rl + u) * P.pitch);
+            } else {
+#pragma unroll
+                for (int u = 0; u < kU; ++u)
+                    t[u] = (u < rows_here && can_load) ? ldg_stream_f4(tbase + (size_t)(rl + u) * P.pitch) : make_float4(0.f, 0.f, 0.f, 0.f);
             }
         }
         process_group<MODE, ROWS>(a, c, t, XiPtr{s_xy + rl, s_z + rl}, rows_here, rg, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1,
@@ -1932,7 +1892,8 @@ cudaError_t launch_mode(int variant, const CUtensorMap& map, const Params& P, di
         e = P.upper ? launch_tma<MODE, true>(map, P, grid, stream) : launch_tma<MODE, false>(map, P, grid, stream);
     } else {
         const size_t smem = (sizeof(float4) + sizeof(float2)) * (size_t)P.rb;
-        pairloss_ldg_kernel<MODE><<<grid, kThreads, smem, stream>>>(P);
+        if (P.upper) pairloss_lane_kernel<MODE, true, false><<<grid, kThreads, smem, stream>>>(P);
+        else pairloss_lane_kernel<MODE, false, false><<<grid, kThreads, smem, stream>>>(P);
         e = cudaGetLastError();
     }
     if (e != cudaSuccess) return e;
@@ -2032,7 +1993,7 @@ extern "C" size_t hicgat_pairloss_workspace_bytes(int64_t n, int64_t r0, int64_t
 extern "C" size_t hicgat_pairloss_workspace_bytes_mode(int64_t n, int64_t r0, int64_t r1, uint32_t mode) {
     if (n <= 0 || r0 < 0 || r1 < r0 || r1 > n) return 0;
     const bool sym = (mode & HICGAT_PAIR_SYMMETRIC) != 0;
-    const size_t a = make_layout(n, r0, r1, 0, sym).total, b = make_layout(n, r0, r1, 1).total, c = make_layout(n, r0, r1, 3, sym).total,
+    const size_t a = make_layout(n, r0, r1, 0, sym).total, b = make_layout(n, r0, r1, 1, sym).total, c = make_layout(n, r0, r1, 3, sym).total,
                  d = make_layout(n, r0, r1, 4, sym).total;
     return std::max(std::max(a, d), std::max(b, c));
 }
@@ -2050,7 +2011,7 @@ static int pairloss_impl(const float* coords, const float* target, int64_t pitch
     HICGAT_REQUIRE((mode & ~63u) == 0, "hicgat_pairloss_fwd_bwd: unknown mode bits 0x%x", mode);
     const bool ws_clean = (mode & HICGAT_PAIR_WS_CLEAN) != 0;  // the persistent variant keeps ONE item counter in the workspace (left at zero by every call)
     mode &= ~HICGAT_PAIR_WS_CLEAN;
-    bool sym = (mode & HICGAT_PAIR_SYMMETRIC) != 0;
+    const bool sym = (mode & HICGAT_PAIR_SYMMETRIC) != 0;
     mode &= ~HICGAT_PAIR_SYMMETRIC;
     if (mode & HICGAT_PAIR_MOMENTS) mode &= ~HICGAT_PAIR_MOMENTS_D;          // full moments include the light set
     if ((mode & HICGAT_PAIR_MOMENTS_D) && (mode & HICGAT_PAIR_GRAD_L1)) {     // the L1 value needs sum |d-t|: full set
@@ -2060,8 +2021,8 @@ static int pairloss_impl(const float* coords, const float* target, int64_t pitch
     HICGAT_REQUIRE(!has_grad(mode) || grad || grad64, "hicgat_pairloss_fwd_bwd: grad is NULL but a gradient mode is set");
     int variant = g_variant;
     CUtensorMap map;
+    // a target no tensor map can be encoded for goes through the per-lane-load kernel (same sums, either triangle mode)
     if (variant != 1 && r1 > r0 && !make_target_map(&map, target, pitch, n, r1 - r0)) variant = 1;
-    if (variant == 1) sym = false;  // the per-lane-load variant streams the whole row block (A/B path; same results)
     const Layout L = make_layout(n, r0, r1, variant, sym);
     if (workspace_bytes < L.total) {
         set_error("hicgat_pairloss_fwd_bwd: workspace %zu < required %zu", workspace_bytes, L.total);
@@ -2074,6 +2035,8 @@ static int pairloss_impl(const float* coords, const float* target, int64_t pitch
         if (grad64) HICGAT_CUDA(cudaMemsetAsync(grad64, 0, sizeof(double) * 3 * (size_t)n, stream));
         return HICGAT_OK;
     }
+    // the combine kernel writes no gradient in a mode without one: the packed buffer is all-reduced whole, so it gets zeros
+    if (grad64 && !has_grad(mode)) HICGAT_CUDA(cudaMemsetAsync(grad64, 0, sizeof(double) * 3 * (size_t)n, stream));
     Params P;
     P.coords = coords; P.target = target; P.pitch = pitch;
     P.n = (int)n; P.r0 = (int)r0; P.r1 = (int)r1; P.rb = L.rb; P.nstrips = L.nstrips; P.nchunks = L.nchunks; P.stagger = L.stagger; P.sch = L.sch;
@@ -2156,8 +2119,8 @@ template <uint32_t MODE>
 cudaError_t launch_sparse(const Params& P, dim3 grid, const int32_t* rowptr, const int32_t* col, const float* tval, int fix_ctas, double* part,
                           unsigned* counter, cudaStream_t stream) {
     const size_t smem = (sizeof(float4) + sizeof(float2)) * (size_t)P.rb;
-    if (P.upper) pairloss_const_kernel<MODE, true><<<grid, kThreads, smem, stream>>>(P);
-    else pairloss_const_kernel<MODE, false><<<grid, kThreads, smem, stream>>>(P);
+    if (P.upper) pairloss_lane_kernel<MODE, true, true><<<grid, kThreads, smem, stream>>>(P);
+    else pairloss_lane_kernel<MODE, false, true><<<grid, kThreads, smem, stream>>>(P);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     e = launch_combine<MODE>(P, stream);

@@ -641,6 +641,10 @@ class HostPairLoss:
     previous block (copy stream / compute stream, events), partial moments and gradients are
     summed on the device and read back once.  This is the end-to-end path ``bench.py`` times
     (``e2e``): PCIe-bound by construction; a training loop keeps the target resident instead.
+
+    The gradient is the column-side sum of the fused kernel, complete only for a symmetric target (``t_ij == t_ji``), in both
+    modes: an asymmetric host target is not supported.  ``symmetric=True`` only selects the upper-triangle upload (columns from
+    each block's diagonal 128-column strip on); the columns left of it are never uploaded and never enter the result.
     """
 
     def __init__(self, n: int, r0: int = 0, r1: int | None = None, block_rows: int = 2048, device="cuda", reduce=None, symmetric: bool = False):
@@ -668,6 +672,9 @@ class HostPairLoss:
         assert not coords_host.is_cuda and not target_host.is_cuda
         assert target_host.shape == (self.r1 - self.r0, self.pitch) and target_host.dtype == torch.float32
         main = torch.cuda.current_stream()
+        # the first two blocks of a call write the staging buffers without waiting on a `free` event: order them after
+        # whatever the caller queued on its stream (work that still reads or writes that memory)
+        self.copy_stream.wait_stream(main)
         self.coords_dev.copy_(coords_host, non_blocking=True)
         self.acc.zero_()
         self.h2d_bytes = coords_host.numel() * 4

@@ -97,8 +97,11 @@ HICGAT_API int hicgat_memcpy2d_h2d_async(void* dst_device, size_t dst_pitch_byte
  * upper triangle (column >= row) of rows [r0,r1) is streamed -- 2 B per ordered pair instead of 4 -- and every
  * unordered pair is evaluated once: its weight feeds the column-side sum of locus j AND the row-side sum of locus i
  * (per-CTA row partials, reduced in strip order by the combine kernel: still bit-reproducible, no atomics).
- * Same results as without the bit up to f32 summation order; the lower triangle is never read (it may even be absent
- * from the buffer: the host-buffer path copies only the upper part).  Needs the workspace size of
+ * Same results as without the bit up to f32 summation order.  What is read of row i: entries in columns left of
+ * 128*floor(i/128) (the start of the row's 128-column strip) never enter the result and may hold anything, NaN included
+ * (the host-buffer path copies only the columns from that strip on); the entries below the diagonal INSIDE that strip are
+ * loaded and cancelled by a weight of 0, so they must be finite.  The buffer still spans the full pitch of every row.
+ * Every kernel variant honours this.  Needs the workspace size of
  * hicgat_pairloss_workspace_bytes_mode(n, r0, r1, mode).  Row blocks of a sharded run should then be balanced by
  * upper-triangle area, not by row count. */
 #define HICGAT_PAIR_SYMMETRIC 32u
@@ -116,13 +119,15 @@ HICGAT_API int hicgat_pairloss_fwd_bwd(const float* coords, const float* target,
                             hicgat_stream_t stream);
 /* Row-sharded variant: one f64 buffer packed[HICGAT_PAIR_NMOM + 3n] = [moments | grad] so that
  * a single all-reduce(sum) over NVLink combines the ranks (grad values are the f32 results,
- * widened). */
+ * widened).  Every element is written by every call: in a mode without a gradient bit, and for an
+ * empty row block, the gradient part is zero. */
 HICGAT_API int hicgat_pairloss_fwd_bwd_packed(const float* coords, const float* target, int64_t pitch,
                                    int64_t n, int64_t r0, int64_t r1, uint32_t mode, float c_mse,
                                    float c_l1, double* packed, void* workspace,
                                    size_t workspace_bytes, hicgat_stream_t stream);
 /* Tuning hook (bench/tests): rows per CTA row-chunk (0 = library default) and kernel variant:
- * 0 = TMA tile ring (cp.async.bulk.tensor + mbarrier), one CTA per (strip, row chunk); 1 = per-lane streaming loads;
+ * 0 = TMA tile ring (cp.async.bulk.tensor + mbarrier), one CTA per (strip, row chunk); 1 = per-lane streaming loads (also taken
+ * when no tensor map can be encoded for the target);
  * 2 = TMA tile ring without the half-chunk stagger of the second CTA slot (A/B only); 3 = the same ring in PERSISTENT CTAs that
  * pull (chunk, strip) items from an atomic queue and prefetch the next item's tiles across the item boundary; 4 = static warp
  * partition: the block's (strip, row) work is cut into equal runs, one per resident warp (no dispatch, no CTA-level
