@@ -10,11 +10,15 @@
     dSCC of the generalised structure      metrics.dscc                                  :335
     PDB file                               utils.WritePDB(coords * 100, ...)             :365
 
-The contact lists come from tests/golden (copies of the reference's Data/ fixtures recorded by make_golden.py); node2vec
-embeddings are replaced by seeded stand-ins (node2vec / gensim are not part of the hot path): the 500 kb stand-ins are a
-rotated, noisy interleaving of the 1 Mb ones, so that the alignment has something to recover.
+The contact lists come from tests/golden (copies of the reference's Data/ fixtures recorded by make_golden.py).
+``--features node2vec`` embeds each resolution's own graph with the reference's node2vec call (``Node2Vec(dimensions=512,
+walk_length=150, num_walks=50, p=1.75, q=0.4, seed=42).fit()``, HiC_GAT_generalize_directly.py:153-155, on the GPU through
+hic_gnn_b200.node2vec) and aligns the 500 kb embeddings onto the 1 Mb ones with ``domain_alignment``: the reference's flow.
+``--features random`` (default) uses seeded stand-ins instead: the 500 kb stand-ins are a rotated, noisy interleaving of the
+1 Mb ones, so that the alignment has something to recover.
 
-    python examples/chr19_generalize.py [--steps 300] [--loss mse_pearson|mse_pearson_grad] [--out /tmp/chr19_500kb_generalized_structure.pdb]
+    python examples/chr19_generalize.py [--steps 300] [--loss mse_pearson|mse_pearson_grad] [--features random|node2vec]
+                                        [--out /tmp/chr19_500kb_generalized_structure.pdb]
 
 ``--loss mse_pearson`` (default) is the reference's loss, whose Pearson term carries no gradient; ``mse_pearson_grad`` trains
 on the same total with the gradient of the (1 - r) term as well.
@@ -30,13 +34,29 @@ sys.path.insert(0, ROOT)
 import numpy as np
 import torch
 
-from hic_gnn_b200 import kr, metrics, models, train, utils
+from hic_gnn_b200 import kr, metrics, models, node2vec, train, utils
 
 
 def normed_map(contacts):
     raw = utils.convert_to_matrix(contacts)
     raw.fill_diagonal_(0)                               # HiC_GAT_generalize_directly.py:118
     return kr.kr_norm(raw)                              # replaces the Rscript subprocess
+
+
+def node2vec_features(normed):
+    graph = utils.load_input(normed, torch.zeros(normed.shape[0], 1)).edge_index
+    model = node2vec.Node2Vec(graph, dimensions=512, walk_length=150, num_walks=50, p=1.75, q=0.4, workers=1, seed=42)  # :153-154
+    return model.fit().wv.vectors                      # :155
+
+
+def random_features(n1, n2):
+    rng = np.random.default_rng(42)
+    emb_trained = 0.25 * rng.standard_normal((n1, 512))
+    q, _ = np.linalg.qr(rng.standard_normal((512, 512)))
+    emb_untrained = np.repeat(emb_trained, 2, axis=0)[:n2] @ q + 0.01 * rng.standard_normal((min(2 * n1, n2), 512))
+    if emb_untrained.shape[0] < n2:
+        emb_untrained = np.vstack([emb_untrained, 0.25 * rng.standard_normal((n2 - emb_untrained.shape[0], 512))])
+    return emb_trained, emb_untrained
 
 
 def main():
@@ -46,18 +66,17 @@ def main():
     ap.add_argument("-thresh", type=float, default=1e-8)
     ap.add_argument("-conversion", type=float, default=1.0)
     ap.add_argument("--loss", default="mse_pearson", choices=["mse_pearson", "mse_pearson_grad"])
+    ap.add_argument("--features", default="random", choices=["random", "node2vec"])
     ap.add_argument("--out", default="")
     args = ap.parse_args()
     g = np.load(os.path.join(ROOT, "tests", "golden", "reference_golden.npz"))
     list_trained, list_untrained = g["1mb_list"], g["500kb_list"]
     normed_trained, normed_untrained = normed_map(list_trained), normed_map(list_untrained)
     n1, n2 = normed_trained.shape[0], normed_untrained.shape[0]
-    rng = np.random.default_rng(42)
-    emb_trained = 0.25 * rng.standard_normal((n1, 512))
-    q, _ = np.linalg.qr(rng.standard_normal((512, 512)))
-    emb_untrained = np.repeat(emb_trained, 2, axis=0)[:n2] @ q + 0.01 * rng.standard_normal((min(2 * n1, n2), 512))
-    if emb_untrained.shape[0] < n2:
-        emb_untrained = np.vstack([emb_untrained, 0.25 * rng.standard_normal((n2 - emb_untrained.shape[0], 512))])
+    if args.features == "node2vec":
+        emb_trained, emb_untrained = node2vec_features(normed_trained), node2vec_features(normed_untrained)
+    else:
+        emb_trained, emb_untrained = random_features(n1, n2)
 
     # ---- train on the 1 Mb map
     data = utils.load_input(normed_trained, emb_trained)
@@ -84,7 +103,7 @@ def main():
     dscc_generalised = metrics.dscc(coords, target_fit)
     if args.out:
         utils.WritePDB(coords * 100, args.out)
-    print(f"loss {args.loss}: trained on {n1} loci: steps={len(hist)} loss {hist[0]:.5f} -> {hist[-1]:.5f} dSCC={dscc_trained:.4f}; "
+    print(f"features {args.features}, loss {args.loss}: trained on {n1} loci: steps={len(hist)} loss {hist[0]:.5f} -> {hist[-1]:.5f} dSCC={dscc_trained:.4f}; "
           f"generalised to {n2} loci: dSCC={dscc_generalised:.4f}" + (f"; wrote {args.out}" if args.out else ""))
     return hist, coords, dscc_trained, dscc_generalised
 

@@ -14,7 +14,7 @@ _PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("HICGAT_LIB") or os.path.join(_PKG, "libhicgat_sm100.so")
 HEADER = os.path.join(os.path.dirname(_PKG), "include", "hicgat.h")
 
-_p, _i64, _i32, _u32, _f32, _f64, _sz = C.c_void_p, C.c_int64, C.c_int, C.c_uint32, C.c_float, C.c_double, C.c_size_t
+_p, _i64, _i32, _u32, _u64, _f32, _f64, _sz = C.c_void_p, C.c_int64, C.c_int, C.c_uint32, C.c_uint64, C.c_float, C.c_double, C.c_size_t
 
 # name -> (restype, argtypes); mirrors include/hicgat.h one to one
 SIGNATURES = {
@@ -80,6 +80,8 @@ SIGNATURES = {
     "hicgat_kr_scale_round_f64": (C.c_int, [_p, _i64, _i64, _p, _p, _i64, _i32, _p]),
     "hicgat_gat_bwd_fused": (C.c_int, [_p, _p, _p, _i64, _i64, _i32, _i32, _p, _p, _p, _p, _f32, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
     "hicgat_gat_bwd": (C.c_int, [_p, _p, _p, _i64, _i64, _i32, _i32, _p, _p, _p, _f32, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
+    "hicgat_node2vec_walks": (C.c_int, [_p, _p, _p, _p, _i64, _i64, _i32, _f32, _f32, _u64, _p, _p]),
+    "hicgat_sgns_epoch": (C.c_int, [_p, _p, _i64, _i32, _p, _p, _i64, _i32, _i32, _i32, _f64, _f64, _i32, _i32, _u64, _i64, _p, _p, _p]),
 }
 
 PAIR_GRAD_MSE, PAIR_GRAD_L1, PAIR_MOMENTS, PAIR_MOMENTS_D, PAIR_WS_CLEAN, PAIR_SYMMETRIC, PAIR_NMOM = 1, 2, 4, 8, 16, 32, 8

@@ -20,7 +20,7 @@ void set_error(const char* fmt, ...) {
 void count_launch(int n) { g_launches.fetch_add((uint64_t)n, std::memory_order_relaxed); }
 }  // namespace hicgat
 
-extern "C" int hicgat_version(void) { return 201; }
+extern "C" int hicgat_version(void) { return 202; }
 extern "C" const char* hicgat_last_error(void) { return hicgat::g_err; }
 extern "C" uint64_t hicgat_launch_count(void) { return hicgat::g_launches.load(std::memory_order_relaxed); }
 

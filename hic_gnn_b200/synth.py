@@ -73,7 +73,9 @@ def synthetic_map(n: int, density: float, seed: int | None = None, device="cpu")
 
 
 def synthetic_features(n: int, dim: int = 512, seed: int | None = None, device="cpu") -> torch.Tensor:
-    """``0.25 * randn(N, 512)`` f32 stand-in for the node2vec / LINE embeddings."""
+    """``0.25 * randn(N, 512)`` f32 seeded random node features: a cheap stand-in for the LINE embeddings (not carried by
+    this package) and for node2vec embeddings where their cost is not wanted; :mod:`hic_gnn_b200.node2vec` computes the
+    real node2vec embeddings of a graph."""
     g = torch.Generator().manual_seed((1234 + n if seed is None else seed) + 1)
     return (0.25 * torch.randn(n, dim, generator=g)).to(device)
 

@@ -456,6 +456,57 @@ HICGAT_API int hicgat_spmv_csr_f64(const int32_t* rowptr, const int32_t* col, co
 HICGAT_API int hicgat_kr_scale_round_f64(const double* A, int64_t ld, int64_t n, const double* x, double* out, int64_t ldo,
                               int decimals, hicgat_stream_t stream);
 
+/* ------------------------------------------------------------------------------------
+ * (f-5) node2vec node features: Node2Vec(graph, ...).fit(...) of node2vec 0.4.3 / gensim 4
+ * (HiC_GAT_generalize_directly.py:153-155, train_and_test_same_res_GAT_node2vec.py:72,
+ * combined_loss_training.py:90, HiC-GNN_node2vec_conversion.py:118).  The Python layer is
+ * hic_gnn_b200/node2vec.py; tests/node2vec_ref.py restates every rule below in numpy.
+ *
+ * Random numbers: one stateless counter hash, mix64 = the splitmix64 finaliser
+ *     h = mix64(seed ^ 0x9E3779B97F4A7C15); h = mix64(h ^ a); h = mix64(h ^ b); h = mix64(h ^ c)
+ * Walk draws use (a, b, c) = (walk id, step, attempt); skip-gram draws use (epoch, raw token
+ * position, purpose << 32 | index) with purpose 0 = down-sampling, 1 = reduced window,
+ * 2 = negatives (index = context ordinal * negative + k).
+ *
+ * hicgat_node2vec_walks: one walk of `walk_length` nodes per start (int32 walks[num_starts][walk_length],
+ *   row i = walk id walk_id0 + i, so a batch of starts can be launched on its own with the same result).
+ *   Graph: the weighted, symmetric, diagonal-free CSR of load_input (rowptr/col int32, columns of a
+ *   row sorted); `cdf` f32[nnz] is the per-row cumulative edge weight whose last entry is the row total.
+ *   First step from v: P(x|v) ~ w(v,x): u = (h >> 40) 2^-24, x = col[first k with cdf[k] > u cdf[end-1]].
+ *   Later steps from t -> v: P(x|t,v) ~ w(v,x) alpha, alpha = 1/p if x = t, 1 if x in N(t), else 1/q,
+ *   by rejection: propose x as in the first step (u from h >> 40 of attempt a = 0, 1, ...), accept
+ *   iff (h & 0xFFFFFF) 2^-24 max(1/p, 1, 1/q) < alpha (x in N(t) by binary search in t's row).
+ *   Exact and O(nnz) memory; the attempts are not capped (that would bias the walk).  The expected
+ *   number of proposals per step is max(1/p, 1, 1/q) / E_{x ~ w(v,.)}[alpha(t, x)].
+ *   A node without neighbours ends its walk; the remaining entries are -1.
+ *
+ * hicgat_sgns_epoch: epoch `epoch` (of `epochs`) of skip-gram with negative sampling over the walks,
+ *   word2vec.c / gensim sg=1, hs=0.  walk_offsets int64[num_walks + 1]: raw-token position of each
+ *   walk's first token (exclusive prefix count of the tokens != -1); T = walk_offsets[num_walks].
+ *   Per walk: token at raw position r is kept iff (h(epoch, r, 0) >> 32) <= keep_threshold[token]
+ *   (uint32(p_keep (2^32 - 1)), gensim's sample_int).  Per kept centre c at raw position r, in order:
+ *   b = (h(epoch, r, 1<<32) >> 32) % window; contexts o = the kept tokens within window - b on each
+ *   side (ascending); alpha_c = max(min_alpha, alpha - (alpha - min_alpha) (epoch T + r) / (epochs T))
+ *   in f64, used as f32.  Per pair (c, o): l1 = syn0[o], neu1e = 0; for target c (label 1) then
+ *   `negative` draws bisect_left(cum_table, (h(epoch, r, 2<<32 | ordinal*negative + k) >> 32) % cum_table[n-1])
+ *   (label 0, a draw equal to c is skipped): f = l1.syn1neg[t]; g = (label - sigma(f)) alpha_c for
+ *   -6 <= f <= 6, (label - 1) alpha_c above, label alpha_c below (exact sigma); neu1e += g syn1neg[t];
+ *   syn1neg[t] += g l1.  Then syn0[o] += neu1e.  Updates are red.global.add.v4.f32.
+ *   num_warps warps own contiguous ranges of walks; num_warps = 1 is the serial order above
+ *   (replayable up to the f32 order of the dot products); num_warps <= 0 fills the GPU (Hogwild:
+ *   concurrent warps race on shared rows, lose no update, and are not bit-reproducible, as
+ *   gensim with workers > 1 is not).  dim % 128 == 0, dim <= 1024, 0 <= negative <= 31 (one lane
+ *   per target), window >= 1, walk_length <= HICGAT_N2V_MAX_WALK_LENGTH (shared-memory cap).
+ * ---------------------------------------------------------------------------------- */
+#define HICGAT_N2V_MAX_WALK_LENGTH 512
+HICGAT_API int hicgat_node2vec_walks(const int32_t* rowptr, const int32_t* col, const float* cdf, const int32_t* starts,
+                          int64_t num_starts, int64_t walk_id0, int walk_length, float p, float q, uint64_t seed,
+                          int32_t* walks, hicgat_stream_t stream);
+HICGAT_API int hicgat_sgns_epoch(const int32_t* walks, const int64_t* walk_offsets, int64_t num_walks, int walk_length,
+                      const uint32_t* cum_table, const uint32_t* keep_threshold, int64_t n, int dim, int window,
+                      int negative, double alpha, double min_alpha, int epoch, int epochs, uint64_t seed,
+                      int64_t num_warps, float* syn0, float* syn1neg, hicgat_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
