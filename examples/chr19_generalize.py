@@ -18,10 +18,11 @@ hic_gnn_b200.node2vec) and aligns the 500 kb embeddings onto the 1 Mb ones with 
 1 Mb ones, so that the alignment has something to recover.
 
     python examples/chr19_generalize.py [--steps 300] [--loss mse_pearson|mse_pearson_grad] [--features random|node2vec]
-                                        [--out /tmp/chr19_500kb_generalized_structure.pdb]
+                                        [--track-dscc] [--out /tmp/chr19_500kb_generalized_structure.pdb]
 
 ``--loss mse_pearson`` (default) is the reference's loss, whose Pearson term carries no gradient; ``mse_pearson_grad`` trains
-on the same total with the gradient of the (1 - r) term as well.
+on the same total with the gradient of the (1 - r) term as well.  ``--track-dscc`` records the dSCC of every training step on the
+device (``fit(dscc_out=...)``), as the reference keeps ``SpRho`` (:242, :189-192), and prints the curve every 50 steps and at the end.
 """
 import argparse
 import io
@@ -67,6 +68,7 @@ def main():
     ap.add_argument("-conversion", type=float, default=1.0)
     ap.add_argument("--loss", default="mse_pearson", choices=["mse_pearson", "mse_pearson_grad"])
     ap.add_argument("--features", default="random", choices=["random", "node2vec"])
+    ap.add_argument("--track-dscc", action="store_true")
     ap.add_argument("--out", default="")
     args = ap.parse_args()
     g = np.load(os.path.join(ROOT, "tests", "golden", "reference_golden.npz"))
@@ -83,8 +85,12 @@ def main():
     target = utils.wish_target(data.y, args.conversion)
     torch.manual_seed(42)
     model = models.GATNetSelectiveResidualsUpdated().cuda()
+    sprho = [] if args.track_dscc else None
     hist = train.fit(model, data.x.float(), data.edge_index, target, mode=args.loss, lr=args.lr, thresh=args.thresh, max_steps=args.steps,
-                     use_cuda_graph=True, check_every=10)
+                     use_cuda_graph=True, check_every=10, dscc_out=sprho)
+    if sprho is not None:
+        for s in list(range(0, len(sprho), 50)) + [len(sprho) - 1]:
+            print(f"step {s:4d}: loss {hist[s]:.5f} dSCC {sprho[s]:.4f}")
     with torch.no_grad():
         dscc_trained = metrics.dscc(model.get_model(data.x.float(), data.edge_index), target)
     buf = io.BytesIO()

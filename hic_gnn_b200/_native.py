@@ -45,6 +45,10 @@ SIGNATURES = {
     "hicgat_rank_cross_sum": (C.c_int, [_p, _p, _i64, _i64, _i64, _i64, _f32, _f32, _i32, _p, _p, _p, _p]),
     "hicgat_dist_histogram": (C.c_int, [_p, _i64, _i64, _i64, _f32, _i32, _p, _p]),
     "hicgat_edge_dist_bins": (C.c_int, [_p, _p, _p, _i64, _i64, _i64, _f32, _i32, _p, _p]),
+    "hicgat_dscc_workspace_bytes": (_sz, [_i64, _i32]),
+    "hicgat_dscc_target_ranks": (C.c_int, [_p, _i64, _i64, _f32, _i32, _p, _p, _p, _sz, _p]),
+    "hicgat_dscc_dense": (C.c_int, [_p, _p, _i64, _i64, _f32, _i32, _p, _p, _p, _p, _sz, _p]),
+    "hicgat_dscc_implicit": (C.c_int, [_p, _p, _p, _p, _i64, _p, _p, _i32, _p, _p, _sz, _p]),
     "hicgat_pairdist_fwd": (C.c_int, [_p, _i64, _p, _i64, _p]),
     "hicgat_pairdist_bwd": (C.c_int, [_p, _i64, _p, _i64, _p, _p]),
     "hicgat_cont2dist_max_f64": (C.c_int, [_p, _i64, _i64, _i64, _i64, _f64, _p, _p, _sz, _p]),

@@ -6,6 +6,8 @@ strict-upper-triangle wish distances and the reconstructed pairwise distances
 AVERAGE ranks for ties -- every zero-contact pair has wish distance exactly 1.0, so ties are the
 rule, not the exception.  The distances come from the library's pair-distance kernel; the rank
 transform is sort-based torch glue (evaluation runs once per model, not per step).
+:class:`DsccMeter` is the per-step form (the reference also evaluates ``spearmanr`` every iteration,
+HiC_GAT_generalize_directly.py:242): histogram mid-ranks entirely on the device, graph-capturable.
 """
 from __future__ import annotations
 
@@ -66,6 +68,21 @@ def _spearman_from_tables(hist_d, hist_t, cross, npairs: float) -> float:
     return cov / (var_d * var_t) ** 0.5
 
 
+def _implicit_target_ranks(tv: torch.Tensor, fill: float, npairs: float):
+    """Average ranks of an implicit target's i<j values: ``tv`` (f64) holds the stored pairs, the other ``npairs - len(tv)`` pairs are
+    ``fill``.  Returns (rank of every stored value, rank of the fill group, var_t = sum (rank - mean)^2 over all pairs), the last two as
+    0-d device tensors."""
+    n_stored = tv.numel()
+    vals, inv, counts = torch.unique(torch.cat((tv, torch.tensor([float(fill)], dtype=torch.float64, device=tv.device))), return_inverse=True, return_counts=True)
+    counts = counts.to(torch.float64)
+    fill_slot = inv[-1]
+    counts[fill_slot] += npairs - n_stored - 1.0   # the appended marker itself is not a pair
+    below = torch.cumsum(counts, 0) - counts
+    rank_vals = below + (counts + 1.0) / 2.0
+    mean = (npairs + 1.0) / 2.0
+    return rank_vals[inv[:-1]], rank_vals[fill_slot], (counts * (rank_vals - mean) ** 2).sum()
+
+
 def dscc_streamed(coords: torch.Tensor, target, nbins: int = NBINS, reduce=None) -> float:
     """dSCC without the N x N distance matrix, the ``triu_indices`` gathers or a sort (``hicgat_rank_*``): two streaming passes over
     the target (dense :class:`ops.WishTarget`, any row block) or one compute-only pass plus O(nnz) work (implicit
@@ -100,22 +117,14 @@ def dscc_streamed(coords: torch.Tensor, target, nbins: int = NBINS, reduce=None)
         # rank of t: the stored values (all ranks' values are needed: gather them when sharded) and the fill group
         if reduce is not None:
             raise NotImplementedError("row-sharded dSCC of an implicit target: gather the stored values first (use the dense streamed form per rank)")
-        n_stored = tv.numel()
-        vals, inv, counts = torch.unique(torch.cat((tv, torch.tensor([float(target.fill)], dtype=torch.float64, device=dev))), return_inverse=True, return_counts=True)
-        counts = counts.to(torch.float64)
-        fill_slot = inv[-1]
-        counts[fill_slot] += npairs - n_stored - 1.0   # the appended marker itself is not a pair
-        below = torch.cumsum(counts, 0) - counts
-        rank_vals = below + (counts + 1.0) / 2.0
-        rt = rank_vals[inv[:-1]]
-        r_fill = float(rank_vals[fill_slot])
+        rt, r_fill, var_t = _implicit_target_ranks(tv, target.fill, npairs)
+        r_fill, var_t = float(r_fill), float(var_t)
         mean = (npairs + 1.0) / 2.0
         hd = hist_d.to(torch.float64)
         sum_rd_all = float((hd * rank_d).sum())
         rd = rank_d[bd]
         cross = float((rt * rd).sum()) + r_fill * (sum_rd_all - float(rd.sum()))
         var_d = float((hd * (rank_d - mean) ** 2).sum())
-        var_t = float((counts * (rank_vals - mean) ** 2).sum())
         return (cross - npairs * mean * mean) / (var_d * var_t) ** 0.5
     if not isinstance(target, ops.WishTarget):
         raise TypeError("dscc_streamed expects a WishTarget or a SparseWishTarget")
@@ -136,6 +145,70 @@ def dscc_streamed(coords: torch.Tensor, target, nbins: int = NBINS, reduce=None)
     if reduce is not None:
         reduce(cross)
     return _spearman_from_tables(hist_d, hist_t, cross, npairs)
+
+
+class DsccMeter:
+    """dSCC of a full target at every training step (``spearmanr`` per iteration, HiC_GAT_generalize_directly.py:242), on the device.
+
+    ``DsccMeter(target)`` takes a dense :class:`ops.WishTarget` or an implicit :class:`ops.SparseWishTarget` of all ``n`` rows and does
+    the target-side work once: the rank table of the target (``hicgat_dscc_target_ranks``), or the ranks of the stored values and of
+    the fill group.  It allocates every buffer here.  ``meter(coords)`` then returns the dSCC as a 0-d f64 CUDA tensor with no host
+    read and no allocation (``hicgat_dscc_dense`` / ``hicgat_dscc_implicit``), so it can be captured in a CUDA graph.  The same tensor
+    is returned and overwritten by every call.  Histogram mid-ranks with ``nbins`` bins, the bins of :func:`dscc_streamed`: the two
+    agree to summation order.  NaN for constant distances or targets, as scipy gives."""
+
+    def __init__(self, target, nbins: int = NBINS):
+        from . import _native as N
+
+        if not isinstance(target, (ops.WishTarget, ops.SparseWishTarget)):
+            raise TypeError("DsccMeter expects a WishTarget or a SparseWishTarget")
+        if target.r0 != 0 or target.r1 != target.n:
+            raise ValueError("DsccMeter needs the full target (rows [0, n)); a row block would need the histograms all-reduced every step")
+        nbins = int(nbins)
+        if nbins <= 0:
+            raise ValueError(f"nbins must be positive, got {nbins}")
+        self.target, self.n, self.nbins = target, target.n, nbins
+        lib, n = N.lib(), target.n
+        dev = target.data.device if isinstance(target, ops.WishTarget) else target.tval.device
+        ws_bytes = lib.hicgat_dscc_workspace_bytes(n, nbins)
+        if ws_bytes == 0:
+            raise ValueError(f"DsccMeter: unsupported size n={n}, nbins={nbins}")
+        self._ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        self.rho = torch.full((), float("nan"), dtype=torch.float64, device=dev)
+        npairs = n * (n - 1) / 2.0
+        if isinstance(target, ops.WishTarget):
+            tmax = float(target.data.max()) if target.data.numel() else 1.0
+            self._t_scale = nbins / (max(tmax, 1e-30) * (1.0 + 1e-6))          # the rule of dscc_streamed
+            self._rank_t = torch.empty(nbins, dtype=torch.float64, device=dev)
+            self._var_t = torch.empty((), dtype=torch.float64, device=dev)
+            N.check(lib.hicgat_dscc_target_ranks(target.data.data_ptr(), target.pitch, n, self._t_scale, nbins, self._rank_t.data_ptr(),
+                                                 self._var_t.data_ptr(), self._ws.data_ptr(), ws_bytes, ops._stream()), "hicgat_dscc_target_ranks")
+        else:
+            row = torch.repeat_interleave(torch.arange(n, device=dev), target.rowptr[1:].long() - target.rowptr[:-1].long())
+            up = target.col.long() > row
+            rt, r_fill, var_t = _implicit_target_ranks(target.tval[up].double(), target.fill, npairs)
+            self._rank_t = torch.zeros(max(target.col.numel(), 1), dtype=torch.float64, device=dev)
+            self._rank_t[: target.col.numel()][up] = rt
+            self._rank_fill, self._var_t = r_fill.reshape(()).clone(), var_t.reshape(()).clone()
+        self._ws_bytes = ws_bytes
+
+    def __call__(self, coords: torch.Tensor) -> torch.Tensor:
+        from . import _native as N
+
+        ops._cuda(coords)
+        if coords.dtype != torch.float32 or coords.dim() != 2 or tuple(coords.shape) != (self.n, 3) or not coords.is_contiguous():
+            raise RuntimeError(f"coords must be contiguous float32 [n,3] with n={self.n}, got {coords.dtype} {tuple(coords.shape)}")
+        lib, t = N.lib(), self.target
+        if isinstance(t, ops.WishTarget):
+            rc = lib.hicgat_dscc_dense(coords.data_ptr(), t.data.data_ptr(), t.pitch, self.n, self._t_scale, self.nbins, self._rank_t.data_ptr(),
+                                       self._var_t.data_ptr(), self.rho.data_ptr(), self._ws.data_ptr(), self._ws_bytes, ops._stream())
+            N.check(rc, "hicgat_dscc_dense")
+        else:
+            rc = lib.hicgat_dscc_implicit(coords.data_ptr(), t.rowptr.data_ptr(), t.col.data_ptr(), self._rank_t.data_ptr(), self.n,
+                                          self._rank_fill.data_ptr(), self._var_t.data_ptr(), self.nbins, self.rho.data_ptr(), self._ws.data_ptr(),
+                                          self._ws_bytes, ops._stream())
+            N.check(rc, "hicgat_dscc_implicit")
+        return self.rho
 
 
 def dscc(coords: torch.Tensor, truth) -> float:

@@ -36,7 +36,10 @@ def drmsd_from_moments(moments: torch.Tensor, n: int) -> torch.Tensor:
 
 def step_loss(model, x, graph, target: WishTarget, mode: str, reducer=None, alpha: float = 1.0):
     """Forward + fused loss; returns (differentiable loss, total value tensor, moments)."""
-    coords = model.get_model(x, graph)
+    return _loss_of_coords(model.get_model(x, graph), target, mode, reducer, alpha)
+
+
+def _loss_of_coords(coords, target, mode: str, reducer, alpha: float):
     loss, moments = pairwise_loss(coords, target, _KERNEL_MODE[mode], reducer)
     total = loss.detach()  # mse_pearson_grad: the f64 total from the same moments as the gradient
     if mode == "mse_spearman":
@@ -57,12 +60,19 @@ def step_loss(model, x, graph, target: WishTarget, mode: str, reducer=None, alph
 
 class TrainStep:
     """One training iteration, optionally captured in a CUDA graph (small N is launch-bound:
-    ~40 kernels per step).  ``total`` / ``moments`` are static device tensors when graphed."""
+    ~40 kernels per step).  ``total`` / ``moments`` are static device tensors when graphed.
+
+    ``track_dscc=True`` also evaluates the dSCC of every step's forward coordinates -- the structure before that step's update, whose
+    ``spearmanr`` the reference records every iteration (HiC_GAT_generalize_directly.py:242) -- with a :class:`metrics.DsccMeter`, on
+    the device and inside the graph.  The value is ``step.dscc`` (0-d f64, overwritten by the next step).  Needs the full target:
+    refused with a sharded ``reducer``."""
 
     def __init__(self, model, x, graph, target: WishTarget, mode: str = "mse", lr: float = 1e-3, use_cuda_graph: bool = False, reducer=None,
-                 alpha: float = 1.0):
+                 alpha: float = 1.0, track_dscc: bool = False):
         if mode not in _KERNEL_MODE:
             raise ValueError(mode)
+        if track_dscc and reducer is not None:
+            raise ValueError("track_dscc needs the full target on one GPU: per-step dSCC of a row-sharded target is not supported")
         if mode == "mse_spearman" and use_cuda_graph:
             raise ValueError("mse_spearman reads the rank correlation back every step: it cannot be captured in a CUDA graph")
         if use_cuda_graph and reducer is not None and not getattr(reducer, "capturable", False):
@@ -74,13 +84,22 @@ class TrainStep:
         self.optimizer = Adam(model.parameters(), lr=lr, capturable=use_cuda_graph)
         self.total = None
         self.moments = None
+        self.dscc = None
+        self._meter = None
+        if track_dscc:
+            from .metrics import DsccMeter
+
+            self._meter = DsccMeter(target)      # target-side tables and every buffer exist before a capture
         self._graph = None
         if use_cuda_graph:
             self._capture()
 
     def _eager(self):
         self.optimizer.zero_grad(set_to_none=True)
-        loss, total, moments = step_loss(self.model, self.x, self.graph, self.target, self.mode, self.reducer, self.alpha)
+        coords = self.model.get_model(self.x, self.graph)
+        if self._meter is not None:
+            self.dscc = self._meter(coords.detach().contiguous())
+        loss, total, moments = _loss_of_coords(coords, self.target, self.mode, self.reducer, self.alpha)
         loss.backward()
         self.optimizer.step()
         return total, moments
@@ -117,25 +136,36 @@ class TrainStep:
 
 
 def fit(model, x, graph, target: WishTarget, mode: str = "mse", lr: float = 1e-3, thresh: float = 1e-8, max_steps: int | None = None,
-        check_every: int = 1, use_cuda_graph: bool = False, reducer=None, alpha: float = 1.0):
+        check_every: int = 1, use_cuda_graph: bool = False, reducer=None, alpha: float = 1.0, dscc_out: list | None = None):
     """Reference loop.  Returns the list of per-step total losses (floats).
 
     ``check_every=1`` evaluates the stop rule every step exactly like the reference (one host
     read per step).  Larger values read the losses back in batches: same trajectory, but the
-    loop may overrun the reference's stopping step by up to ``check_every-1`` iterations."""
-    step = TrainStep(model, x, graph, target, mode, lr, use_cuda_graph, reducer, alpha)
+    loop may overrun the reference's stopping step by up to ``check_every-1`` iterations.
+
+    ``dscc_out``: a list to which the dSCC of every step's (pre-update) structure is appended, like the reference's ``SpRho``
+    history (``TrainStep(track_dscc=True)``); read back in the same batched reads as the losses."""
+    track = dscc_out is not None
+    step = TrainStep(model, x, graph, target, mode, lr, use_cuda_graph, reducer, alpha, track_dscc=track)
     hist: list[float] = []
     pending: list[torch.Tensor] = []
+    pending_dscc: list[torch.Tensor] = []
     old = 1.0
     done = False
     while not done and (max_steps is None or len(hist) + len(pending) < max_steps):
         model.train()
         total, _ = step()
         pending.append(total.clone() if use_cuda_graph else total)
+        if track:
+            pending_dscc.append(step.dscc.clone())
         if len(pending) >= check_every or (max_steps is not None and len(hist) + len(pending) >= max_steps):
-            vals = torch.stack([p.double().reshape(()) for p in pending]).tolist()
+            k = len(pending)
+            vals = torch.stack([p.double().reshape(()) for p in pending + pending_dscc]).tolist()
             pending.clear()
-            for v in vals:
+            pending_dscc.clear()
+            if track:
+                dscc_out.extend(vals[k:])
+            for v in vals[:k]:
                 hist.append(v)
                 if not (abs(old - v) > thresh):  # the reference loops `while lossdiff > thresh`: a NaN loss ends training
                     done = True

@@ -269,6 +269,36 @@ HICGAT_API int hicgat_dist_histogram(const float* coords, int64_t n, int64_t r0,
 HICGAT_API int hicgat_edge_dist_bins(const float* coords, const int32_t* rowptr, const int32_t* col, int64_t n, int64_t r0, int64_t r1,
                           float d_scale, int nbins, int32_t* bins, hicgat_stream_t stream);
 
+/* Per-step dSCC of a FULL target (rows [0, n)), entirely on the device: no host read, no floating-point atomics, bit-reproducible
+ * for a given launch, capturable in a CUDA graph (the reference evaluates spearmanr every iteration: HiC_GAT_generalize_directly.py:242).
+ * Same bins and mid-ranks as the hicgat_rank_* path above (metrics.dscc_streamed):
+ *   d_scale = (float)(nbins / dmax), dmax = sqrt(sum_xyz span^2) (1 + 1e-6) + 1e-30 in f64, span = max - min of the coordinates in f32
+ *             (computed on the device and read by the later kernels through a pointer);
+ *   t_scale = nbins / (max(t) (1 + 1e-6)), chosen by the caller once per target;
+ *   rank[b] = (pairs in bins < b) + (hist[b] + 1) / 2, exact in f64;  P = n (n - 1) / 2,  mean = (P + 1) / 2;
+ *   rho = (cross - P mean^2) / sqrt(var_d var_t), var_x = sum_b hist_x[b] (rank_x[b] - mean)^2;  rho is NaN when var_d var_t is
+ *   not finite or <= 0 (constant input, n < 3), as scipy.stats.spearmanr gives.
+ * Histograms use uint64 atomics, one per warp when all of its pairs share a bin; every floating-point sum is per block, then
+ * reduced in a fixed order by one block.
+ *   hicgat_dscc_workspace_bytes  scratch of one evaluation: hist and rank_d (8 nbins B each) + per-block partials; 0 for bad
+ *                                arguments.  0 < n <= 2 097 120 (65535 tiles of 32 rows), nbins > 0.
+ *   hicgat_dscc_target_ranks     once per dense target (pitch >= n; only i < j is read): rank_t f64[nbins] and var_t (f64 scalar)
+ *   hicgat_dscc_dense            per step, dense target: rho (f64 scalar) from coords f32[n][3], the target and its rank_t / var_t
+ *   hicgat_dscc_implicit         per step, implicit target (the CSR pattern and fill of a SparseWishTarget): rank_t_csr f64[nnz] is
+ *                                the rank of the stored value of every entry k = (i, j) with j > i (other entries are not read),
+ *                                rank_fill / var_t device f64 scalars of the full target (stored values + the fill group);
+ *                                cross = sum_stored rank_t rank_d + rank_fill (sum_b hist_d rank_d - sum_stored rank_d)
+ * The workspace may be shared by calls on one stream; it holds rank_d of the last call. */
+HICGAT_API size_t hicgat_dscc_workspace_bytes(int64_t n, int nbins);
+HICGAT_API int hicgat_dscc_target_ranks(const float* target, int64_t pitch, int64_t n, float t_scale, int nbins, double* rank_t, double* var_t,
+                             void* workspace, size_t workspace_bytes, hicgat_stream_t stream);
+HICGAT_API int hicgat_dscc_dense(const float* coords, const float* target, int64_t pitch, int64_t n, float t_scale, int nbins,
+                      const double* rank_t, const double* var_t, double* rho, void* workspace, size_t workspace_bytes,
+                      hicgat_stream_t stream);
+HICGAT_API int hicgat_dscc_implicit(const float* coords, const int32_t* rowptr, const int32_t* col, const double* rank_t_csr, int64_t n,
+                         const double* rank_fill, const double* var_t, int nbins, double* rho, void* workspace,
+                         size_t workspace_bytes, hicgat_stream_t stream);
+
 /* Materialising variant kept for API parity of model.forward() (returns the N x N matrix,
  * models.py:39): dist[i,j] = |x_i - x_j|, and its backward
  * grad_coords[i] = sum_j (G[i,j] + G[j,i]) (x_i - x_j)/d_ij  (ATen _euclidean_dist_backward). */
