@@ -41,6 +41,13 @@ void count_launch(int n = 1);
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// (heads, channels per head) of GATConv that both message-passing paths take: exactly the instantiations of
+// HICGAT_DISPATCH_HQ in conv.cu, whose logit kernel the dense path shares.  H*C/128 is 1, 2, 4 or 8.
+static inline bool gat_shape_supported(int H, int C) {
+    return (H == 1 && (C == 128 || C == 256 || C == 512)) || (H == 2 && (C == 128 || C == 256 || C == 512)) ||
+           (H == 4 && (C == 128 || C == 256));
+}
+
 // ---------------------------------------------------------------- packed fp32x2 (Blackwell FADD2/FMUL2/FFMA2)
 typedef unsigned long long f2;  // two f32 in one 64-bit register pair
 

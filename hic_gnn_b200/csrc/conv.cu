@@ -616,11 +616,6 @@ __global__ void __launch_bounds__(256) gat_bwd_param_reduce_kernel(const float* 
 
 int param_ctas(int64_t n) { return (int)(n < kParamCtas ? n : kParamCtas); }
 
-bool supported(int H, int C) {
-    const int F = H * C;
-    return (H == 1 || H == 2 || H == 4) && C % 128 == 0 && (F == 128 || F == 256 || F == 512 || F == 1024);
-}
-
 // warps (= consecutive rows) per CTA of the two gather kernels (gat_fwd / gat_bwd_fused): 8 or 16, see hicgat_gat_set_tuning
 int g_gather_warps = 8;
 // bytes of L2 set aside for the GATHERED matrix (xl in the forward, gout in the backward): 0 = off
@@ -711,7 +706,7 @@ extern "C" int hicgat_gat_fwd(const int32_t* rowptr, const int32_t* col, int64_t
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     HICGAT_REQUIRE(rowptr && col && xl && att_l && att_r && bias && a_src && a_dst && alpha && out, "hicgat_gat_fwd: null pointer");
     HICGAT_REQUIRE(n > 0 && n < (1ll << 31), "hicgat_gat_fwd: bad n");
-    HICGAT_REQUIRE(supported(heads, channels), "hicgat_gat_fwd: unsupported heads=%d channels=%d", heads, channels);
+    HICGAT_REQUIRE(gat_shape_supported(heads, channels), "hicgat_gat_fwd: unsupported heads=%d channels=%d", heads, channels);
     HICGAT_REQUIRE(aligned16(xl) && aligned16(out) && aligned16(att_l) && aligned16(att_r) && aligned16(bias), "hicgat_gat_fwd: 16-byte alignment required");
     const unsigned grid = (unsigned)((n + kRowsPerCta - 1) / kRowsPerCta);
 #define CALL_LOGIT(H, Q) gat_logit_kernel<H, Q><<<grid, 256, 0, stream>>>(xl, att_l, att_r, (int)n, a_src, a_dst)
@@ -749,7 +744,7 @@ BwdLayout bwd_layout(int64_t n, int64_t nnz, int H, int C) {
 }  // namespace
 
 extern "C" size_t hicgat_gat_bwd_workspace_bytes(int64_t n, int64_t nnz, int heads, int channels) {
-    if (n <= 0 || nnz < 0 || !supported(heads, channels)) return 0;
+    if (n <= 0 || nnz < 0 || !gat_shape_supported(heads, channels)) return 0;
     return bwd_layout(n, nnz, heads, channels).total;
 }
 
@@ -762,7 +757,7 @@ extern "C" int hicgat_gat_bwd(const int32_t* rowptr, const int32_t* col, const i
     HICGAT_REQUIRE(rowptr && col && perm && xl && att_l && att_r && a_src && a_dst && alpha && gout && dxl && datt_l && datt_r && dbias && workspace,
                    "hicgat_gat_bwd: null pointer");
     HICGAT_REQUIRE(n > 0 && n < (1ll << 31) && nnz >= 0 && nnz < (1ll << 31), "hicgat_gat_bwd: bad n/nnz");
-    HICGAT_REQUIRE(supported(heads, channels), "hicgat_gat_bwd: unsupported heads=%d channels=%d", heads, channels);
+    HICGAT_REQUIRE(gat_shape_supported(heads, channels), "hicgat_gat_bwd: unsupported heads=%d channels=%d", heads, channels);
     HICGAT_REQUIRE(aligned16(xl) && aligned16(gout) && aligned16(dxl) && aligned16(att_l) && aligned16(att_r), "hicgat_gat_bwd: 16-byte alignment required");
     const BwdLayout L = bwd_layout(n, nnz, heads, channels);
     if (workspace_bytes < L.total) {
@@ -800,7 +795,7 @@ extern "C" int hicgat_gat_bwd_fused(const int32_t* rowptr, const int32_t* col, c
     HICGAT_REQUIRE(rowptr && col && perm && xl && att_l && att_r && bias && a_src && a_dst && alpha && out && gout && dxl && datt_l && datt_r && dbias && workspace,
                    "hicgat_gat_bwd_fused: null pointer");
     HICGAT_REQUIRE(n > 0 && n < (1ll << 31) && nnz >= 0 && nnz < (1ll << 31), "hicgat_gat_bwd_fused: bad n/nnz");
-    HICGAT_REQUIRE(supported(heads, channels), "hicgat_gat_bwd_fused: unsupported heads=%d channels=%d", heads, channels);
+    HICGAT_REQUIRE(gat_shape_supported(heads, channels), "hicgat_gat_bwd_fused: unsupported heads=%d channels=%d", heads, channels);
     HICGAT_REQUIRE(aligned16(xl) && aligned16(gout) && aligned16(out) && aligned16(dxl) && aligned16(att_l) && aligned16(att_r) && aligned16(bias),
                    "hicgat_gat_bwd_fused: 16-byte alignment required");
     const BwdLayout L = bwd_layout(n, nnz, heads, channels);
@@ -843,7 +838,7 @@ extern "C" int hicgat_gat_logits(int64_t n, int heads, int channels, const float
                                  float* a_src, float* a_dst, hicgat_stream_t stream_) {
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     HICGAT_REQUIRE(xl && att_l && att_r && a_src && a_dst && n > 0 && n < (1ll << 31), "hicgat_gat_logits: bad arguments");
-    HICGAT_REQUIRE(supported(heads, channels), "hicgat_gat_logits: unsupported heads=%d channels=%d", heads, channels);
+    HICGAT_REQUIRE(gat_shape_supported(heads, channels), "hicgat_gat_logits: unsupported heads=%d channels=%d", heads, channels);
     HICGAT_REQUIRE(aligned16(xl) && aligned16(att_l) && aligned16(att_r), "hicgat_gat_logits: 16-byte alignment required");
     const unsigned grid = (unsigned)((n + kRowsPerCta - 1) / kRowsPerCta);
 #define CALL_LOGIT(H, Q) gat_logit_kernel<H, Q><<<grid, 256, 0, stream>>>(xl, att_l, att_r, (int)n, a_src, a_dst)
@@ -854,7 +849,7 @@ extern "C" int hicgat_gat_logits(int64_t n, int heads, int channels, const float
 }
 
 extern "C" size_t hicgat_gat_param_grads_workspace_bytes(int64_t n, int heads, int channels) {
-    if (n <= 0 || !supported(heads, channels)) return 0;
+    if (n <= 0 || !gat_shape_supported(heads, channels)) return 0;
     return 256 + sizeof(float) * 3 * (size_t)heads * channels * (size_t)param_ctas(n);
 }
 
@@ -864,7 +859,7 @@ extern "C" int hicgat_gat_param_grads(int64_t n, int heads, int channels, const 
                                       size_t workspace_bytes, hicgat_stream_t stream_) {
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     HICGAT_REQUIRE(xl && gout && d_a_src && d_a_dst && datt_l && datt_r && dbias && workspace && n > 0 && n < (1ll << 31), "hicgat_gat_param_grads: bad arguments");
-    HICGAT_REQUIRE(supported(heads, channels), "hicgat_gat_param_grads: unsupported heads=%d channels=%d", heads, channels);
+    HICGAT_REQUIRE(gat_shape_supported(heads, channels), "hicgat_gat_param_grads: unsupported heads=%d channels=%d", heads, channels);
     const size_t need = hicgat_gat_param_grads_workspace_bytes(n, heads, channels);
     if (workspace_bytes < need) {
         set_error("hicgat_gat_param_grads: workspace %zu < required %zu", workspace_bytes, need);

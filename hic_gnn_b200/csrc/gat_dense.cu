@@ -437,7 +437,6 @@ DenseLayout dense_layout(int64_t n, int H, int C = 0) {
     L.total = L.off_split + (L.nsplit > 1 ? sizeof(float) * (size_t)L.nsplit * n * H * C : 0);
     return L;
 }
-bool dense_supported(int H, int C) { return (H == 1 || H == 2 || H == 4) && C % BN == 0 && C >= BN; }
 }  // namespace
 
 extern "C" size_t hicgat_gat_dense_mask_words(int64_t n) { return n > 0 ? (size_t)((n + 31) / 32) : 0; }
@@ -453,7 +452,7 @@ extern "C" int hicgat_gat_dense_build_mask(const int32_t* rowptr, const int32_t*
 }
 
 extern "C" size_t hicgat_gat_dense_workspace_bytes(int64_t n, int heads, int channels) {
-    if (n <= 0 || !dense_supported(heads, channels)) return 0;
+    if (n <= 0 || !gat_shape_supported(heads, channels)) return 0;
     return dense_layout(n, heads, channels).total;
 }
 
@@ -463,7 +462,7 @@ extern "C" int hicgat_gat_dense_fwd(const int32_t* rowptr, const int32_t* col, c
                                     float* out, void* workspace, size_t workspace_bytes, hicgat_stream_t stream_) {
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     HICGAT_REQUIRE(rowptr && col && mask && xl && a_src && a_dst && bias && out && workspace, "hicgat_gat_dense_fwd: null pointer");
-    HICGAT_REQUIRE(n > 0 && n < (1ll << 24) && dense_supported(heads, channels), "hicgat_gat_dense_fwd: unsupported n/heads/channels (%lld,%d,%d)", (long long)n, heads, channels);
+    HICGAT_REQUIRE(n > 0 && n < (1ll << 24) && gat_shape_supported(heads, channels), "hicgat_gat_dense_fwd: unsupported n/heads/channels (%lld,%d,%d)", (long long)n, heads, channels);
     HICGAT_REQUIRE(aligned16(xl) && aligned16(out) && aligned16(bias), "hicgat_gat_dense_fwd: 16-byte alignment required");
     const DenseLayout L = dense_layout(n, heads, channels);
     if (workspace_bytes < L.total) { set_error("hicgat_gat_dense_fwd: workspace %zu < required %zu", workspace_bytes, L.total); return HICGAT_ERR_WORKSPACE; }
@@ -497,7 +496,7 @@ extern "C" int hicgat_gat_dense_bwd(const uint32_t* mask, int64_t n, int heads, 
                                     void* workspace, size_t workspace_bytes, hicgat_stream_t stream_) {
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     HICGAT_REQUIRE(mask && xl && a_src && a_dst && att_l && att_r && bias && out && gout && dxl && d_a_src && d_a_dst && workspace, "hicgat_gat_dense_bwd: null pointer");
-    HICGAT_REQUIRE(n > 0 && n < (1ll << 24) && dense_supported(heads, channels), "hicgat_gat_dense_bwd: unsupported n/heads/channels");
+    HICGAT_REQUIRE(n > 0 && n < (1ll << 24) && gat_shape_supported(heads, channels), "hicgat_gat_dense_bwd: unsupported n/heads/channels");
     HICGAT_REQUIRE(aligned16(xl) && aligned16(out) && aligned16(gout) && aligned16(dxl) && aligned16(att_l) && aligned16(att_r) && aligned16(bias), "hicgat_gat_dense_bwd: 16-byte alignment required");
     const DenseLayout L = dense_layout(n, heads, channels);
     if (workspace_bytes < L.total) { set_error("hicgat_gat_dense_bwd: workspace %zu < required %zu", workspace_bytes, L.total); return HICGAT_ERR_WORKSPACE; }

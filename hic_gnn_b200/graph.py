@@ -10,6 +10,21 @@ from . import _native as N
 from .ops import _cuda, _stream
 
 
+_PLACEHOLDER: dict = {}
+
+
+def _addr(t: torch.Tensor) -> int:
+    """``t.data_ptr()``, or for an empty ``t`` (whose ``data_ptr()`` is 0) the address of a small placeholder on its device: the
+    C ABI refuses null arrays, and a pattern without edges (a map with no off-diagonal contact, a single locus) has empty ``col``
+    and value arrays, which the kernels -- bounded by ``rowptr`` -- never read."""
+    if t.numel():
+        return t.data_ptr()
+    buf = _PLACEHOLDER.get(t.device)
+    if buf is None:
+        buf = _PLACEHOLDER[t.device] = torch.zeros(4, dtype=torch.int32, device=t.device)
+    return buf.data_ptr()
+
+
 class _Storage:
     """``SparseTensor.storage`` look-alike (``rowptr()/col()/value()/row()``)."""
 
@@ -96,7 +111,7 @@ class CSRGraph:
                 raise RuntimeError("CSRGraph.with_self_loops: the stored pattern already has diagonal entries")
             orow = torch.empty(self.n + 1, dtype=torch.int32, device=self.device)
             ocol = torch.empty(self.nnz + self.n, dtype=torch.int32, device=self.device)
-            N.check(N.lib().hicgat_csr_add_self_loops_i32(r32.data_ptr(), c32.data_ptr(), self.n, orow.data_ptr(), ocol.data_ptr(), _stream()), "hicgat_csr_add_self_loops_i32")
+            N.check(N.lib().hicgat_csr_add_self_loops_i32(r32.data_ptr(), _addr(c32), self.n, orow.data_ptr(), ocol.data_ptr(), _stream()), "hicgat_csr_add_self_loops_i32")
             perm = torch.empty(self.nnz + self.n, dtype=torch.int32, device=self.device)
             N.check(N.lib().hicgat_csr_transpose_perm(orow.data_ptr(), ocol.data_ptr(), self.n, perm.data_ptr(), _stream()), "hicgat_csr_transpose_perm")
             _check_transpose_perm(perm, "CSRGraph.with_self_loops")
@@ -128,9 +143,9 @@ class CSRGraph:
             r32, c32 = self.i32()
             colsum = torch.empty(self.n, dtype=torch.float32, device=self.device)
             norm = torch.empty(max(self.nnz, 1), dtype=torch.float32, device=self.device)
-            N.check(N.lib().hicgat_sage_norm_values(r32.data_ptr(), c32.data_ptr(), self.value.data_ptr(), self.n, colsum.data_ptr(), norm.data_ptr(), _stream()), "hicgat_sage_norm_values")
+            N.check(N.lib().hicgat_sage_norm_values(r32.data_ptr(), _addr(c32), _addr(self.value), self.n, colsum.data_ptr(), norm.data_ptr(), _stream()), "hicgat_sage_norm_values")
             perm = torch.empty(max(self.nnz, 1), dtype=torch.int32, device=self.device)
-            N.check(N.lib().hicgat_csr_transpose_perm(r32.data_ptr(), c32.data_ptr(), self.n, perm.data_ptr(), _stream()), "hicgat_csr_transpose_perm")
+            N.check(N.lib().hicgat_csr_transpose_perm(r32.data_ptr(), _addr(c32), self.n, perm.data_ptr(), _stream()), "hicgat_csr_transpose_perm")
             norm = norm[: self.nnz]
             _check_transpose_perm(perm[: self.nnz], "CSRGraph.sage_weights")
             return norm, norm[perm[: self.nnz].long()].contiguous()

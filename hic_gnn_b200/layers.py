@@ -14,7 +14,7 @@ import torch
 from torch import nn
 
 from . import _native as N
-from .graph import CSRGraph, as_graph
+from .graph import CSRGraph, _addr, as_graph
 from . import ops as _ops
 from .ops import _cuda, _stream
 
@@ -29,7 +29,7 @@ class _SageAggregate(torch.autograd.Function):
         r32, c32 = graph.i32()
         w, _ = graph.sage_weights()
         out = torch.empty_like(x)
-        N.check(N.lib().hicgat_spmm_csr_f32(r32.data_ptr(), c32.data_ptr(), w.data_ptr(), x.data_ptr(), graph.n, x.shape[1], out.data_ptr(), _stream()), "hicgat_spmm_csr_f32")
+        N.check(N.lib().hicgat_spmm_csr_f32(r32.data_ptr(), _addr(c32), _addr(w), x.data_ptr(), graph.n, x.shape[1], out.data_ptr(), _stream()), "hicgat_spmm_csr_f32")
         ctx.graph = graph
         return out
 
@@ -40,7 +40,7 @@ class _SageAggregate(torch.autograd.Function):
         r32, c32 = graph.i32()
         _, wt = graph.sage_weights()
         dx = torch.empty_like(g)
-        N.check(N.lib().hicgat_spmm_csr_f32(r32.data_ptr(), c32.data_ptr(), wt.data_ptr(), g.data_ptr(), graph.n, g.shape[1], dx.data_ptr(), _stream()), "hicgat_spmm_csr_f32")
+        N.check(N.lib().hicgat_spmm_csr_f32(r32.data_ptr(), _addr(c32), _addr(wt), g.data_ptr(), graph.n, g.shape[1], dx.data_ptr(), _stream()), "hicgat_spmm_csr_f32")
         return dx, None
 
 
@@ -75,6 +75,13 @@ class SAGEConv(nn.Module):
 
 # CSR GAT backward: "fused" (one 2 KB-per-edge gather pass) or "split" (two passes); env HICGAT_GAT_BWD overrides
 GAT_BACKWARD = os.environ.get("HICGAT_GAT_BWD", "fused")
+
+# (heads, channels per head) the GAT kernels are compiled for, on both message-passing paths (conv.cu HICGAT_DISPATCH_HQ)
+GAT_SHAPES = ((1, 128), (1, 256), (1, 512), (2, 128), (2, 256), (2, 512), (4, 128), (4, 256))
+
+
+def gat_shape_supported(heads: int, channels: int) -> bool:
+    return (heads, channels) in GAT_SHAPES
 
 
 class _GatWorkspace:
@@ -212,6 +219,9 @@ class GATConv(nn.Module):
         super().__init__()
         if not concat or dropout != 0.0 or not add_self_loops or not bias:
             raise NotImplementedError("only the configuration the reference uses: concat=True, dropout=0, add_self_loops=True, bias=True")
+        if not gat_shape_supported(heads, out_channels):
+            raise NotImplementedError(f"GATConv kernels support (heads, out_channels) in {', '.join(map(str, GAT_SHAPES))}; "
+                                      f"got ({heads}, {out_channels})")
         self.in_channels, self.out_channels, self.heads, self.negative_slope = in_channels, out_channels, heads, negative_slope
         # message-passing path: "auto" = dense tiles when >= dense_threshold of all pairs are edges
         # (and the kernels support the shape), else the CSR warp-per-row kernels; "csr" / "dense" force one
@@ -249,10 +259,10 @@ class GATConv(nn.Module):
     def forward(self, x, edge_index, edge_weight=None, size=None):
         graph = as_graph(edge_index, edge_weight, x.shape[0])
         xl = self.lin_l(x)
-        dense_ok = self.out_channels % 128 == 0 and self.heads in (1, 2, 4) and graph.n <= self.dense_max_n
+        dense_ok = gat_shape_supported(self.heads, self.out_channels) and graph.n <= self.dense_max_n
         use_dense = self.path == "dense" or (self.path == "auto" and dense_ok and graph.n >= 256 and graph.density() >= self.dense_threshold)
         if use_dense and not dense_ok:
-            raise RuntimeError("dense GAT path: channels must be a multiple of 128 and heads in {1,2,4}")
+            raise RuntimeError(f"dense GAT path: needs at most dense_max_n = {self.dense_max_n} loci and (heads, channels) in {GAT_SHAPES}")
         fn = _GatAttendDense if use_dense else _GatAttend
         return fn.apply(xl, self.att_l, self.att_r, self.bias, graph, self.heads, self.out_channels, self.negative_slope)
 

@@ -406,10 +406,12 @@ HICGAT_API int hicgat_csr_transpose_perm(const int32_t* rowptr, const int32_t* c
 /* ------------------------------------------------------------------------------------
  * (1c) GATConv message passing (torch-geometric 1.7.2 GATConv, ctor sites models.py:619,1013;
  * semantics in SURVEY.md Appendix A.3).  `xl` [n, H*C] = lin_l(x) (cuBLAS, outside);
- * CSR pattern includes self loops.  H in {1,2,4}, C multiple of 128/H... see gat.cu.
+ * CSR pattern includes self loops.  (heads H, channels per head C) is one of (1,128) (1,256) (1,512) (2,128)
+ * (2,256) (2,512) (4,128) (4,256), for these entry points and the dense-tile ones in (1d); any other pair is
+ * HICGAT_ERR_INVALID and its workspace size is 0.
  *   fwd : a_src/a_dst [n,H] (logit halves), alpha [nnz,H] (saved attention), out [n,H*C]
  *         out = softmax_row(leaky_relu(a_src[j] + a_dst[i], slope)) @ xl  + bias
- *   bwd : given g = dL/dout: dxl [n,H*C], datt_l/datt_r [H*C] (+=), dbias [H*C]
+ *   bwd : given g = dL/dout: dxl [n,H*C], datt_l/datt_r [H*C], dbias [H*C] (all overwritten)
  * ---------------------------------------------------------------------------------- */
 /* Process-wide tuning of the two gather kernels (gat_fwd, gat_bwd_fused).
  * rows_per_cta: consecutive rows (= warps) per CTA, 8 (default) or 16 -- consecutive rows of a Hi-C map share neighbours,
@@ -444,7 +446,7 @@ HICGAT_API int hicgat_gat_bwd_fused(const int32_t* rowptr, const int32_t* col, c
  * (1d) Dense-tile path of the same GATConv for near-dense graphs (1 Mb / 100 kb maps): per head the
  * attention matrix is regenerated tile by tile from the rank-1 logits, the row statistics and a
  * bit mask of the pattern and fed to register-tiled fp32 GEMMs; nothing of size N x N is stored.
- * Same results as hicgat_gat_fwd / _bwd up to fp32 summation order.  channels % 128 == 0.
+ * Same results as hicgat_gat_fwd / _bwd up to fp32 summation order.  Same (heads, channels) pairs as (1c).
  *   logits      : a_src/a_dst [n,H] = <xl, att_l>, <xl, att_r> per head (shared with the CSR path)
  *   build_mask  : mask u32[n][ceil(n/32)] from the self-loop CSR pattern (once per graph)
  *   fwd         : out [n,H*C]; row max / 1/sum stay in `workspace` for the backward

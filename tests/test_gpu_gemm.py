@@ -8,7 +8,10 @@ from helpers import rel_err
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.parametrize("m,n,k", [(128, 128, 32), (300, 70, 100), (129, 257, 33), (1000, 512, 512), (4100, 256, 512), (49850, 512, 512), (20000, 3, 64)])
+# the last three are GATConv projections with H*C = 1024 (test_gpu_conv_shapes.py): the dx GEMM of 512 -> 1024 on 5 000 loci (K' = 3 072:
+# two split-K partials over 40 M tiles), the forward of 512 -> 1024 at 9 970 loci (128 x 256 tiles, 4 N tiles) and of 128 -> 1024
+@pytest.mark.parametrize("m,n,k", [(128, 128, 32), (300, 70, 100), (129, 257, 33), (1000, 512, 512), (4100, 256, 512), (49850, 512, 512), (20000, 3, 64),
+                                   (5000, 512, 1024), (9970, 1024, 512), (5000, 1024, 128)])
 def test_gemm_tf32x3_matches_f64(m, n, k):
     from hic_gnn_b200 import ops
 
