@@ -718,12 +718,21 @@ __global__ void __launch_bounds__(kCombineThreads, 2) pairloss_combine_kernel(co
 //     pairloss_csr_fix_kernel then corrects the nnz pairs that do carry a contact.
 // ROWS: upper-triangle mode (chunk_rows clips every strip at its last column, so no row below the diagonal strip is loaded).
 // Same decomposition, arithmetic and reductions as the TMA kernels.
+// x_i is staged in pieces of at most kStageRows rows, so a chunk of any length fits the default 48 KB of shared memory (the
+// layout doubles the chunk length of long row blocks to stay within kMaxChunks).  kStageRows is a multiple of kTileRows: every
+// warp visits the same row groups in the same order as with the whole chunk staged at once.
+constexpr int kStageRows = 1024;
+static_assert(kStageRows % kTileRows == 0, "a staging piece must hold whole tiles");
+__host__ __device__ constexpr size_t lane_smem_bytes(int rb) {
+    return (sizeof(float4) + sizeof(float2)) * (size_t)(rb < kStageRows ? rb : kStageRows);
+}
 template <uint32_t MODE, bool ROWS, bool IMPLICIT>
 __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_lane_kernel(const Params P) {
     pdl_launch_dependents();
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    float4* s_xy = reinterpret_cast<float4*>(smem_raw);                          // [rb] (x,x,y,y)
-    float2* s_z = reinterpret_cast<float2*>(smem_raw + sizeof(float4) * P.rb);   // [rb] (z,z)
+    const int stage_rows = min(P.rb, kStageRows);
+    float4* s_xy = reinterpret_cast<float4*>(smem_raw);                                 // [stage_rows] (x,x,y,y)
+    float2* s_z = reinterpret_cast<float2*>(smem_raw + sizeof(float4) * stage_rows);    // [stage_rows] (z,z)
     __shared__ CombineSmem S;
 
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -734,52 +743,56 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_lane_kernel(con
     const int count = chunk_rows(P, strip, chunk, row_begin, nrows);
     if (chunk >= count || nrows <= 0) return;  // unstaggered strips leave the extra chunk slot empty
     const bool edge = (strip + 1) * kCols > n;
-    for (int r = threadIdx.x; r < nrows; r += kThreads) {
-        const float* c = P.coords + (size_t)(row_begin + r) * 3;
-        float x = c[0], y = c[1], z = c[2];
-        s_xy[r] = make_float4(x, x, y, y);
-        s_z[r] = make_float2(z, z);
-    }
     ColumnRegs c;
     load_columns(c, P.coords, col0, n);
     Acc a;
     acc_zero(a);
     const PearsonCoef pc = pearson_coef<MODE>(P.pmom, n, P.c_mse, P.dyn_alpha);
-    __syncthreads();
     const bool can_load = col0 + 3 < P.pitch;  // pitch is a multiple of 4 (0 for the implicit target)
     const float* tbase = P.target + (size_t)(row_begin - P.r0) * P.pitch + col0;
     const int strip_lo = strip * kCols, strip_hi = strip_lo + kCols - 1;
-    const int ngroups = (nrows + kU - 1) / kU;
     const float f = P.fill;
-    for (int g = warp; g < ngroups; g += kWarps) {
-        const int rl = g * kU, rg = row_begin + rl;
-        const int rows_here = min(kU, nrows - rl);
-        float4 t[kU];
-        if constexpr (IMPLICIT) {
+    for (int p0 = 0; p0 < nrows; p0 += kStageRows) {
+        const int prows = min(kStageRows, nrows - p0);
+        if (p0 > 0) __syncthreads();  // every warp is done with the previous piece
+        for (int r = threadIdx.x; r < prows; r += kThreads) {
+            const float* cr = P.coords + (size_t)(row_begin + p0 + r) * 3;
+            float x = cr[0], y = cr[1], z = cr[2];
+            s_xy[r] = make_float4(x, x, y, y);
+            s_z[r] = make_float2(z, z);
+        }
+        __syncthreads();
+        const int ngroups = (prows + kU - 1) / kU;
+        for (int g = warp; g < ngroups; g += kWarps) {
+            const int rl = p0 + g * kU, rg = row_begin + rl;
+            const int rows_here = min(kU, nrows - rl);
+            float4 t[kU];
+            if constexpr (IMPLICIT) {
 #pragma unroll
-            for (int u = 0; u < kU; ++u) t[u] = make_float4(f, f, f, f);
-            if (rg + kU - 1 >= strip_lo && rg <= strip_hi) {  // the group touches the diagonal: t_ii = 0
+                for (int u = 0; u < kU; ++u) t[u] = make_float4(f, f, f, f);
+                if (rg + kU - 1 >= strip_lo && rg <= strip_hi) {  // the group touches the diagonal: t_ii = 0
 #pragma unroll
-                for (int u = 0; u < kU; ++u) {
-                    const int dc = rg + u - col0;
-                    if (dc == 0) t[u].x = 0.f;
-                    if (dc == 1) t[u].y = 0.f;
-                    if (dc == 2) t[u].z = 0.f;
-                    if (dc == 3) t[u].w = 0.f;
+                    for (int u = 0; u < kU; ++u) {
+                        const int dc = rg + u - col0;
+                        if (dc == 0) t[u].x = 0.f;
+                        if (dc == 1) t[u].y = 0.f;
+                        if (dc == 2) t[u].z = 0.f;
+                        if (dc == 3) t[u].w = 0.f;
+                    }
+                }
+            } else {
+                if (rows_here == kU && can_load) {
+#pragma unroll
+                    for (int u = 0; u < kU; ++u) t[u] = ldg_stream_f4(tbase + (size_t)(rl + u) * P.pitch);
+                } else {
+#pragma unroll
+                    for (int u = 0; u < kU; ++u)
+                        t[u] = (u < rows_here && can_load) ? ldg_stream_f4(tbase + (size_t)(rl + u) * P.pitch) : make_float4(0.f, 0.f, 0.f, 0.f);
                 }
             }
-        } else {
-            if (rows_here == kU && can_load) {
-#pragma unroll
-                for (int u = 0; u < kU; ++u) t[u] = ldg_stream_f4(tbase + (size_t)(rl + u) * P.pitch);
-            } else {
-#pragma unroll
-                for (int u = 0; u < kU; ++u)
-                    t[u] = (u < rows_here && can_load) ? ldg_stream_f4(tbase + (size_t)(rl + u) * P.pitch) : make_float4(0.f, 0.f, 0.f, 0.f);
-            }
+            process_group<MODE, ROWS>(a, c, t, XiPtr{s_xy + g * kU, s_z + g * kU}, rows_here, rg, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1,
+                                      ROWS ? P.rpart + (size_t)strip * P.rpitch + (size_t)(rg - P.r0) * 3 : nullptr, lane, pc);
         }
-        process_group<MODE, ROWS>(a, c, t, XiPtr{s_xy + rl, s_z + rl}, rows_here, rg, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1,
-                                  ROWS ? P.rpart + (size_t)strip * P.rpitch + (size_t)(rg - P.r0) * 3 : nullptr, lane, pc);
     }
     park_warp<MODE, ROWS>(a, S, warp, lane);
     __syncthreads();
@@ -1658,7 +1671,7 @@ Layout make_layout_uncached(int64_t n, int64_t r0, int64_t r1, int variant, bool
     } else if (sym && g_rows_per_cta == 0 && g_tail_depth < 0 && nrows > 0) {
         // equal chunks, no explicit tail (the triangle tapers by itself): pick the chunk length by simulation
         static const int cand0[] = {256, 384, 512, 640, 768, 1024, 1280, 1536, 2048, 3072, 4096};
-        static const int cand1[] = {256, 384, 512, 768, 1024};  // the implicit-target kernel stages a chunk of x_i in 48 KB of shared memory
+        static const int cand1[] = {256, 384, 512, 768, 1024};  // per-lane kernels: a chunk is at most one x_i staging piece (kStageRows)
         const int* cand = variant == 0 ? cand0 : cand1;
         const int ncand = variant == 0 ? 11 : 5;
         double best = 1e300;
@@ -1707,7 +1720,7 @@ Layout make_layout_uncached(int64_t n, int64_t r0, int64_t r1, int variant, bool
     }
     build_schedule(nrows > 0 ? nrows : 1, L.rb, depth, tail_min, L.stagger != 0, unit, L.sch);
     L.nchunks = L.sch.count[0] > L.sch.count[1] ? L.sch.count[0] : L.sch.count[1];
-    // the per-lane-load and implicit-target kernels stage one chunk of x_i in shared memory: size = longest chunk
+    // the per-lane-load and implicit-target kernels stage x_i of the longest chunk in shared memory, kStageRows rows at a time
     int longest = 0;
     for (int par = 0; par < 2; ++par)
         for (int k = 0; k < L.sch.count[par]; ++k) longest = std::max(longest, L.sch.bounds[par][k + 1] - L.sch.bounds[par][k]);
@@ -1891,7 +1904,7 @@ cudaError_t launch_mode(int variant, const CUtensorMap& map, const Params& P, di
     } else if (variant == 0) {
         e = P.upper ? launch_tma<MODE, true>(map, P, grid, stream) : launch_tma<MODE, false>(map, P, grid, stream);
     } else {
-        const size_t smem = (sizeof(float4) + sizeof(float2)) * (size_t)P.rb;
+        const size_t smem = lane_smem_bytes(P.rb);
         if (P.upper) pairloss_lane_kernel<MODE, true, false><<<grid, kThreads, smem, stream>>>(P);
         else pairloss_lane_kernel<MODE, false, false><<<grid, kThreads, smem, stream>>>(P);
         e = cudaGetLastError();
@@ -1956,7 +1969,7 @@ extern "C" int hicgat_pairloss_describe_schedule_mode(int64_t n, int64_t r0, int
         set_error("hicgat_pairloss_describe_schedule: bad arguments");
         return HICGAT_ERR_INVALID;
     }
-    const Layout L = make_layout(n, r0, r1, g_variant, g_variant == 0 && (mode & HICGAT_PAIR_SYMMETRIC) != 0);
+    const Layout L = make_layout(n, r0, r1, g_variant, (mode & HICGAT_PAIR_SYMMETRIC) != 0);
     const int need = 4 + (L.sch.count[0] + 1) + (L.sch.count[1] + 1);
     if (capacity < need) {
         set_error("hicgat_pairloss_describe_schedule: capacity %d < %d", (int)capacity, need);
@@ -1975,7 +1988,7 @@ extern "C" int hicgat_pairloss_describe_schedule_mode(int64_t n, int64_t r0, int
 extern "C" double hicgat_pairloss_estimate_cost(int64_t n, int64_t r0, int64_t r1, uint32_t mode) {
     if (n <= 0 || r0 < 0 || r1 < r0 || r1 > n) return -1.0;
     if (r1 == r0) return 0.0;
-    const bool sym = g_variant == 0 && (mode & HICGAT_PAIR_SYMMETRIC) != 0;
+    const bool sym = (mode & HICGAT_PAIR_SYMMETRIC) != 0;
     const Layout L = make_layout(n, r0, r1, g_variant, sym);
     if (sym) return simulate_upper(r0, L.nstrips, L.sch, L.stagger);
     // full-matrix mode: every strip has every chunk
@@ -2106,7 +2119,7 @@ struct SparseLayout {
 };
 SparseLayout sparse_layout(int64_t n, int64_t r0, int64_t r1, bool sym = false) {
     SparseLayout L;
-    L.dense = make_layout(n, r0, r1, 1, sym);  // row chunks <= 1024: the x_i staging fits the default 48 KB of shared memory
+    L.dense = make_layout(n, r0, r1, 1, sym);  // the per-lane kernel's chunks and partial slots
     L.fix_ctas = (int)((r1 - r0 + 7) / 8);
     if (L.fix_ctas < 1) L.fix_ctas = 1;
     L.off_counter = align_up(L.dense.total, 256);
@@ -2118,7 +2131,7 @@ SparseLayout sparse_layout(int64_t n, int64_t r0, int64_t r1, bool sym = false) 
 template <uint32_t MODE>
 cudaError_t launch_sparse(const Params& P, dim3 grid, const int32_t* rowptr, const int32_t* col, const float* tval, int fix_ctas, double* part,
                           unsigned* counter, cudaStream_t stream) {
-    const size_t smem = (sizeof(float4) + sizeof(float2)) * (size_t)P.rb;
+    const size_t smem = lane_smem_bytes(P.rb);
     if (P.upper) pairloss_lane_kernel<MODE, true, true><<<grid, kThreads, smem, stream>>>(P);
     else pairloss_lane_kernel<MODE, false, true><<<grid, kThreads, smem, stream>>>(P);
     cudaError_t e = cudaGetLastError();

@@ -7,22 +7,7 @@ from __future__ import annotations
 import torch
 
 from . import _native as N
-from .ops import _cuda, _stream
-
-
-_PLACEHOLDER: dict = {}
-
-
-def _addr(t: torch.Tensor) -> int:
-    """``t.data_ptr()``, or for an empty ``t`` (whose ``data_ptr()`` is 0) the address of a small placeholder on its device: the
-    C ABI refuses null arrays, and a pattern without edges (a map with no off-diagonal contact, a single locus) has empty ``col``
-    and value arrays, which the kernels -- bounded by ``rowptr`` -- never read."""
-    if t.numel():
-        return t.data_ptr()
-    buf = _PLACEHOLDER.get(t.device)
-    if buf is None:
-        buf = _PLACEHOLDER[t.device] = torch.zeros(4, dtype=torch.int32, device=t.device)
-    return buf.data_ptr()
+from .ops import _addr, _cuda, _stream
 
 
 class _Storage:

@@ -37,6 +37,21 @@ def _ptr(t):
     return None if t is None else t.data_ptr()
 
 
+_PLACEHOLDER: dict = {}
+
+
+def _addr(t: torch.Tensor) -> int:
+    """``t.data_ptr()``, or for an empty ``t`` (whose ``data_ptr()`` is 0) the address of a small placeholder on its device: the
+    C ABI refuses null arrays, and a pattern without edges (a map with no off-diagonal contact, a single locus) has empty ``col``
+    and value arrays, which the kernels -- bounded by ``rowptr`` -- never read."""
+    if t.numel():
+        return t.data_ptr()
+    buf = _PLACEHOLDER.get(t.device)
+    if buf is None:
+        buf = _PLACEHOLDER[t.device] = torch.zeros(4, dtype=torch.int32, device=t.device)
+    return buf.data_ptr()
+
+
 # ------------------------------------------------------------------------------ target
 class WishTarget:
     """f32 wish-distance row block ``rows [r0, r1) x n`` with a 16-byte-aligned pitch.
@@ -211,7 +226,7 @@ def pairloss_raw(coords: torch.Tensor, target: WishTarget, mode: int, c_mse: flo
             grad = torch.empty(n, 3, dtype=torch.float32, device=coords.device)
         ws = _PairWorkspace.get(coords.device, n, target.r0, target.r1, sparse=True, sym=_USE_UPPER)  # the layout depends on the mode
         rc = N.lib().hicgat_pairloss_sparse_fwd_bwd(
-            coords.data_ptr(), target.rowptr.data_ptr(), target.col.data_ptr(), target.tval.data_ptr(), target.fill, n, target.r0, target.r1,
+            coords.data_ptr(), target.rowptr.data_ptr(), _addr(target.col), _addr(target.tval), target.fill, n, target.r0, target.r1,
             mode | N.PAIR_WS_CLEAN | (N.PAIR_SYMMETRIC if _USE_UPPER else 0), c_mse, c_l1, moments.data_ptr(), _ptr(grad), ws.data_ptr(), ws.numel(), _stream(),
         )
         N.check(rc, "hicgat_pairloss_sparse_fwd_bwd")
@@ -261,7 +276,7 @@ def pearson_grad_raw(coords: torch.Tensor, target, moments: torch.Tensor, with_m
     if isinstance(target, SparseWishTarget):
         ws = _PairWorkspace.get(coords.device, n, target.r0, target.r1, sparse=True, sym=_USE_UPPER)
         rc = N.lib().hicgat_pairloss_sparse_pearson_grad(
-            coords.data_ptr(), target.rowptr.data_ptr(), target.col.data_ptr(), target.tval.data_ptr(), target.fill, n, target.r0, target.r1,
+            coords.data_ptr(), target.rowptr.data_ptr(), _addr(target.col), _addr(target.tval), target.fill, n, target.r0, target.r1,
             mode | (N.PAIR_SYMMETRIC if _USE_UPPER else 0), moments.data_ptr(), c_mse, int(with_mse), grad.data_ptr(), ws.data_ptr(), ws.numel(), _stream(),
         )
         N.check(rc, "hicgat_pairloss_sparse_pearson_grad")

@@ -4,6 +4,7 @@ The kernels trust these tables blindly (chunk c of a strip = rows [bounds[c], bo
 block), so the CPU suite checks, through the C ABI's introspection entry point, that for any shape and
 tuning they tile the block exactly once, in order, within the table size."""
 import ctypes as C
+import itertools
 
 import numpy as np
 import pytest
@@ -13,9 +14,9 @@ from hic_gnn_b200 import _native as N
 MAX_CHUNKS = 128
 
 
-def schedule(n, r0, r1):
+def schedule(n, r0, r1, mode=0):
     buf = (C.c_int32 * 600)()
-    k = N.lib().hicgat_pairloss_describe_schedule(n, r0, r1, C.addressof(buf), 600)
+    k = N.lib().hicgat_pairloss_describe_schedule_mode(n, r0, r1, mode, C.addressof(buf), 600)
     assert k > 0, N.lib().hicgat_last_error()
     a = list(buf[:k])
     nstrips, stagger, c0, c1 = a[:4]
@@ -40,14 +41,16 @@ SHAPES = [(58, 0, 58), (130, 0, 130), (1000, 999, 1000), (2493, 0, 2493), (9970,
 @pytest.mark.parametrize("rb", [0, 8, 64, 256, 1024, 4096])
 @pytest.mark.parametrize("tail", [(-1, 256), (0, 256), (1, 256), (3, 128), (8, 64)])
 def test_schedule_tiles_the_row_block(variant, rb, tail):
+    """Full-row and upper-triangle (``PAIR_SYMMETRIC``) layouts: the launches of every variant, the implicit target's
+    included, take the mode's schedule."""
     N.set_pairloss_tuning(rb, variant)
     N.set_pairloss_schedule(*tail)
-    for n, r0, r1 in SHAPES:
-        nstrips, stagger, b0, b1 = schedule(n, r0, r1)
+    for (n, r0, r1), mode in itertools.product(SHAPES, (0, N.PAIR_SYMMETRIC)):
+        nstrips, stagger, b0, b1 = schedule(n, r0, r1, mode)
         assert nstrips == (n + 127) // 128
         for b in (b0, b1):
-            assert b[0] == 0 and b[-1] == r1 - r0, (n, r0, r1, b)
-            assert (np.diff(b) > 0).all(), (n, r0, r1, b)
+            assert b[0] == 0 and b[-1] == r1 - r0, (n, r0, r1, mode, b)
+            assert (np.diff(b) > 0).all(), (n, r0, r1, mode, b)
             assert len(b) - 1 <= MAX_CHUNKS
         if not stagger:
             assert (b0 == b1).all() if len(b0) == len(b1) else False
