@@ -7,9 +7,11 @@
 //
 // Work decomposition (both kernel variants)
 //   CTA  = 8 consumer warps x 128 columns x rb rows; grid = (column strips, row chunks).
-//   lane = 4 consecutive columns j, kept as two packed f32x2 pairs so the arithmetic runs on
-//          FADD2/FMUL2/FFMA2; x_j and the column-side gradient accumulators live in registers
-//          for the whole CTA lifetime, x_i (warp-uniform) is broadcast from shared memory.
+//   warp = groups of 8 rows x 128 columns; lanes 0-15 take rows 0-3 of a group, lanes 16-31 rows 4-7.
+//   lane = 8 columns j, 4k..4k+3 and 64+4k..64+4k+3 (k = lane % 16), kept as four packed f32x2
+//          pairs so the arithmetic runs on FADD2/FMUL2/FFMA2; x_j and the column-side gradient
+//          accumulators live in registers for the whole CTA lifetime, x_i (uniform per half-warp)
+//          is broadcast from shared memory.
 //   Because the target is symmetric the column-side sum  g_j = sum_i w_ij (x_j - x_i)  is the
 //   complete gradient: no row-side reduction, no atomics.  Row chunks are combined by the last
 //   CTA to finish each column strip (fixed summation order => bit-reproducible).
@@ -19,7 +21,7 @@
 //   warp's mbarriers and refills a slot as soon as the warp has consumed it, so no warp ever
 //   waits on a global load it issued itself and 2 CTAs x 8 warps x 3 x 4 KB = 192 KB of target
 //   are in flight per SM.  TMA zero-fills columns >= n and rows >= r1-r0 (no edge address logic).
-// Variant 1 ("ldg"): each lane issues 8 streaming 128-bit ld.global.nc per row group; kept for
+// Variant 1 ("ldg"): each lane issues 4 rows x 2 streaming 128-bit ld.global.nc per row group; kept for
 //   A/B measurements and as the path used when a tensor map cannot be encoded.  Same triangle modes.
 #include <cuda.h>  // CUtensorMap (types only; the encoder is resolved through cudart at run time)
 
@@ -44,8 +46,10 @@ namespace {
 constexpr int kWarps = HICGAT_PAIR_WARPS; // consumer warps
 constexpr int kCtasPerSm = 16 / kWarps;   // 16 resident warps of 128 registers per SM
 constexpr int kThreads = kWarps * 32;     // variant 1 block size
-constexpr int kCols = 128;                // columns per CTA strip (32 lanes x 4)
+constexpr int kCols = 128;                // columns per CTA strip (16 lanes x 8)
 constexpr int kU = 8;                     // rows per warp per group / tile
+constexpr int kR = kU / 2;                // rows per lane per group (one half-warp's share)
+constexpr int kP = 4;                     // packed column pairs per lane
 constexpr int kNM = HICGAT_PAIR_NMOM;
 constexpr int kCtaSlots = 148 * kCtasPerSm;  // resident CTAs of the TMA kernel (2 per SM)
 constexpr int kTileRows = kWarps * kU;    // 64 rows per CTA tile step (8 per warp)
@@ -81,7 +85,7 @@ __device__ __forceinline__ unsigned long long gtimer() {
 #endif
 
 struct Acc {
-    f2 gx[2], gy[2], gz[2];          // column-side gradient, 2 column pairs
+    f2 gx[kP], gy[kP], gz[kP];       // column-side gradient, 4 column pairs
     f2 see;                          // sum (d-t)^2 over pairs NOT counted in seu
     f2 sd, sdd, st, stt, sdt, seu;   // upper-triangle moments
     float sabs0, sabs1;              // upper-triangle sum |d-t|
@@ -89,7 +93,7 @@ struct Acc {
 
 __device__ __forceinline__ void acc_zero(Acc& a) {
 #pragma unroll
-    for (int p = 0; p < 2; ++p) a.gx[p] = a.gy[p] = a.gz[p] = 0ull;
+    for (int p = 0; p < kP; ++p) a.gx[p] = a.gy[p] = a.gz[p] = 0ull;
     a.see = a.sd = a.sdd = a.st = a.stt = a.sdt = a.seu = 0ull;
     a.sabs0 = a.sabs1 = 0.f;
 }
@@ -310,27 +314,52 @@ __device__ __forceinline__ PearsonCoef pearson_coef(const double* pm, int n, flo
 }
 
 struct ColumnRegs {
-    f2 xjx[2], xjy[2], xjz[2], mv[2];
+    f2 xjx[kP], xjy[kP], xjz[kP];
 };
 
+// first column of the lane's packed pair p; col0 = strip * kCols + 4 * (lane % 16)
+__device__ __forceinline__ int pair_col(int col0, int p) { return col0 + (p >> 1) * (kCols / 2) + (p & 1) * 2; }
+__device__ __forceinline__ int lane_col0(int strip, int lane) { return strip * kCols + (lane & 15) * 4; }
+
 __device__ __forceinline__ void load_columns(ColumnRegs& c, const float* __restrict__ coords, int col0, int n) {
-    float cj[4][3];
 #pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        int cc = min(col0 + k, n - 1);
-#pragma unroll
-        for (int q = 0; q < 3; ++q) cj[k][q] = coords[(size_t)cc * 3 + q];
-    }
-#pragma unroll
-    for (int p = 0; p < 2; ++p) {
-        c.xjx[p] = f2_pack(cj[2 * p][0], cj[2 * p + 1][0]);
-        c.xjy[p] = f2_pack(cj[2 * p][1], cj[2 * p + 1][1]);
-        c.xjz[p] = f2_pack(cj[2 * p][2], cj[2 * p + 1][2]);
-        c.mv[p] = f2_pack(col0 + 2 * p < n ? 1.f : 0.f, col0 + 2 * p + 1 < n ? 1.f : 0.f);
+    for (int p = 0; p < kP; ++p) {
+        const int ca = min(pair_col(col0, p), n - 1), cb = min(pair_col(col0, p) + 1, n - 1);
+        c.xjx[p] = f2_pack(coords[(size_t)ca * 3], coords[(size_t)cb * 3]);
+        c.xjy[p] = f2_pack(coords[(size_t)ca * 3 + 1], coords[(size_t)cb * 3 + 1]);
+        c.xjz[p] = f2_pack(coords[(size_t)ca * 3 + 2], coords[(size_t)cb * 3 + 2]);
     }
 }
 
-// kU rows of one warp: t[u] = the lane's 4 target values of row (rg + u); xi from shared memory.
+// The lane's kR rows of a group: ts.load(r, lo, hi) = its target values of row (rg + 4 * (lane / 16) + r) at columns col0 .. col0+3
+// (lo) and col0+64 .. col0+67 (hi); x_i of group row u from shared memory.
+struct TileRegs {  // already in registers (per-lane loads)
+    float4 t[kR][2];
+    __device__ __forceinline__ void load(int r, float4& lo, float4& hi) const { lo = t[r][0]; hi = t[r][1]; }
+};
+struct TileFill {  // implicit target: `fill` everywhere but on the diagonal (t_ii = 0); dc = the lane's first row - col0
+    float f;
+    int dc;
+    bool diag;  // the group touches the diagonal
+    __device__ __forceinline__ void load(int r, float4& lo, float4& hi) const {
+        lo = hi = make_float4(f, f, f, f);
+        if (diag) {
+            const int d = dc + r;  // row - col0: the diagonal is at d = 0..3 (lo) or d = 64..67 (hi)
+            if (d == 0) lo.x = 0.f;
+            if (d == 1) lo.y = 0.f;
+            if (d == 2) lo.z = 0.f;
+            if (d == 3) lo.w = 0.f;
+            if (d == kCols / 2 + 0) hi.x = 0.f;
+            if (d == kCols / 2 + 1) hi.y = 0.f;
+            if (d == kCols / 2 + 2) hi.z = 0.f;
+            if (d == kCols / 2 + 3) hi.w = 0.f;
+        }
+    }
+};
+struct TileAddr {  // read from a TMA ring slot right before use: `base` = the lane's first value of its first row
+    uint32_t base;
+    __device__ __forceinline__ void load(int r, float4& lo, float4& hi) const;
+};
 struct XiPtr {  // x_i rows behind ordinary shared-memory pointers (variant 1)
     const float4* xy;
     const float2* z;
@@ -341,16 +370,14 @@ struct XiAddr {  // x_i rows behind 32-bit shared-space addresses (TMA variant)
     __device__ __forceinline__ void load(int u, float4& oxy, float2& oz) const;
 };
 
-// Transpose-reduce of the 24 row-side sums of one 8-row group (v[3 * u + comp]) across the warp: 24 shuffles instead of
-// 24 x 5.  On return lane L holds the warp total of slot  12*b4 + 6*b3 + 3*b2 + (b0 ? 2 : b1)  (b_k = bit k of L);
-// lanes with b0 = 1 hold their slot twice (b1 = 0 and b1 = 1).  Fixed order: bit-reproducible.
-__device__ __forceinline__ float row_butterfly(const float (&v)[3 * kU], int lane) {
-    const bool b4 = lane & 16, b3 = lane & 8, b2 = lane & 4, b1 = lane & 2, b0 = lane & 1;
-    float w12[12], w6[6], w3[3];
+// Transpose-reduce of the 12 row-side sums of a half-warp's 4 rows (v[3 * r + comp]) across its 16 lanes: 12 shuffles instead
+// of 12 x 4.  On return lane L holds the half-warp total of group slot  12*b4 + 6*b3 + 3*b2 + (b0 ? 2 : b1)  (b_k = bit k of L,
+// slot = 3 * row + comp); lanes with b0 = 1 hold their slot twice (b1 = 0 and b1 = 1).  Fixed order: bit-reproducible.
+__device__ __forceinline__ float row_butterfly(const float (&v)[3 * kR], int lane) {
+    const bool b3 = lane & 8, b2 = lane & 4, b1 = lane & 2, b0 = lane & 1;
+    float w6[6], w3[3];
 #pragma unroll
-    for (int k = 0; k < 12; ++k) w12[k] = (b4 ? v[k + 12] : v[k]) + __shfl_xor_sync(0xffffffffu, b4 ? v[k] : v[k + 12], 16);
-#pragma unroll
-    for (int k = 0; k < 6; ++k) w6[k] = (b3 ? w12[k + 6] : w12[k]) + __shfl_xor_sync(0xffffffffu, b3 ? w12[k] : w12[k + 6], 8);
+    for (int k = 0; k < 6; ++k) w6[k] = (b3 ? v[k + 6] : v[k]) + __shfl_xor_sync(0xffffffffu, b3 ? v[k] : v[k + 6], 8);
 #pragma unroll
     for (int k = 0; k < 3; ++k) w3[k] = (b2 ? w6[k + 3] : w6[k]) + __shfl_xor_sync(0xffffffffu, b2 ? w6[k] : w6[k + 3], 4);
     const float a = (b1 ? w3[1] : w3[0]) + __shfl_xor_sync(0xffffffffu, b1 ? w3[0] : w3[1], 2);
@@ -363,61 +390,73 @@ __device__ __forceinline__ int row_butterfly_slot(int lane) {
 
 // ROWS (upper-triangle mode): `rowdst` points at the 3 * kU row-side partials of this group's rows for this strip;
 // the group is never strictly below the diagonal (the CTA's row range is clipped at the strip's last column).
-template <uint32_t MODE, bool ROWS, typename XI>
-__device__ __forceinline__ void process_group(Acc& a, const ColumnRegs& c, const float4 (&t)[kU], const XI xi,
+// A lane evaluates its kR rows (those of its half-warp) against its 8 columns: one row's sum spans 16 lanes, so the horizontal
+// sums and the transpose-reduce of the row-side accumulators cost half as much per pair as with 4 columns x 8 rows per lane.
+template <uint32_t MODE, bool ROWS, typename TS, typename XI>
+__device__ __forceinline__ void process_group(Acc& a, const ColumnRegs& c, const TS& ts, const XI xi,
                                               int rows_here, int rg, int col0, int n, bool edge,
                                               int strip_lo, int strip_hi, float c_mse, float c_l1, float* __restrict__ rowdst, int lane,
                                               const PearsonCoef& pc) {
     const bool fast = !edge && rows_here == kU;
     constexpr bool kRowGrad = ROWS && has_grad(MODE);
-    float rv[kRowGrad ? 3 * kU : 1];
+    const int hr = (lane >> 4) * kR;  // first group row of this lane's half-warp
+    float rv[kRowGrad ? 3 * kR : 1];
     if (fast && rg + kU - 1 < strip_lo) {  // strictly above the diagonal
 #pragma unroll
-        for (int u = 0; u < kU; ++u) {
-            float4 xy;
+        for (int r = 0; r < kR; ++r) {
+            float4 xy, lo, hi;
             float2 zz;
-            xi.load(u, xy, zz);
-            f2 xix = f2_pack(xy.x, xy.y), xiy = f2_pack(xy.z, xy.w), xiz = f2_pack(zz.x, zz.y);
+            xi.load(hr + r, xy, zz);
+            ts.load(r, lo, hi);
+            const f2 xix = f2_pack(xy.x, xy.y), xiy = f2_pack(xy.z, xy.w), xiz = f2_pack(zz.x, zz.y);
+            const f2 t[kP] = {f2_pack(lo.x, lo.y), f2_pack(lo.z, lo.w), f2_pack(hi.x, hi.y), f2_pack(hi.z, hi.w)};
             RowAcc ra = {0ull, 0ull, 0ull};
-            pair_fast<MODE, true, ROWS>(a, ra, 0, c.xjx[0], c.xjy[0], c.xjz[0], xix, xiy, xiz, f2_pack(t[u].x, t[u].y), c_mse, c_l1, pc);
-            pair_fast<MODE, true, ROWS>(a, ra, 1, c.xjx[1], c.xjy[1], c.xjz[1], xix, xiy, xiz, f2_pack(t[u].z, t[u].w), c_mse, c_l1, pc);
+#pragma unroll
+            for (int p = 0; p < kP; ++p)
+                pair_fast<MODE, true, ROWS>(a, ra, p, c.xjx[p], c.xjy[p], c.xjz[p], xix, xiy, xiz, t[p], c_mse, c_l1, pc);
             if constexpr (kRowGrad) {
-                rv[3 * u] = f2_hsum(ra.x); rv[3 * u + 1] = f2_hsum(ra.y); rv[3 * u + 2] = f2_hsum(ra.z);
+                rv[3 * r] = f2_hsum(ra.x); rv[3 * r + 1] = f2_hsum(ra.y); rv[3 * r + 2] = f2_hsum(ra.z);
             }
         }
     } else if (!ROWS && fast && rg > strip_hi) {    // strictly below
 #pragma unroll
-        for (int u = 0; u < kU; ++u) {
-            float4 xy;
+        for (int r = 0; r < kR; ++r) {
+            float4 xy, lo, hi;
             float2 zz;
-            xi.load(u, xy, zz);
-            f2 xix = f2_pack(xy.x, xy.y), xiy = f2_pack(xy.z, xy.w), xiz = f2_pack(zz.x, zz.y);
+            xi.load(hr + r, xy, zz);
+            ts.load(r, lo, hi);
+            const f2 xix = f2_pack(xy.x, xy.y), xiy = f2_pack(xy.z, xy.w), xiz = f2_pack(zz.x, zz.y);
+            const f2 t[kP] = {f2_pack(lo.x, lo.y), f2_pack(lo.z, lo.w), f2_pack(hi.x, hi.y), f2_pack(hi.z, hi.w)};
             RowAcc ra = {0ull, 0ull, 0ull};
-            pair_fast<MODE, false, false>(a, ra, 0, c.xjx[0], c.xjy[0], c.xjz[0], xix, xiy, xiz, f2_pack(t[u].x, t[u].y), c_mse, c_l1, pc);
-            pair_fast<MODE, false, false>(a, ra, 1, c.xjx[1], c.xjy[1], c.xjz[1], xix, xiy, xiz, f2_pack(t[u].z, t[u].w), c_mse, c_l1, pc);
+#pragma unroll
+            for (int p = 0; p < kP; ++p)
+                pair_fast<MODE, false, false>(a, ra, p, c.xjx[p], c.xjy[p], c.xjz[p], xix, xiy, xiz, t[p], c_mse, c_l1, pc);
         }
     } else {
 #pragma unroll
-        for (int u = 0; u < kU; ++u) {
+        for (int r = 0; r < kR; ++r) {
             RowAcc ra = {0ull, 0ull, 0ull};
-            if (u < rows_here) {
-                const int r = rg + u;
-                float4 xy;
+            if (hr + r < rows_here) {
+                const int row = rg + hr + r;
+                float4 xy, lo, hi;
                 float2 zz;
-                xi.load(u, xy, zz);
-                f2 xix = f2_pack(xy.x, xy.y), xiy = f2_pack(xy.z, xy.w), xiz = f2_pack(zz.x, zz.y);
-                f2 mu0 = f2_pack((col0 + 0 < n && r < col0 + 0) ? 1.f : 0.f, (col0 + 1 < n && r < col0 + 1) ? 1.f : 0.f);
-                f2 mu1 = f2_pack((col0 + 2 < n && r < col0 + 2) ? 1.f : 0.f, (col0 + 3 < n && r < col0 + 3) ? 1.f : 0.f);
-                f2 mv0 = c.mv[0], mv1 = c.mv[1];
-                if constexpr (ROWS) {  // upper-triangle mode: pairs below the diagonal belong to another tile (as its upper pairs)
-                    mv0 = f2_pack((col0 + 0 < n && r <= col0 + 0) ? 1.f : 0.f, (col0 + 1 < n && r <= col0 + 1) ? 1.f : 0.f);
-                    mv1 = f2_pack((col0 + 2 < n && r <= col0 + 2) ? 1.f : 0.f, (col0 + 3 < n && r <= col0 + 3) ? 1.f : 0.f);
+                xi.load(hr + r, xy, zz);
+                ts.load(r, lo, hi);
+                const f2 xix = f2_pack(xy.x, xy.y), xiy = f2_pack(xy.z, xy.w), xiz = f2_pack(zz.x, zz.y);
+                const f2 t[kP] = {f2_pack(lo.x, lo.y), f2_pack(lo.z, lo.w), f2_pack(hi.x, hi.y), f2_pack(hi.z, hi.w)};
+#pragma unroll
+                for (int p = 0; p < kP; ++p) {
+                    const int j = pair_col(col0, p);
+                    // mv: valid column (upper-triangle mode: also row <= column -- pairs below the diagonal belong to another tile,
+                    // as its upper pairs); mu: strictly upper
+                    const f2 mv = ROWS ? f2_pack((j < n && row <= j) ? 1.f : 0.f, (j + 1 < n && row <= j + 1) ? 1.f : 0.f)
+                                       : f2_pack(j < n ? 1.f : 0.f, j + 1 < n ? 1.f : 0.f);
+                    const f2 mu = f2_pack((j < n && row < j) ? 1.f : 0.f, (j + 1 < n && row < j + 1) ? 1.f : 0.f);
+                    pair_masked<MODE, ROWS>(a, ra, p, c.xjx[p], c.xjy[p], c.xjz[p], xix, xiy, xiz, t[p], mv, mu, c_mse, c_l1, pc);
                 }
-                pair_masked<MODE, ROWS>(a, ra, 0, c.xjx[0], c.xjy[0], c.xjz[0], xix, xiy, xiz, f2_pack(t[u].x, t[u].y), mv0, mu0, c_mse, c_l1, pc);
-                pair_masked<MODE, ROWS>(a, ra, 1, c.xjx[1], c.xjy[1], c.xjz[1], xix, xiy, xiz, f2_pack(t[u].z, t[u].w), mv1, mu1, c_mse, c_l1, pc);
             }
             if constexpr (kRowGrad) {
-                rv[3 * u] = f2_hsum(ra.x); rv[3 * u + 1] = f2_hsum(ra.y); rv[3 * u + 2] = f2_hsum(ra.z);
+                rv[3 * r] = f2_hsum(ra.x); rv[3 * r + 1] = f2_hsum(ra.y); rv[3 * r + 2] = f2_hsum(ra.z);
             }
         }
     }
@@ -471,16 +510,31 @@ struct CombineSmem {
     double m[kWarps][kNM];
 };
 
+// Lanes l and l ^ 16 hold column-side partials of the same 8 columns (over different rows).  Adds them once, own + partner's
+// (commutative, so both lanes of a column would round alike), and leaves lane l with the two pairs of columns 4l .. 4l+3:
+// lanes 0-15 keep their low 64 columns, lanes 16-31 their high ones.  All 32 lanes must call it.
+__device__ __forceinline__ void fold_columns(const Acc& a, int lane, f2 (&gx)[2], f2 (&gy)[2], f2 (&gz)[2]) {
+    const bool hi = lane & 16;
+#pragma unroll
+    for (int q = 0; q < 2; ++q) {
+        gx[q] = f2_add(hi ? a.gx[2 + q] : a.gx[q], __shfl_xor_sync(0xffffffffu, hi ? a.gx[q] : a.gx[2 + q], 16));
+        gy[q] = f2_add(hi ? a.gy[2 + q] : a.gy[q], __shfl_xor_sync(0xffffffffu, hi ? a.gy[q] : a.gy[2 + q], 16));
+        gz[q] = f2_add(hi ? a.gz[2 + q] : a.gz[q], __shfl_xor_sync(0xffffffffu, hi ? a.gz[q] : a.gz[2 + q], 16));
+    }
+}
+
 // warp-level part of the CTA combine: park this warp's gradients / moments in shared memory
 template <uint32_t MODE, bool ROWS = false>
 __device__ __forceinline__ void park_warp(const Acc& a, CombineSmem& S, int warp, int lane) {
     if constexpr (has_grad(MODE)) {
+        f2 gx[2], gy[2], gz[2];
+        fold_columns(a, lane, gx, gy, gz);
 #pragma unroll
         for (int p = 0; p < 2; ++p) {
             float x0, x1, y0, y1, z0, z1;
-            f2_unpack(a.gx[p], x0, x1);
-            f2_unpack(a.gy[p], y0, y1);
-            f2_unpack(a.gz[p], z0, z1);
+            f2_unpack(gx[p], x0, x1);
+            f2_unpack(gy[p], y0, y1);
+            f2_unpack(gz[p], z0, z1);
             float* dst = &S.g[warp][(lane * 4 + 2 * p) * 3];
             dst[0] = x0; dst[1] = y0; dst[2] = z0;
             dst[3] = x1; dst[4] = y1; dst[5] = z1;
@@ -738,7 +792,8 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_lane_kernel(con
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int strip = blockIdx.x, chunk = blockIdx.y;
     const int n = P.n;
-    const int col0 = strip * kCols + lane * 4;
+    const int col0 = lane_col0(strip, lane);
+    const int hr = (lane >> 4) * kR;  // first group row of this lane's half-warp
     int row_begin, nrows;
     const int count = chunk_rows(P, strip, chunk, row_begin, nrows);
     if (chunk >= count || nrows <= 0) return;  // unstaggered strips leave the extra chunk slot empty
@@ -748,8 +803,9 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_lane_kernel(con
     Acc a;
     acc_zero(a);
     const PearsonCoef pc = pearson_coef<MODE>(P.pmom, n, P.c_mse, P.dyn_alpha);
-    const bool can_load = col0 + 3 < P.pitch;  // pitch is a multiple of 4 (0 for the implicit target)
-    const float* tbase = P.target + (size_t)(row_begin - P.r0) * P.pitch + col0;
+    // the lane's low / high 4 columns lie inside the pitch (a multiple of 4; 0 for the implicit target)
+    const bool can_load[2] = {col0 + 3 < P.pitch, col0 + kCols / 2 + 3 < P.pitch};
+    const float* tbase = P.target + (size_t)(row_begin - P.r0 + hr) * P.pitch + col0;
     const int strip_lo = strip * kCols, strip_hi = strip_lo + kCols - 1;
     const float f = P.fill;
     for (int p0 = 0; p0 < nrows; p0 += kStageRows) {
@@ -766,32 +822,28 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_lane_kernel(con
         for (int g = warp; g < ngroups; g += kWarps) {
             const int rl = p0 + g * kU, rg = row_begin + rl;
             const int rows_here = min(kU, nrows - rl);
-            float4 t[kU];
+            const XiPtr xi{s_xy + g * kU, s_z + g * kU};
+            float* const rowdst = ROWS ? P.rpart + (size_t)strip * P.rpitch + (size_t)(rg - P.r0) * 3 : nullptr;
             if constexpr (IMPLICIT) {
-#pragma unroll
-                for (int u = 0; u < kU; ++u) t[u] = make_float4(f, f, f, f);
-                if (rg + kU - 1 >= strip_lo && rg <= strip_hi) {  // the group touches the diagonal: t_ii = 0
-#pragma unroll
-                    for (int u = 0; u < kU; ++u) {
-                        const int dc = rg + u - col0;
-                        if (dc == 0) t[u].x = 0.f;
-                        if (dc == 1) t[u].y = 0.f;
-                        if (dc == 2) t[u].z = 0.f;
-                        if (dc == 3) t[u].w = 0.f;
-                    }
-                }
+                const TileFill t{f, rg + hr - col0, rg + kU - 1 >= strip_lo && rg <= strip_hi};
+                process_group<MODE, ROWS>(a, c, t, xi, rows_here, rg, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1, rowdst, lane, pc);
             } else {
-                if (rows_here == kU && can_load) {
+                TileRegs t;
+                if (rows_here == kU && can_load[1]) {
 #pragma unroll
-                    for (int u = 0; u < kU; ++u) t[u] = ldg_stream_f4(tbase + (size_t)(rl + u) * P.pitch);
+                    for (int r = 0; r < kR; ++r)
+#pragma unroll
+                        for (int h = 0; h < 2; ++h) t.t[r][h] = ldg_stream_f4(tbase + (size_t)(rl + r) * P.pitch + h * (kCols / 2));
                 } else {
 #pragma unroll
-                    for (int u = 0; u < kU; ++u)
-                        t[u] = (u < rows_here && can_load) ? ldg_stream_f4(tbase + (size_t)(rl + u) * P.pitch) : make_float4(0.f, 0.f, 0.f, 0.f);
+                    for (int r = 0; r < kR; ++r)
+#pragma unroll
+                        for (int h = 0; h < 2; ++h)
+                            t.t[r][h] = (hr + r < rows_here && can_load[h]) ? ldg_stream_f4(tbase + (size_t)(rl + r) * P.pitch + h * (kCols / 2))
+                                                                            : make_float4(0.f, 0.f, 0.f, 0.f);
                 }
+                process_group<MODE, ROWS>(a, c, t, xi, rows_here, rg, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1, rowdst, lane, pc);
             }
-            process_group<MODE, ROWS>(a, c, t, XiPtr{s_xy + g * kU, s_z + g * kU}, rows_here, rg, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1,
-                                      ROWS ? P.rpart + (size_t)strip * P.rpitch + (size_t)(rg - P.r0) * 3 : nullptr, lane, pc);
         }
     }
     park_warp<MODE, ROWS>(a, S, warp, lane);
@@ -954,6 +1006,15 @@ __device__ __forceinline__ void XiAddr::load(int u, float4& oxy, float2& oz) con
     oxy = lds_f4(xy + u * 16);
     oz = lds_f2(z + u * 8);
 }
+__device__ __forceinline__ void TileAddr::load(int r, float4& lo, float4& hi) const {
+    lo = lds_f4(base + r * (kCols * 4));
+    hi = lds_f4(base + r * (kCols * 4) + (kCols / 2) * 4);
+}
+// the lane's TileAddr in a ring slot (8 rows x 128 columns, row-major): rows 4 * (lane / 16) + r, columns 4 * (lane % 16) + {0, 64}.
+// Each ld.shared.v4 reads 256 contiguous bytes per half-warp: no bank conflicts.
+__device__ __forceinline__ TileAddr tile_addr(uint32_t slot, int lane) {
+    return TileAddr{slot + (uint32_t)((lane >> 4) * kR * (kCols * 4) + (lane & 15) * 16)};
+}
 __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, int c0, int c1, uint64_t* bar) {
     asm volatile(
         "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(smem_u32(dst)),
@@ -982,7 +1043,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_kernel(cons
     const int count = chunk_rows(P, strip, chunk, row_begin, nrows);
     if (chunk >= count || nrows <= 0) return;  // unstaggered strips leave the extra chunk slot empty; upper mode clips strips at the diagonal
     const int ntiles = (nrows + kTileRows - 1) / kTileRows;
-    const int col0 = strip * kCols + lane * 4;
+    const int col0 = lane_col0(strip, lane);
     const bool edge = (strip + 1) * kCols > n;
     const int strip_lo = strip * kCols, strip_hi = strip_lo + kCols - 1;
     unsigned char* wring = ring + (size_t)warp * (kStages * kSlotBytes);   // this warp's slots
@@ -1037,11 +1098,8 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_kernel(cons
         const uint32_t slot = wring_s + s * kSlotBytes;
         const XiAddr xi{slot + kSubTileBytes, slot + kSubTileBytes + kU * 16};
         const int rows_here = max(0, min(kU, nrows - (t * kTileRows + wrow)));
-        float4 tv[kU];
-#pragma unroll
-        for (int u = 0; u < kU; ++u) tv[u] = lds_f4(slot + lane * 16 + u * (kCols * 4));
         const int rg = row_begin + t * kTileRows + wrow;
-        process_group<MODE, ROWS>(a, c, tv, xi, rows_here, rg, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1,
+        process_group<MODE, ROWS>(a, c, tile_addr(slot, lane), xi, rows_here, rg, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1,
                                   ROWS ? P.rpart + (size_t)strip * P.rpitch + (size_t)(rg - P.r0) * 3 : nullptr, lane, pc);
         __syncwarp();  // every lane is done with slot s
         if (refill) {
@@ -1143,7 +1201,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_persist_ker
     __syncwarp();
     for (int it = 0; cur < P.nitems; ++it) {
         const int ntiles = (nrows + kTileRows - 1) / kTileRows;
-        const int col0 = strip * kCols + lane * 4;
+        const int col0 = lane_col0(strip, lane);
         const bool edge = (strip + 1) * kCols > n;
         const int strip_lo = strip * kCols, strip_hi = strip_lo + kCols - 1;
         ColumnRegs c;
@@ -1160,11 +1218,8 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_persist_ker
             const uint32_t slot = wring_s + s * kSlotBytes;
             const XiAddr xi{slot + kSubTileBytes, slot + kSubTileBytes + kU * 16};
             const int rows_here = max(0, min(kU, nrows - (t * kTileRows + wrow)));
-            float4 tv[kU];
-#pragma unroll
-            for (int u = 0; u < kU; ++u) tv[u] = lds_f4(slot + lane * 16 + u * (kCols * 4));
             const int rg = row_begin + t * kTileRows + wrow;
-            process_group<MODE, ROWS>(a, c, tv, xi, rows_here, rg, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1,
+            process_group<MODE, ROWS>(a, c, tile_addr(slot, lane), xi, rows_here, rg, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1,
                                       ROWS ? P.rpart + (size_t)strip * P.rpitch + (size_t)(rg - P.r0) * 3 : nullptr, lane, pc);
             __syncwarp();  // every lane is done with slot s
             if (refill) issue(strip, row_begin, t + kStages, g + kStages, xi_next);
@@ -1201,11 +1256,13 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_persist_ker
         }
         float gv[2][6];
         if constexpr (has_grad(MODE)) {
+            f2 gx[2], gy[2], gz[2];
+            fold_columns(a, lane, gx, gy, gz);
 #pragma unroll
             for (int p = 0; p < 2; ++p) {
-                f2_unpack(a.gx[p], gv[p][0], gv[p][3]);
-                f2_unpack(a.gy[p], gv[p][1], gv[p][4]);
-                f2_unpack(a.gz[p], gv[p][2], gv[p][5]);
+                f2_unpack(gx[p], gv[p][0], gv[p][3]);
+                f2_unpack(gy[p], gv[p][1], gv[p][4]);
+                f2_unpack(gz[p], gv[p][2], gv[p][5]);
             }
             if (warp >= kWarps / 2) {
 #pragma unroll
@@ -1332,7 +1389,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_warp_kernel
         const int nrows = (int)take;
         const int row_begin = P.r0 + row_lo;
         const int ntiles = (nrows + kU - 1) / kU;
-        const int col0 = strip * kCols + lane * 4;
+        const int col0 = lane_col0(strip, lane);
         const bool edge = (strip + 1) * kCols > n;
         const int strip_lo = strip * kCols, strip_hi = strip_lo + kCols - 1;
         auto xi_fetch = [&](int t) -> float {
@@ -1363,11 +1420,8 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_warp_kernel
             const uint32_t slot = wring_s + s * kSlotBytes;
             const XiAddr xi{slot + kSubTileBytes, slot + kSubTileBytes + kU * 16};
             const int rows_here = min(kU, nrows - t * kU);
-            float4 tv[kU];
-#pragma unroll
-            for (int u = 0; u < kU; ++u) tv[u] = lds_f4(slot + lane * 16 + u * (kCols * 4));
             const int rg = row_begin + t * kU;
-            process_group<MODE, ROWS>(a, c, tv, xi, rows_here, rg, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1,
+            process_group<MODE, ROWS>(a, c, tile_addr(slot, lane), xi, rows_here, rg, col0, n, edge, strip_lo, strip_hi, P.c_mse, P.c_l1,
                                       ROWS ? P.rpart + (size_t)strip * P.rpitch + (size_t)(rg - P.r0) * 3 : nullptr, lane, pc);
             __syncwarp();
             if (refill) issue(t + kStages, g + kStages, xi_next);
@@ -1378,9 +1432,11 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) pairloss_tma_warp_kernel
         const size_t slot_id = (size_t)seg * P.nstrips + strip;
         if constexpr (has_grad(MODE)) {
             float* gp = P.gpart + slot_id * (kCols * 3) + lane * 12;
+            f2 gx[2], gy[2], gz[2];
+            fold_columns(a, lane, gx, gy, gz);
             float x0, x1, y0, y1, z0, z1, x2, x3, y2, y3, z2, z3;
-            f2_unpack(a.gx[0], x0, x1); f2_unpack(a.gy[0], y0, y1); f2_unpack(a.gz[0], z0, z1);
-            f2_unpack(a.gx[1], x2, x3); f2_unpack(a.gy[1], y2, y3); f2_unpack(a.gz[1], z2, z3);
+            f2_unpack(gx[0], x0, x1); f2_unpack(gy[0], y0, y1); f2_unpack(gz[0], z0, z1);
+            f2_unpack(gx[1], x2, x3); f2_unpack(gy[1], y2, y3); f2_unpack(gz[1], z2, z3);
             __stcg(reinterpret_cast<float4*>(gp), make_float4(x0, y0, z0, x1));
             __stcg(reinterpret_cast<float4*>(gp) + 1, make_float4(y1, z1, x2, y2));
             __stcg(reinterpret_cast<float4*>(gp) + 2, make_float4(z2, x3, y3, z3));
