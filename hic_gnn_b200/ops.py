@@ -6,6 +6,7 @@ path.  Reference call sites are cited on each wrapper.
 from __future__ import annotations
 
 import os
+import weakref
 
 import torch
 
@@ -562,33 +563,41 @@ def ln_relu_add(x: torch.Tensor, norm: torch.nn.LayerNorm, residual: torch.Tenso
 
 # ------------------------------------------------------------------------------ Linear layers on the tcgen05 tensor cores (3xTF32)
 TF32X3_MIN_ROWS = int(os.environ.get("HICGAT_TF32X3_MIN_ROWS", "4096"))  # below this the cuBLAS fp32 GEMM is launch-bound anyway
+# Memo of splits, keyed on the source tensor OBJECT (plus its address, version, shape, pattern): the constant input features are
+# split once per pattern for as long as the features tensor lives, and two Linear layers that read the same activation (densea /
+# align_densea) share one split.  An entry holds only a weak reference to its source and is dropped when the source dies, so the
+# memo holds no more than the splits of live tensors.
 _split_cache: dict = {}
 
 
-def split_tf32(x: torch.Tensor, pattern: int, transpose: bool = False, cache: bool = False) -> torch.Tensor:
+def _drop_split(key, ref) -> None:
+    hit = _split_cache.get(key)
+    if hit is not None and hit[0] is ref:
+        del _split_cache[key]
+
+
+def split_tf32(x: torch.Tensor, pattern: int, transpose: bool = False, memo: bool = False) -> torch.Tensor:
     """``hicgat_split_tf32``: ``[s0 | s1 | s2]`` along the reduction dimension, ``s_p`` = hi or lo TF32 part by bit p of ``pattern``
-    (0b100 for the left operand, 0b010 for the right one).  ``cache``: memoise for a constant tensor (the input features)."""
+    (0b100 for the left operand, 0b010 for the right one).  ``memo``: reuse the split of this same tensor object (a Linear input
+    that other layers or steps read again) -- outside CUDA-graph capture only."""
     _cuda(x)
     if x.dtype != torch.float32 or x.dim() != 2 or x.stride(1) != 1:
         raise RuntimeError("split_tf32 expects a row-major float32 CUDA matrix")
+    # While a graph is captured the memo is neither read nor written: a hit would make the graph read a buffer that it does not own
+    # (freed and reused behind its back), and an entry made during capture is a buffer of the graph's pool that only its replays fill.
+    memo = memo and not torch.cuda.is_current_stream_capturing()
     key = (x.data_ptr(), x._version, tuple(x.shape), x.stride(0), pattern, transpose)
-    hit = _split_cache.get(key)
-    if hit is not None and hit[0] is x:  # the entry holds a reference to its source, so the address cannot have been recycled
-        return hit[1]
+    if memo:
+        hit = _split_cache.get(key)
+        if hit is not None and hit[0]() is x:
+            return hit[1]
     rows, cols = x.shape
     red = rows if transpose else cols
     kpad = (red + 31) // 32 * 32
     out = torch.empty(cols if transpose else rows, 3 * kpad, dtype=torch.float32, device=x.device)
     N.check(N.lib().hicgat_split_tf32(x.data_ptr(), rows, cols, x.stride(0), out.data_ptr(), pattern, int(transpose), _stream()), "hicgat_split_tf32")
-    # memo: constant tensors (`cache`: the input features, split once per run) and, briefly, the latest activations (two Linear
-    # layers that read the same tensor -- densea / align_densea -- share one split)
-    if not cache:
-        for k in [k for k, v in _split_cache.items() if not v[2]]:
-            if len(_split_cache) > 6:
-                del _split_cache[k]
-    elif len(_split_cache) > 12:
-        _split_cache.clear()
-    _split_cache[key] = (x, out, cache)
+    if memo:
+        _split_cache[key] = (weakref.ref(x, lambda ref, key=key: _drop_split(key, ref)), out)
     return out
 
 
@@ -613,7 +622,7 @@ class _Linear3xTF32(torch.autograd.Function):
     def forward(ctx, x, weight, bias):
         x = x.contiguous()
         w = weight.detach().contiguous()
-        y = gemm_tf32_tn(split_tf32(x.detach(), 0b100, cache=not x.requires_grad), split_tf32(w, 0b010), None if bias is None else bias.detach().contiguous())
+        y = gemm_tf32_tn(split_tf32(x, 0b100, memo=True), split_tf32(w, 0b010), None if bias is None else bias.detach().contiguous())
         ctx.save_for_backward(x, w)
         ctx.has_bias = bias is not None
         return y
@@ -626,7 +635,7 @@ class _Linear3xTF32(torch.autograd.Function):
         if ctx.needs_input_grad[0]:  # dx[m, k] = dy[m, n] . (W^T)[k, n]^T : reduction over the output features
             gx = gemm_tf32_tn(split_tf32(gy, 0b100), split_tf32(w, 0b010, transpose=True))
         if ctx.needs_input_grad[1]:  # dW[n, k] = (dy^T)[n, m] . (x^T)[k, m]^T : reduction over the rows
-            gw = gemm_tf32_tn(split_tf32(gy, 0b100, transpose=True), split_tf32(x, 0b010, transpose=True, cache=not x.requires_grad))
+            gw = gemm_tf32_tn(split_tf32(gy, 0b100, transpose=True), split_tf32(x, 0b010, transpose=True, memo=True))
         if ctx.has_bias and ctx.needs_input_grad[2]:
             gb = gy.sum(dim=0)
         return gx, gw, gb

@@ -312,7 +312,8 @@ HICGAT_API int hicgat_pairdist_bwd(const float* coords, int64_t n, const float* 
  * heads / the GATConv projection (models.py:23-55, 634-691, 1020-1047) and its two backward GEMMs on large maps.
  *   hicgat_split_tf32: src [rows, cols] f32 (ld elements per row) -> dst = the three parts s0, s1, s2 interleaved per 32 elements
  *     along the REDUCTION dimension ([s0(0:32) | s1(0:32) | s2(0:32) | s0(32:64) | ...]), s_p = tf32(a) ("hi") or tf32(a - tf32(a))
- *     ("lo") by bit p of `pattern`:
+ *     ("lo") by bit p of `pattern`, tf32() being cvt.rna (round to nearest, ties away from zero).  Inputs must be finite with
+ *     |a| < (2 - 2^-11) 2^127: at and above that, tf32(a) rounds to +-inf, lo is -+inf and the product of the parts is NaN.
  *       transpose = 0: dst [rows, 3 kpad], reduction over the columns, kpad = cols rounded up to 32 (padding written as 0);
  *       transpose = 1: dst [cols, 3 kpad], reduction over the rows,    kpad = rows rounded up to 32.
  *     With A' = split(A, pattern 0b100) = [hi|hi|lo] and B' = split(B, pattern 0b010) = [hi|lo|hi],
@@ -323,7 +324,8 @@ HICGAT_API int hicgat_pairdist_bwd(const float* coords, int64_t n, const float* 
  *     k-blocks (the tensor core truncates on every accumulation step: one accumulator fed all 3K/8 steps is off by 5.8e-6 at K = 512
  *     and by 4e-5 at K = 50k); longer reductions run split-K with an f64 reduce;
  *     kparts = 1: plain TF32 GEMM.  tcgen05.mma kind::tf32, operands by TMA; split-K (deterministic reduce) when the output tiles
- *     alone cannot fill the chip: pass a workspace of hicgat_gemm_tf32_workspace_bytes(m, n, k) bytes.
+ *     alone cannot fill the chip: pass a workspace of hicgat_gemm_tf32_workspace_bytes(m, n, k, kparts) bytes (0 when one
+ *     split suffices; the plan depends on kparts).
  * ---------------------------------------------------------------------------------- */
 HICGAT_API int hicgat_split_tf32(const float* src, int64_t rows, int64_t cols, int64_t ld, float* dst, int pattern, int transpose,
                       hicgat_stream_t stream);
