@@ -61,9 +61,11 @@ SIGNATURES = {
     "hicgat_csr_add_self_loops_i32": (C.c_int, [_p, _p, _i64, _p, _p, _p]),
     "hicgat_sage_norm_values": (C.c_int, [_p, _p, _p, _i64, _p, _p, _p]),
     "hicgat_spmm_csr_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i64, _p, _p]),
+    "hicgat_spmm_csr_rows_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i64, _i64, _i64, _p, _p]),
     "hicgat_csr_transpose_perm": (C.c_int, [_p, _p, _i64, _p, _p]),
     "hicgat_gat_set_tuning": (C.c_int, [_i32, _i32]),
     "hicgat_gat_fwd": (C.c_int, [_p, _p, _i64, _i32, _i32, _p, _p, _p, _p, _f32, _p, _p, _p, _p, _p]),
+    "hicgat_gat_fwd_rows": (C.c_int, [_p, _p, _i64, _i64, _i64, _i64, _i32, _i32, _p, _p, _p, _p, _f32, _p, _p, _p, _p, _p]),
     "hicgat_gat_bwd_workspace_bytes": (_sz, [_i64, _i64, _i32, _i32]),
     "hicgat_gat_logits": (C.c_int, [_i64, _i32, _i32, _p, _p, _p, _p, _p, _p]),
     "hicgat_gat_dense_mask_words": (_sz, [_i64]),
@@ -83,6 +85,7 @@ SIGNATURES = {
     "hicgat_spmv_csr_f64": (C.c_int, [_p, _p, _p, _i64, _p, _p, _p]),
     "hicgat_kr_scale_round_f64": (C.c_int, [_p, _i64, _i64, _p, _p, _i64, _i32, _p]),
     "hicgat_gat_bwd_fused": (C.c_int, [_p, _p, _p, _i64, _i64, _i32, _i32, _p, _p, _p, _p, _f32, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
+    "hicgat_gat_bwd_fused_rows": (C.c_int, [_p, _p, _p, _i64, _i64, _i64, _i64, _i64, _i32, _i32, _p, _p, _p, _p, _f32, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
     "hicgat_gat_bwd": (C.c_int, [_p, _p, _p, _i64, _i64, _i32, _i32, _p, _p, _p, _f32, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
     "hicgat_node2vec_walks": (C.c_int, [_p, _p, _p, _p, _i64, _i64, _i32, _f32, _f32, _u64, _p, _p]),
     "hicgat_sgns_epoch": (C.c_int, [_p, _p, _i64, _i32, _p, _p, _i64, _i32, _i32, _i32, _f64, _f64, _i32, _i32, _u64, _i64, _p, _p, _p]),

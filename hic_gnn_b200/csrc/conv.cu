@@ -28,15 +28,24 @@ __device__ __forceinline__ void fma4(float4& acc, float a, const float4& v) {
 __device__ __forceinline__ float dot4(const float4& a, const float4& b) {
     return fmaf(a.x, b.x, fmaf(a.y, b.y, fmaf(a.z, b.z, a.w * b.w)));
 }
+// first k in [lo, hi) with col[k] >= v (col ascending on [lo, hi)), hi if none
+__device__ __forceinline__ int lower_bound_i32(const int32_t* __restrict__ col, int lo, int hi, int v) {
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (__ldg(col + mid) < v) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo;
+}
 
 // ------------------------------------------------------------------ weighted CSR SpMM
 template <int Q>
 __global__ void __launch_bounds__(256) spmm_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
-                                                   const float* __restrict__ w, const float* __restrict__ x, int n,
+                                                   const float* __restrict__ w, const float* __restrict__ x, int g0, int g1,
                                                    float* __restrict__ out) {
     constexpr int F = Q * 128;
-    const int i = blockIdx.x * kRowsPerCta + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-    if (i >= n) return;
+    const int i = g0 + blockIdx.x * kRowsPerCta + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (i >= g1) return;
     float4 acc[Q];
 #pragma unroll
     for (int q = 0; q < Q; ++q) acc[q] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -70,7 +79,7 @@ __global__ void __launch_bounds__(256) spmm_kernel(const int32_t* __restrict__ r
         }
     }
 #pragma unroll
-    for (int q = 0; q < Q; ++q) *reinterpret_cast<float4*>(out + (size_t)i * F + q * 128 + lane * 4) = acc[q];
+    for (int q = 0; q < Q; ++q) *reinterpret_cast<float4*>(out + (size_t)(i - g0) * F + q * 128 + lane * 4) = acc[q];
 }
 
 // ------------------------------------------------------------------ GAT: logit halves
@@ -106,10 +115,10 @@ template <int H, int Q, int W>
 __global__ void __launch_bounds__(W * 32) gat_fwd_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
                                                       const float* __restrict__ xl, const float* __restrict__ a_src,
                                                       const float* __restrict__ a_dst, const float* __restrict__ bias,
-                                                      float slope, int n, float* __restrict__ alpha, float* __restrict__ out) {
+                                                      float slope, int g0, int g1, float* __restrict__ alpha, float* __restrict__ out) {
     constexpr int F = Q * 128, QH = Q / H;
-    const int i = blockIdx.x * W + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-    if (i >= n) return;
+    const int i = g0 + blockIdx.x * W + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (i >= g1) return;
     const int rs = rowptr[i], re = rowptr[i + 1];
     float adst[H], m[H], s[H];
 #pragma unroll
@@ -419,18 +428,30 @@ __global__ void __launch_bounds__(256) gat_bwd_rowdot_kernel(const float* __rest
     }
 }
 
-template <int H, int Q, int W>
+// Row block [g0, g1) (kRows): only the targets i of the block contribute to source row jn.  The columns of row jn are sorted, so
+// they are the contiguous entries ranges[jn] = [lower_bound(g0), lower_bound(g1)) (gat_block_ranges_kernel).  alpha / dz / rowdot /
+// gout hold the block's entries / rows only: the host passes them offset back by rowptr[g0] entries / g0 rows, so that entry k and
+// row i index them unchanged.  kRows = false is the whole graph, without the range table.
+template <int H, int Q, int W, bool kRows>
 __global__ void __launch_bounds__(W * 32, 16 / W) gat_bwd_fused_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
                                                                const int32_t* __restrict__ perm, const float* __restrict__ xl,
                                                                const float* __restrict__ a_src, const float* __restrict__ a_dst,
                                                                const float* __restrict__ alpha, const float* __restrict__ rowdot,
                                                                const float* __restrict__ gout, const float* __restrict__ att_l, float slope,
-                                                               int n, float* __restrict__ dz, float* __restrict__ d_a_src,
-                                                               float* __restrict__ dxl) {
+                                                               int n, const int2* __restrict__ ranges, float* __restrict__ dz,
+                                                               float* __restrict__ d_a_src, float* __restrict__ dxl) {
     constexpr int F = Q * 128, QH = Q / H;
     const int jn = blockIdx.x * W + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (jn >= n) return;
-    const int rs = rowptr[jn], re = rowptr[jn + 1];
+    int rs, re;
+    if constexpr (kRows) {
+        const int2 r = ranges[jn];
+        rs = r.x;
+        re = r.y;
+    } else {
+        rs = rowptr[jn];
+        re = rowptr[jn + 1];
+    }
     float4 x[Q], acc[Q];
 #pragma unroll
     for (int q = 0; q < Q; ++q) {
@@ -528,14 +549,25 @@ __global__ void __launch_bounds__(W * 32, 16 / W) gat_bwd_fused_kernel(const int
     }
 }
 
-// d a_dst[i,h] = sum of the row's dz (contiguous), then dxl[i,:] += d a_dst[i,h] att_r
+// ranges[j] = the entries of row j whose column lies in [g0, g1): [lower_bound(g0), lower_bound(g1)) on the sorted columns
+__global__ void __launch_bounds__(256) gat_block_ranges_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, int n,
+                                                               int g0, int g1, int2* __restrict__ ranges) {
+    const int j = blockIdx.x * 256 + threadIdx.x;
+    if (j >= n) return;
+    const int rs = rowptr[j], re = rowptr[j + 1];
+    const int lo = lower_bound_i32(col, rs, re, g0);
+    ranges[j] = make_int2(lo, lower_bound_i32(col, lo, re, g1));
+}
+
+// d a_dst[i,h] = sum of the row's dz (contiguous), then dxl[i,:] += d a_dst[i,h] att_r; rows i of the block [g0, g1) (dz offset
+// back by the host like in gat_bwd_fused_kernel)
 template <int H, int Q>
 __global__ void __launch_bounds__(256) gat_bwd_dst_kernel(const int32_t* __restrict__ rowptr, const float* __restrict__ dz,
-                                                          const float* __restrict__ att_r, int n, float* __restrict__ d_a_dst,
+                                                          const float* __restrict__ att_r, int g0, int g1, float* __restrict__ d_a_dst,
                                                           float* __restrict__ dxl) {
     constexpr int F = Q * 128, QH = Q / H;
-    const int i = blockIdx.x * kRowsPerCta + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-    if (i >= n) return;
+    const int i = g0 + blockIdx.x * kRowsPerCta + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (i >= g1) return;
     const int rs = rowptr[i], re = rowptr[i + 1];
     float s[H];
 #pragma unroll
@@ -600,6 +632,32 @@ __global__ void __launch_bounds__(128) gat_bwd_param_kernel(const float* __restr
     }
 }
 
+// Stage A of a row block [g0, g1): datt_l runs over all n rows (d a_src is a partial sum on every row), datt_r and dbias over the
+// block's rows only (gout offset back by g0 rows by the host; d a_dst is read on the block's rows).  Same partial layout.
+__global__ void __launch_bounds__(128) gat_bwd_param_rows_kernel(const float* __restrict__ xl, const float* __restrict__ gout,
+                                                                 const float* __restrict__ d_a_src, const float* __restrict__ d_a_dst,
+                                                                 int n, int g0, int g1, int H, int C, float* __restrict__ part) {
+    const int F = H * C, nblk = gridDim.x, blk = blockIdx.x;
+    for (int c = threadIdx.x * 4; c < F; c += blockDim.x * 4) {
+        const int h = c / C;
+        float4 sl = make_float4(0.f, 0.f, 0.f, 0.f), sr = sl, sb = sl;
+        for (int r = blk; r < n; r += nblk) fma4(sl, d_a_src[r * H + h], __ldg(reinterpret_cast<const float4*>(xl + (size_t)r * F + c)));
+        for (int r = g0 + blk; r < g1; r += nblk) {
+            const float4 x0 = __ldg(reinterpret_cast<const float4*>(xl + (size_t)r * F + c));
+            const float4 g = __ldg(reinterpret_cast<const float4*>(gout + (size_t)r * F + c));
+            fma4(sr, d_a_dst[r * H + h], x0);
+            sb.x += g.x; sb.y += g.y; sb.z += g.z; sb.w += g.w;
+        }
+        const float vl[4] = {sl.x, sl.y, sl.z, sl.w}, vr[4] = {sr.x, sr.y, sr.z, sr.w}, vb[4] = {sb.x, sb.y, sb.z, sb.w};
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            part[((size_t)(0 * F + c + q)) * nblk + blk] = vl[q];
+            part[((size_t)(1 * F + c + q)) * nblk + blk] = vr[q];
+            part[((size_t)(2 * F + c + q)) * nblk + blk] = vb[q];
+        }
+    }
+}
+
 __global__ void __launch_bounds__(256) gat_bwd_param_reduce_kernel(const float* __restrict__ part, int nblk, int F,
                                                                    float* __restrict__ datt_l, float* __restrict__ datt_r, float* __restrict__ dbias) {
     const int o = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
@@ -630,7 +688,7 @@ void launch_gather(void (*kernel)(KArgs...), unsigned grid, unsigned block, cuda
     cfg.blockDim = dim3(block);
     cfg.stream = stream;
     cudaLaunchAttribute attr[1];
-    if (g_l2_persist_bytes > 0) {
+    if (g_l2_persist_bytes > 0 && bytes > 0) {
         attr[0].id = cudaLaunchAttributeAccessPolicyWindow;
         attr[0].val.accessPolicyWindow.base_ptr = const_cast<void*>(gathered);
         attr[0].val.accessPolicyWindow.num_bytes = bytes;
@@ -662,21 +720,39 @@ void launch_gather(void (*kernel)(KArgs...), unsigned grid, unsigned block, cuda
 
 using namespace hicgat;
 
-extern "C" int hicgat_spmm_csr_f32(const int32_t* rowptr, const int32_t* col, const float* w, const float* x, int64_t n,
-                                   int64_t f, float* out, hicgat_stream_t stream_) {
-    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-    HICGAT_REQUIRE(rowptr && col && w && x && out && n > 0 && n < (1ll << 31), "hicgat_spmm_csr_f32: bad arguments");
-    HICGAT_REQUIRE(aligned16(x) && aligned16(out), "hicgat_spmm_csr_f32: x/out must be 16-byte aligned");
-    const unsigned grid = (unsigned)((n + kRowsPerCta - 1) / kRowsPerCta);
+namespace {
+int spmm_rows(const char* fn, const int32_t* rowptr, const int32_t* col, const float* w, const float* x, int64_t n, int64_t g0, int64_t g1,
+              int64_t f, float* out, cudaStream_t stream) {
+    HICGAT_REQUIRE(rowptr && col && w && x && n > 0 && n < (1ll << 31), "%s: bad arguments", fn);
+    HICGAT_REQUIRE(0 <= g0 && g0 <= g1 && g1 <= n, "%s: bad row block [%lld, %lld) of n = %lld", fn, (long long)g0, (long long)g1, (long long)n);
+    HICGAT_REQUIRE(out || g0 == g1, "%s: null out", fn);
+    HICGAT_REQUIRE(aligned16(x) && aligned16(out), "%s: x/out must be 16-byte aligned", fn);
+    if (f != 128 && f != 256 && f != 512 && f != 1024) {
+        set_error("%s: feature width %lld not in {128,256,512,1024}", fn, (long long)f);
+        return HICGAT_ERR_INVALID;
+    }
+    if (g0 == g1) return HICGAT_OK;
+    const unsigned grid = (unsigned)((g1 - g0 + kRowsPerCta - 1) / kRowsPerCta);
     switch (f) {
-        case 128: spmm_kernel<1><<<grid, 256, 0, stream>>>(rowptr, col, w, x, (int)n, out); break;
-        case 256: spmm_kernel<2><<<grid, 256, 0, stream>>>(rowptr, col, w, x, (int)n, out); break;
-        case 512: spmm_kernel<4><<<grid, 256, 0, stream>>>(rowptr, col, w, x, (int)n, out); break;
-        case 1024: spmm_kernel<8><<<grid, 256, 0, stream>>>(rowptr, col, w, x, (int)n, out); break;
-        default: set_error("hicgat_spmm_csr_f32: feature width %lld not in {128,256,512,1024}", (long long)f); return HICGAT_ERR_INVALID;
+        case 128: spmm_kernel<1><<<grid, 256, 0, stream>>>(rowptr, col, w, x, (int)g0, (int)g1, out); break;
+        case 256: spmm_kernel<2><<<grid, 256, 0, stream>>>(rowptr, col, w, x, (int)g0, (int)g1, out); break;
+        case 512: spmm_kernel<4><<<grid, 256, 0, stream>>>(rowptr, col, w, x, (int)g0, (int)g1, out); break;
+        default: spmm_kernel<8><<<grid, 256, 0, stream>>>(rowptr, col, w, x, (int)g0, (int)g1, out); break;
     }
     HICGAT_CHECK_LAUNCH("spmm_kernel");
     return HICGAT_OK;
+}
+}  // namespace
+
+extern "C" int hicgat_spmm_csr_f32(const int32_t* rowptr, const int32_t* col, const float* w, const float* x, int64_t n,
+                                   int64_t f, float* out, hicgat_stream_t stream_) {
+    HICGAT_REQUIRE(out, "hicgat_spmm_csr_f32: bad arguments");
+    return spmm_rows("hicgat_spmm_csr_f32", rowptr, col, w, x, n, 0, n, f, out, static_cast<cudaStream_t>(stream_));
+}
+
+extern "C" int hicgat_spmm_csr_rows_f32(const int32_t* rowptr, const int32_t* col, const float* w, const float* x, int64_t n, int64_t g0,
+                                        int64_t g1, int64_t f, float* out, hicgat_stream_t stream_) {
+    return spmm_rows("hicgat_spmm_csr_rows_f32", rowptr, col, w, x, n, g0, g1, f, out, static_cast<cudaStream_t>(stream_));
 }
 
 extern "C" int hicgat_gat_set_tuning(int rows_per_cta, int l2_persist_mb) {
@@ -700,32 +776,55 @@ extern "C" int hicgat_gat_set_tuning(int rows_per_cta, int l2_persist_mb) {
     return HICGAT_OK;
 }
 
-extern "C" int hicgat_gat_fwd(const int32_t* rowptr, const int32_t* col, int64_t n, int heads, int channels, const float* xl,
-                              const float* att_l, const float* att_r, const float* bias, float slope, float* a_src,
-                              float* a_dst, float* alpha, float* out, hicgat_stream_t stream_) {
-    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-    HICGAT_REQUIRE(rowptr && col && xl && att_l && att_r && bias && a_src && a_dst && alpha && out, "hicgat_gat_fwd: null pointer");
-    HICGAT_REQUIRE(n > 0 && n < (1ll << 31), "hicgat_gat_fwd: bad n");
-    HICGAT_REQUIRE(gat_shape_supported(heads, channels), "hicgat_gat_fwd: unsupported heads=%d channels=%d", heads, channels);
-    HICGAT_REQUIRE(aligned16(xl) && aligned16(out) && aligned16(att_l) && aligned16(att_r) && aligned16(bias), "hicgat_gat_fwd: 16-byte alignment required");
+namespace {
+int gat_fwd_rows(const char* fn, const int32_t* rowptr, const int32_t* col, int64_t n, int64_t g0, int64_t g1, int64_t e0, int heads, int channels,
+                 const float* xl, const float* att_l, const float* att_r, const float* bias, float slope, float* a_src, float* a_dst,
+                 float* alpha, float* out, cudaStream_t stream) {
+    HICGAT_REQUIRE(rowptr && col && xl && att_l && att_r && bias && a_src && a_dst, "%s: null pointer", fn);
+    HICGAT_REQUIRE(n > 0 && n < (1ll << 31), "%s: bad n", fn);
+    HICGAT_REQUIRE(0 <= g0 && g0 <= g1 && g1 <= n && e0 >= 0, "%s: bad row block [%lld, %lld) of n = %lld", fn, (long long)g0, (long long)g1, (long long)n);
+    HICGAT_REQUIRE((alpha && out) || g0 == g1, "%s: null pointer", fn);
+    HICGAT_REQUIRE(gat_shape_supported(heads, channels), "%s: unsupported heads=%d channels=%d", fn, heads, channels);
+    HICGAT_REQUIRE(aligned16(xl) && aligned16(out) && aligned16(att_l) && aligned16(att_r) && aligned16(bias), "%s: 16-byte alignment required", fn);
     const unsigned grid = (unsigned)((n + kRowsPerCta - 1) / kRowsPerCta);
 #define CALL_LOGIT(H, Q) gat_logit_kernel<H, Q><<<grid, 256, 0, stream>>>(xl, att_l, att_r, (int)n, a_src, a_dst)
     HICGAT_DISPATCH_HQ(heads, channels, CALL_LOGIT);
 #undef CALL_LOGIT
     HICGAT_CHECK_LAUNCH("gat_logit_kernel");
+    if (g0 == g1) return HICGAT_OK;
+    const int64_t nb = g1 - g0;
+    // the kernel indexes entry k / row i of the whole graph: offset the block's arrays back by e0 entries / g0 rows
+    float* const alpha_b = alpha - e0 * heads;
+    float* const out_b = out - g0 * heads * channels;
     const size_t gathered_bytes = (size_t)n * heads * channels * sizeof(float);
 #define CALL_FWD(H, Q)                                                                                                                  \
-    if (g_gather_warps == 16) launch_gather(gat_fwd_kernel<H, Q, 16>, (unsigned)((n + 15) / 16), 512, stream, xl, gathered_bytes, rowptr, col, xl, a_src, a_dst, bias, slope, (int)n, alpha, out); \
-    else launch_gather(gat_fwd_kernel<H, Q, 8>, grid, 256, stream, xl, gathered_bytes, rowptr, col, xl, a_src, a_dst, bias, slope, (int)n, alpha, out)
+    if (g_gather_warps == 16) launch_gather(gat_fwd_kernel<H, Q, 16>, (unsigned)((nb + 15) / 16), 512, stream, xl, gathered_bytes, rowptr, col, xl, a_src, a_dst, bias, slope, (int)g0, (int)g1, alpha_b, out_b); \
+    else launch_gather(gat_fwd_kernel<H, Q, 8>, (unsigned)((nb + kRowsPerCta - 1) / kRowsPerCta), 256, stream, xl, gathered_bytes, rowptr, col, xl, a_src, a_dst, bias, slope, (int)g0, (int)g1, alpha_b, out_b)
     HICGAT_DISPATCH_HQ(heads, channels, CALL_FWD);
 #undef CALL_FWD
     HICGAT_CHECK_LAUNCH("gat_fwd_kernel");
     return HICGAT_OK;
 }
+}  // namespace
+
+extern "C" int hicgat_gat_fwd(const int32_t* rowptr, const int32_t* col, int64_t n, int heads, int channels, const float* xl,
+                              const float* att_l, const float* att_r, const float* bias, float slope, float* a_src,
+                              float* a_dst, float* alpha, float* out, hicgat_stream_t stream_) {
+    HICGAT_REQUIRE(alpha && out, "hicgat_gat_fwd: null pointer");
+    return gat_fwd_rows("hicgat_gat_fwd", rowptr, col, n, 0, n, 0, heads, channels, xl, att_l, att_r, bias, slope, a_src, a_dst, alpha, out,
+                        static_cast<cudaStream_t>(stream_));
+}
+
+extern "C" int hicgat_gat_fwd_rows(const int32_t* rowptr, const int32_t* col, int64_t n, int64_t g0, int64_t g1, int64_t e0, int heads, int channels,
+                                   const float* xl, const float* att_l, const float* att_r, const float* bias, float slope, float* a_src,
+                                   float* a_dst, float* alpha, float* out, hicgat_stream_t stream_) {
+    return gat_fwd_rows("hicgat_gat_fwd_rows", rowptr, col, n, g0, g1, e0, heads, channels, xl, att_l, att_r, bias, slope, a_src, a_dst, alpha, out,
+                        static_cast<cudaStream_t>(stream_));
+}
 
 namespace {
 struct BwdLayout {
-    size_t off_dz, off_dsrc, off_ddst, off_rowdot, off_part, off_counter, total;
+    size_t off_dz, off_dsrc, off_ddst, off_rowdot, off_part, off_ranges, off_counter, total;
     int nchunks;
 };
 BwdLayout bwd_layout(int64_t n, int64_t nnz, int H, int C) {
@@ -738,7 +837,8 @@ BwdLayout bwd_layout(int64_t n, int64_t nnz, int H, int C) {
     L.off_ddst = L.off_dsrc + align_up(sizeof(float) * (size_t)n * H, 256);
     L.off_rowdot = L.off_ddst + align_up(sizeof(float) * (size_t)n * H, 256);
     L.off_part = L.off_rowdot + align_up(sizeof(float) * (size_t)n * H, 256);
-    L.total = L.off_part + sizeof(float) * 3 * F * (size_t)param_ctas(n);
+    L.off_ranges = L.off_part + align_up(sizeof(float) * 3 * F * (size_t)param_ctas(n), 256);
+    L.total = L.off_ranges + sizeof(int2) * (size_t)n;  // row-block calls only
     return L;
 }
 }  // namespace
@@ -786,21 +886,23 @@ extern "C" int hicgat_gat_bwd(const int32_t* rowptr, const int32_t* col, const i
     return HICGAT_OK;
 }
 
-extern "C" int hicgat_gat_bwd_fused(const int32_t* rowptr, const int32_t* col, const int32_t* perm, int64_t n, int64_t nnz, int heads,
-                                    int channels, const float* xl, const float* att_l, const float* att_r, const float* bias, float slope,
-                                    const float* a_src, const float* a_dst, const float* alpha, const float* out, const float* gout,
-                                    float* dxl, float* datt_l, float* datt_r, float* dbias, void* workspace, size_t workspace_bytes,
-                                    hicgat_stream_t stream_) {
-    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-    HICGAT_REQUIRE(rowptr && col && perm && xl && att_l && att_r && bias && a_src && a_dst && alpha && out && gout && dxl && datt_l && datt_r && dbias && workspace,
-                   "hicgat_gat_bwd_fused: null pointer");
-    HICGAT_REQUIRE(n > 0 && n < (1ll << 31) && nnz >= 0 && nnz < (1ll << 31), "hicgat_gat_bwd_fused: bad n/nnz");
-    HICGAT_REQUIRE(gat_shape_supported(heads, channels), "hicgat_gat_bwd_fused: unsupported heads=%d channels=%d", heads, channels);
+namespace {
+int gat_bwd_fused_rows(const char* fn, const int32_t* rowptr, const int32_t* col, const int32_t* perm, int64_t n, int64_t nnz, int64_t g0,
+                       int64_t g1, int64_t e0, int heads, int channels, const float* xl, const float* att_l, const float* att_r, const float* bias,
+                       float slope, const float* a_src, const float* a_dst, const float* alpha, const float* out, const float* gout,
+                       float* dxl, float* datt_l, float* datt_r, float* dbias, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+    HICGAT_REQUIRE(rowptr && col && perm && xl && att_l && att_r && bias && a_src && a_dst && dxl && datt_l && datt_r && dbias && workspace,
+                   "%s: null pointer", fn);
+    HICGAT_REQUIRE(n > 0 && n < (1ll << 31) && nnz >= 0 && nnz < (1ll << 31), "%s: bad n/nnz", fn);
+    HICGAT_REQUIRE(0 <= g0 && g0 <= g1 && g1 <= n && 0 <= e0 && e0 <= nnz, "%s: bad row block [%lld, %lld) of n = %lld", fn, (long long)g0, (long long)g1,
+                   (long long)n);
+    HICGAT_REQUIRE((alpha && out && gout) || g0 == g1, "%s: null pointer", fn);
+    HICGAT_REQUIRE(gat_shape_supported(heads, channels), "%s: unsupported heads=%d channels=%d", fn, heads, channels);
     HICGAT_REQUIRE(aligned16(xl) && aligned16(gout) && aligned16(out) && aligned16(dxl) && aligned16(att_l) && aligned16(att_r) && aligned16(bias),
-                   "hicgat_gat_bwd_fused: 16-byte alignment required");
+                   "%s: 16-byte alignment required", fn);
     const BwdLayout L = bwd_layout(n, nnz, heads, channels);
     if (workspace_bytes < L.total) {
-        set_error("hicgat_gat_bwd_fused: workspace %zu < required %zu", workspace_bytes, L.total);
+        set_error("%s: workspace %zu < required %zu", fn, workspace_bytes, L.total);
         return HICGAT_ERR_WORKSPACE;
     }
     unsigned char* ws = static_cast<unsigned char*>(workspace);
@@ -809,28 +911,74 @@ extern "C" int hicgat_gat_bwd_fused(const int32_t* rowptr, const int32_t* col, c
     float* ddst = reinterpret_cast<float*>(ws + L.off_ddst);
     float* rowdot = reinterpret_cast<float*>(ws + L.off_rowdot);
     float* part = reinterpret_cast<float*>(ws + L.off_part);
-    const unsigned grid = (unsigned)((n + kRowsPerCta - 1) / kRowsPerCta);
-#define CALL_ROWDOT(H, Q) gat_bwd_rowdot_kernel<H, Q><<<grid, 256, 0, stream>>>(gout, out, bias, (int)n, rowdot)
-    HICGAT_DISPATCH_HQ(heads, channels, CALL_ROWDOT);
+    const int64_t nb = g1 - g0, F = (int64_t)heads * channels;
+    // the kernels index entry k / row i of the whole graph: the block's arrays are offset back by e0 entries / g0 rows
+    const float* const alpha_b = alpha - e0 * heads;
+    const float* const gout_b = gout - g0 * F;
+    float* const dz_b = dz - e0 * heads;
+    float* const rowdot_b = rowdot - g0 * heads;
+    const bool whole = g0 == 0 && g1 == n;
+    int2* const ranges = reinterpret_cast<int2*>(ws + L.off_ranges);
+    const unsigned grid = (unsigned)((n + kRowsPerCta - 1) / kRowsPerCta), grid_b = (unsigned)((nb + kRowsPerCta - 1) / kRowsPerCta);
+    if (nb > 0) {  // the block's rows: rowdot [nb, H] from the block's gout / out
+#define CALL_ROWDOT(H, Q) gat_bwd_rowdot_kernel<H, Q><<<grid_b, 256, 0, stream>>>(gout, out, bias, (int)nb, rowdot)
+        HICGAT_DISPATCH_HQ(heads, channels, CALL_ROWDOT);
 #undef CALL_ROWDOT
-    HICGAT_CHECK_LAUNCH("gat_bwd_rowdot_kernel");
-    const size_t gathered_bytes = (size_t)n * heads * channels * sizeof(float);
+        HICGAT_CHECK_LAUNCH("gat_bwd_rowdot_kernel");
+    }
+    if (!whole) {
+        gat_block_ranges_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(rowptr, col, (int)n, (int)g0, (int)g1, ranges);
+        HICGAT_CHECK_LAUNCH("gat_block_ranges_kernel");
+    }
+    // every source row j (dxl and d a_src are partial sums over the block's targets when the block is not all rows)
+    const size_t gathered_bytes = (size_t)nb * heads * channels * sizeof(float);
+#define LAUNCH_FUSED(H, Q, W, R, G, B) launch_gather(gat_bwd_fused_kernel<H, Q, W, R>, G, B, stream, gout, gathered_bytes, rowptr, col, perm, xl, a_src, a_dst, alpha_b, rowdot_b, gout_b, att_l, slope, (int)n, ranges, dz_b, dsrc, dxl)
 #define CALL_FUSED(H, Q)                                                                                                                \
-    if (g_gather_warps == 16) launch_gather(gat_bwd_fused_kernel<H, Q, 16>, (unsigned)((n + 15) / 16), 512, stream, gout, gathered_bytes, rowptr, col, perm, xl, a_src, a_dst, alpha, rowdot, gout, att_l, slope, (int)n, dz, dsrc, dxl); \
-    else launch_gather(gat_bwd_fused_kernel<H, Q, 8>, grid, 256, stream, gout, gathered_bytes, rowptr, col, perm, xl, a_src, a_dst, alpha, rowdot, gout, att_l, slope, (int)n, dz, dsrc, dxl)
+    if (g_gather_warps == 16 && whole) LAUNCH_FUSED(H, Q, 16, false, (unsigned)((n + 15) / 16), 512);                                   \
+    else if (g_gather_warps == 16) LAUNCH_FUSED(H, Q, 16, true, (unsigned)((n + 15) / 16), 512);                                        \
+    else if (whole) LAUNCH_FUSED(H, Q, 8, false, grid, 256);                                                                            \
+    else LAUNCH_FUSED(H, Q, 8, true, grid, 256)
     HICGAT_DISPATCH_HQ(heads, channels, CALL_FUSED);
 #undef CALL_FUSED
+#undef LAUNCH_FUSED
     HICGAT_CHECK_LAUNCH("gat_bwd_fused_kernel");
-#define CALL_DST(H, Q) gat_bwd_dst_kernel<H, Q><<<grid, 256, 0, stream>>>(rowptr, dz, att_r, (int)n, ddst, dxl)
-    HICGAT_DISPATCH_HQ(heads, channels, CALL_DST);
+    if (nb > 0) {
+#define CALL_DST(H, Q) gat_bwd_dst_kernel<H, Q><<<grid_b, 256, 0, stream>>>(rowptr, dz_b, att_r, (int)g0, (int)g1, ddst, dxl)
+        HICGAT_DISPATCH_HQ(heads, channels, CALL_DST);
 #undef CALL_DST
-    HICGAT_CHECK_LAUNCH("gat_bwd_dst_kernel");
+        HICGAT_CHECK_LAUNCH("gat_bwd_dst_kernel");
+    }
     const int nblk = param_ctas(n);
-    gat_bwd_param_kernel<<<nblk, 128, 0, stream>>>(xl, gout, dsrc, ddst, (int)n, heads, channels, part);
-    HICGAT_CHECK_LAUNCH("gat_bwd_param_kernel");
+    if (g0 == 0 && g1 == n) {
+        gat_bwd_param_kernel<<<nblk, 128, 0, stream>>>(xl, gout, dsrc, ddst, (int)n, heads, channels, part);
+        HICGAT_CHECK_LAUNCH("gat_bwd_param_kernel");
+    } else {
+        gat_bwd_param_rows_kernel<<<nblk, 128, 0, stream>>>(xl, gout_b, dsrc, ddst, (int)n, (int)g0, (int)g1, heads, channels, part);
+        HICGAT_CHECK_LAUNCH("gat_bwd_param_rows_kernel");
+    }
     gat_bwd_param_reduce_kernel<<<(3 * heads * channels + 7) / 8, 256, 0, stream>>>(part, nblk, heads * channels, datt_l, datt_r, dbias);
     HICGAT_CHECK_LAUNCH("gat_bwd_param_reduce_kernel");
     return HICGAT_OK;
+}
+}  // namespace
+
+extern "C" int hicgat_gat_bwd_fused(const int32_t* rowptr, const int32_t* col, const int32_t* perm, int64_t n, int64_t nnz, int heads,
+                                    int channels, const float* xl, const float* att_l, const float* att_r, const float* bias, float slope,
+                                    const float* a_src, const float* a_dst, const float* alpha, const float* out, const float* gout,
+                                    float* dxl, float* datt_l, float* datt_r, float* dbias, void* workspace, size_t workspace_bytes,
+                                    hicgat_stream_t stream_) {
+    HICGAT_REQUIRE(alpha && out && gout, "hicgat_gat_bwd_fused: null pointer");
+    return gat_bwd_fused_rows("hicgat_gat_bwd_fused", rowptr, col, perm, n, nnz, 0, n, 0, heads, channels, xl, att_l, att_r, bias, slope, a_src, a_dst,
+                              alpha, out, gout, dxl, datt_l, datt_r, dbias, workspace, workspace_bytes, static_cast<cudaStream_t>(stream_));
+}
+
+extern "C" int hicgat_gat_bwd_fused_rows(const int32_t* rowptr, const int32_t* col, const int32_t* perm, int64_t n, int64_t nnz, int64_t g0,
+                                         int64_t g1, int64_t e0, int heads, int channels, const float* xl, const float* att_l, const float* att_r,
+                                         const float* bias, float slope, const float* a_src, const float* a_dst, const float* alpha,
+                                         const float* out, const float* gout, float* dxl, float* datt_l, float* datt_r, float* dbias,
+                                         void* workspace, size_t workspace_bytes, hicgat_stream_t stream_) {
+    return gat_bwd_fused_rows("hicgat_gat_bwd_fused_rows", rowptr, col, perm, n, nnz, g0, g1, e0, heads, channels, xl, att_l, att_r, bias, slope, a_src,
+                              a_dst, alpha, out, gout, dxl, datt_l, datt_r, dbias, workspace, workspace_bytes, static_cast<cudaStream_t>(stream_));
 }
 
 // ------------------------------------------------------------------ pieces shared with the dense-tile path (gat_dense.cu)

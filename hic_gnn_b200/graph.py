@@ -43,6 +43,7 @@ class CSRGraph:
         self.nnz = int(col.numel())
         self.storage = _Storage(self)
         self._cache: dict = {}
+        self.block: tuple[int, int] | None = None  # (g0, g1) of a row-block view, see row_block
 
     # -- SparseTensor-like surface ------------------------------------------------
     def sizes(self):
@@ -69,6 +70,29 @@ class CSRGraph:
         rowptr = torch.zeros(n + 1, dtype=torch.int64, device=row.device)
         rowptr[1:] = torch.cumsum(torch.bincount(row, minlength=n), 0)
         return cls(rowptr, col, val, n)
+
+    def row_block(self, g0: int, g1: int) -> "CSRGraph":
+        """View of target rows ``[g0, g1)`` for a GNN whose rows are sharded across GPUs: the conv layers given it take the
+        full input ``x [n, F]`` and return the block's ``g1 - g0`` rows (CSR kernels only).  It shares this graph's arrays and
+        its cache of derived index arrays, so blocks of one graph build them once."""
+        g0, g1 = int(g0), int(g1)
+        if not 0 <= g0 <= g1 <= self.n:
+            raise ValueError(f"CSRGraph.row_block: need 0 <= g0 <= g1 <= n = {self.n}, got [{g0}, {g1})")
+        view = object.__new__(CSRGraph)
+        view.__dict__.update(self.__dict__)
+        view.storage = _Storage(view)
+        view.block = (g0, g1)
+        return view
+
+    @property
+    def rows(self) -> tuple[int, int]:
+        """(g0, g1): the target rows the conv layers produce, ``(0, n)`` unless this is a row-block view."""
+        return self.block if self.block is not None else (0, self.n)
+
+    def block_entries(self) -> tuple[int, int]:
+        """(e0, e1): the block's entries ``[rowptr[g0] + g0, rowptr[g1] + g1)`` in the self-loop pattern (read once, cached)."""
+        g0, g1 = self.rows
+        return self._get(("block_entries", g0, g1), lambda: tuple(int(v) + g for v, g in zip(self.rowptr[[g0, g1]].tolist(), (g0, g1))))
 
     # -- derived arrays -----------------------------------------------------------
     def _get(self, key, builder):

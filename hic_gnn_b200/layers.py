@@ -44,6 +44,22 @@ class _SageAggregate(torch.autograd.Function):
         return dx, None
 
 
+def _sage_aggregate_rows(x, graph: CSRGraph):
+    """Rows ``[g0, g1)`` of ``D^-1 A x`` for a row-block view of the graph (``x`` holds all rows).  No backward: ``x`` is the
+    model input, which needs no gradient."""
+    _cuda(x)
+    if x.requires_grad:
+        raise NotImplementedError("SAGEConv on a row block: the aggregation has no backward (its input x must not require grad)")
+    x = x.contiguous().float()
+    g0, g1 = graph.rows
+    r32, c32 = graph.i32()
+    w, _ = graph.sage_weights()
+    out = torch.empty(g1 - g0, x.shape[1], dtype=torch.float32, device=x.device)
+    N.check(N.lib().hicgat_spmm_csr_rows_f32(r32.data_ptr(), _addr(c32), _addr(w), x.data_ptr(), graph.n, g0, g1, x.shape[1], _addr(out), _stream()),
+            "hicgat_spmm_csr_rows_f32")
+    return out
+
+
 class SAGEConv(nn.Module):
     """``lin_l(D^-1 A x) + lin_r(trunc(x))`` -- layers.py:57-73, including the reference's
     ``x.long()`` truncation of the root features (layers.py:64; ``trunc_root=False`` disables
@@ -60,7 +76,12 @@ class SAGEConv(nn.Module):
 
     def forward(self, x, edge_index, edge_attr=None, size=None):
         graph = as_graph(edge_index, edge_attr, x.shape[0])
-        out = _SageAggregate.apply(x.float(), graph)
+        if graph.block is not None:  # row block: the block's rows of the aggregation and of the root term
+            g0, g1 = graph.block
+            out = _sage_aggregate_rows(x, graph)
+            x = x[g0:g1]
+        else:
+            out = _SageAggregate.apply(x.float(), graph)
         out = self.lin_l(out)
         if self.root_weight:
             x_r = torch.trunc(x).float() if self.trunc_root else x.float()
@@ -149,6 +170,52 @@ class _GatAttend(torch.autograd.Function):
                                        ws.data_ptr(), ws.numel(), _stream()),
                 "hicgat_gat_bwd",
             )
+        return dxl, datt_l.view(ctx.att_shape), datt_r.view(ctx.att_shape), dbias, None, None, None, None
+
+
+class _GatAttendRows(torch.autograd.Function):
+    """:class:`_GatAttend` on the target rows ``[g0, g1)`` of a row-block view: ``xl`` is the projection of ALL rows, the output
+    the block's rows.  The backward returns PARTIAL gradients (``dxl`` on every row, the att / bias gradients) that, summed over a
+    partition of the rows, are the full-graph gradients."""
+
+    @staticmethod
+    def forward(ctx, xl, att_l, att_r, bias, graph: CSRGraph, heads: int, channels: int, slope: float):
+        _cuda(xl)
+        xl = xl.contiguous()
+        att_l_f, att_r_f, bias_f = att_l.contiguous().view(-1), att_r.contiguous().view(-1), bias.contiguous()
+        r32, c32, _ = graph.with_self_loops()
+        (g0, g1), (e0, e1) = graph.rows, graph.block_entries()
+        n, dev = graph.n, xl.device
+        a_src = torch.empty(n, heads, dtype=torch.float32, device=dev)
+        a_dst = torch.empty(n, heads, dtype=torch.float32, device=dev)
+        alpha = torch.empty(e1 - e0, heads, dtype=torch.float32, device=dev)
+        out = torch.empty(g1 - g0, heads * channels, dtype=torch.float32, device=dev)
+        N.check(
+            N.lib().hicgat_gat_fwd_rows(r32.data_ptr(), c32.data_ptr(), n, g0, g1, e0, heads, channels, xl.data_ptr(), att_l_f.data_ptr(), att_r_f.data_ptr(),
+                                        bias_f.data_ptr(), slope, a_src.data_ptr(), a_dst.data_ptr(), _addr(alpha), _addr(out), _stream()),
+            "hicgat_gat_fwd_rows",
+        )
+        ctx.save_for_backward(xl, att_l_f, att_r_f, bias_f, a_src, a_dst, alpha, out)
+        ctx.graph, ctx.hc, ctx.slope, ctx.att_shape = graph, (heads, channels), slope, att_l.shape
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        xl, att_l_f, att_r_f, bias_f, a_src, a_dst, alpha, out = ctx.saved_tensors
+        graph, (heads, channels) = ctx.graph, ctx.hc
+        g = g.contiguous()
+        r32, c32, perm = graph.with_self_loops()
+        (g0, g1), (e0, _) = graph.rows, graph.block_entries()
+        n, nnz = graph.n, c32.numel()
+        dxl = torch.empty_like(xl)
+        datt_l, datt_r, dbias = torch.empty_like(att_l_f), torch.empty_like(att_r_f), torch.empty(heads * channels, dtype=torch.float32, device=xl.device)
+        ws = _GatWorkspace.get(xl.device, n, nnz, heads, channels)
+        N.check(
+            N.lib().hicgat_gat_bwd_fused_rows(r32.data_ptr(), c32.data_ptr(), perm.data_ptr(), n, nnz, g0, g1, e0, heads, channels, xl.data_ptr(), att_l_f.data_ptr(),
+                                              att_r_f.data_ptr(), bias_f.data_ptr(), ctx.slope, a_src.data_ptr(), a_dst.data_ptr(), _addr(alpha), _addr(out), _addr(g),
+                                              dxl.data_ptr(), datt_l.data_ptr(), datt_r.data_ptr(), dbias.data_ptr(), ws.data_ptr(), ws.numel(), _stream()),
+            "hicgat_gat_bwd_fused_rows",
+        )
         return dxl, datt_l.view(ctx.att_shape), datt_r.view(ctx.att_shape), dbias, None, None, None, None
 
 
@@ -259,6 +326,12 @@ class GATConv(nn.Module):
     def forward(self, x, edge_index, edge_weight=None, size=None):
         graph = as_graph(edge_index, edge_weight, x.shape[0])
         xl = self.lin_l(x)
+        if graph.block is not None:  # row block: CSR kernels with the one-pass backward only
+            if self.path == "dense":
+                raise ValueError("GATConv: the dense-tile path has no row-block form; use path='csr' or 'auto' with a row-block graph")
+            if GAT_BACKWARD != "fused":
+                raise ValueError(f"GATConv: the {GAT_BACKWARD!r} backward has no row-block form; a row-block graph needs the fused backward")
+            return _GatAttendRows.apply(xl, self.att_l, self.att_r, self.bias, graph, self.heads, self.out_channels, self.negative_slope)
         dense_ok = gat_shape_supported(self.heads, self.out_channels) and graph.n <= self.dense_max_n
         use_dense = self.path == "dense" or (self.path == "auto" and dense_ok and graph.n >= 256 and graph.density() >= self.dense_threshold)
         if use_dense and not dense_ok:

@@ -533,8 +533,9 @@ class _LnReluAddFn(torch.autograd.Function):
         y = torch.empty_like(x)
         mean = torch.empty(n, dtype=torch.float32, device=x.device)
         rstd = torch.empty(n, dtype=torch.float32, device=x.device)
-        N.check(N.lib().hicgat_ln_relu_add_fwd(x.data_ptr(), _ptr(res), w.data_ptr(), b.data_ptr(), float(eps), n, c, y.data_ptr(), mean.data_ptr(),
-                                               rstd.data_ptr(), _stream()), "hicgat_ln_relu_add_fwd")
+        if n > 0:  # no rows (an empty row block of a sharded GNN): nothing to launch
+            N.check(N.lib().hicgat_ln_relu_add_fwd(x.data_ptr(), _ptr(res), w.data_ptr(), b.data_ptr(), float(eps), n, c, y.data_ptr(), mean.data_ptr(),
+                                                   rstd.data_ptr(), _stream()), "hicgat_ln_relu_add_fwd")
         ctx.save_for_backward(x, mean, rstd, w, b)
         ctx.has_res = residual is not None
         return y
@@ -547,6 +548,8 @@ class _LnReluAddFn(torch.autograd.Function):
         dx = torch.empty_like(x)
         dgamma = torch.empty_like(w)
         dbeta = torch.empty_like(b)
+        if n == 0:
+            return dx, (gy if ctx.has_res else None), torch.zeros_like(w), torch.zeros_like(b), None
         ws = torch.empty(N.lib().hicgat_ln_relu_add_bwd_workspace_bytes(n, c), dtype=torch.uint8, device=x.device)
         N.check(N.lib().hicgat_ln_relu_add_bwd(gy.data_ptr(), x.data_ptr(), mean.data_ptr(), rstd.data_ptr(), w.data_ptr(), b.data_ptr(), n, c, dx.data_ptr(),
                                                dgamma.data_ptr(), dbeta.data_ptr(), ws.data_ptr(), ws.numel(), _stream()), "hicgat_ln_relu_add_bwd")

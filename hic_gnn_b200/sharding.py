@@ -337,3 +337,197 @@ def cuda_local_split_fn(target, mode: int, c_mse: float, c_l1: float):
         pairloss_raw(coords, target, mode, c_mse, c_l1, moments=moments, grad=grad)
 
     return fn
+
+
+# ------------------------------------------------------------------------------ row-sharded GNN
+def gnn_blocks(rowptr, world: int) -> list[tuple[int, int]]:
+    """Partition of the GNN's target rows into ``world`` contiguous blocks of equal work.  The message-passing kernels cost one
+    warp-row per locus plus one gather per edge, so row i weighs ``deg(i) + 1`` (its row of the self-loop pattern), and the rows
+    ``[0, i)`` weigh ``rowptr[i] + i``.  Cut r is the row whose prefix weight is nearest to ``r / world`` of the total (ties to the
+    lower row); blocks may be empty when one row outweighs a whole share.  Pure arithmetic on the host (one read of ``rowptr``
+    if it is a device tensor); independent of the loss's :func:`row_block` cuts."""
+    import bisect
+
+    if world < 1:
+        raise ValueError(f"gnn_blocks: world must be >= 1, got {world}")
+    rp = [int(v) for v in (rowptr.tolist() if torch.is_tensor(rowptr) else rowptr)]
+    n = len(rp) - 1
+    if n < 0:
+        raise ValueError("gnn_blocks: rowptr needs n + 1 >= 1 entries")
+    mass = [(rp[i] + i) * world for i in range(n + 1)]  # prefix weights, scaled so that cut r aims at r * total
+    total = rp[n] + n
+    cuts = [0]
+    for r in range(1, world):
+        want = r * total
+        i = bisect.bisect_left(mass, want)
+        if i > 0 and want - mass[i - 1] <= mass[min(i, n)] - want:
+            i -= 1
+        cuts.append(max(cuts[-1], min(i, n)))
+    cuts.append(n)
+    return list(zip(cuts[:-1], cuts[1:]))
+
+
+class _GatherCoords(torch.autograd.Function):
+    """Block rows ``[g0, g1)`` of the coordinates -> all N rows (exchange); backward: rows ``[g0, g1)`` of the incoming gradient,
+    which every rank already holds in full (a sharded loss reduces it, an unsharded one computes it on every rank alike)."""
+
+    @staticmethod
+    def forward(ctx, local, shard):
+        ctx.block = (shard.g0, shard.g1)
+        return shard._x.gather(local.detach(), shard.g0, shard.g1)
+
+    @staticmethod
+    def backward(ctx, g):
+        g0, g1 = ctx.block
+        return g[g0:g1], None
+
+
+class _CollectiveExchange:
+    """Both exchanges as ONE ``all_reduce`` each of an f64 buffer (NCCL, or gloo on CPU): the coordinate partial is zero outside
+    the rank's rows, so the gather is exact; the gradient sum is rounded to f32 once.  Eager only: not capturable."""
+
+    capturable = False
+
+    def __init__(self, n: int, numel: int, device, group):
+        self.n, self.numel, self.device, self.group = n, numel, device, group
+
+    def gather(self, local, g0, g1):
+        buf = torch.zeros(self.n, 3, dtype=torch.float64, device=self.device)
+        buf[g0:g1] = local.double()
+        return allreduce_packed(buf, self.group).to(torch.float32)
+
+    def reduce(self, grads):
+        flat = torch.cat([g.reshape(-1).double() for g in grads])
+        allreduce_packed(flat, self.group)
+        torch._foreach_copy_(grads, [v.view_as(g) for v, g in zip(flat.split([g.numel() for g in grads]), grads)])
+
+
+class _P2PExchange:
+    """Both exchanges over NVLink peer memory with the two-shot all-reduce of the sharded loss (``hicgat_allreduce_partials_twoshot``):
+    an f32 buffer is reduced as the ``[k, 3]`` gradient part of a partial whose moment part stays zero (f64 accumulation in rank
+    order, one rounding: bit-identical on every rank; the coordinate gather is exact, the other ranks add zeros).  Each exchange has
+    its own state array and signal-slot range, beyond those of the sharded loss exchanges, so all of them can share a step and a
+    CUDA graph (``capturable``)."""
+
+    capturable = True
+    SLOTS_COORDS = P2PShardedPairLoss.SLOT_BASE + 128  # the loss exchanges use SLOT_BASE + 0 .. + 127
+    SLOTS_GRADS = P2PShardedPairLoss.SLOT_BASE + 160
+
+    def __init__(self, n: int, numel: int, device, group):
+        import ctypes as C
+
+        import torch.distributed._symmetric_memory as symm
+
+        group = group if group is not None else dist.group.WORLD
+        self.n, self.numel = n, numel
+        self.kg = (numel + 2) // 3  # rows of the [k, 3] view of the flat gradient
+        cbytes, gbytes = (12 * n + 15) // 16 * 16, (12 * self.kg + 15) // 16 * 16
+        # layout: [coords partial: 64 + cbytes | coords result: cbytes | grads partial: 64 + gbytes | grads result: gbytes]
+        self.c_part, self.c_res = 0, 64 + cbytes
+        self.g_part = self.c_res + cbytes
+        self.g_res = self.g_part + 64 + gbytes
+        self.buf = symm.empty(self.g_res + gbytes, dtype=torch.uint8, device=device)
+        self.buf.zero_()
+        self.hdl = symm.rendezvous(self.buf, group)
+        self.world, self.rank = self.hdl.world_size, self.hdl.rank
+        if self.hdl.signal_pad_size < 4 * (self.SLOTS_GRADS + 32):
+            raise RuntimeError("symmetric-memory signal pad too small")
+        ptrs = [int(p) for p in self.hdl.buffer_ptrs]
+        table = lambda off: (C.c_uint64 * self.world)(*[p + off for p in ptrs])
+        self._c_bufs, self._c_res = table(self.c_part), table(self.c_res)
+        self._g_bufs, self._g_res = table(self.g_part), table(self.g_res)
+        self._pads = (C.c_uint64 * self.world)(*[int(p) for p in self.hdl.signal_pad_ptrs])
+        f32 = lambda off, k: self.buf[off: off + 4 * k].view(torch.float32)
+        self.part_c = f32(self.c_part + 64, 3 * n).view(n, 3)   # rows outside the block stay zero forever
+        self.res_c = f32(self.c_res, 3 * n).view(n, 3)
+        self.part_g = f32(self.g_part + 64, numel)
+        self.res_g = f32(self.g_res, numel)
+        self.scratch_m = torch.empty(N.PAIR_NMOM, dtype=torch.float64, device=device)  # the (zero) moment sums
+        self.state_c = torch.zeros(4, dtype=torch.int32, device=device)
+        self.state_g = torch.zeros(4, dtype=torch.int32, device=device)
+        torch.cuda.synchronize(device)
+        dist.barrier(group)  # every rank's buffer is zeroed and mapped before the first signal
+
+    def _twoshot(self, bufs, res, k, slots, state):
+        N.check(N.lib().hicgat_allreduce_partials_twoshot(bufs, res, self._pads, self.rank, self.world, k, slots, state.data_ptr(), None,
+                                                          self.scratch_m.data_ptr(), torch.cuda.current_stream().cuda_stream),
+                "hicgat_allreduce_partials_twoshot")
+
+    def gather(self, local, g0, g1):
+        self.part_c[g0:g1].copy_(local)
+        self._twoshot(self._c_bufs, self._c_res, self.n, self.SLOTS_COORDS, self.state_c)
+        return self.res_c.clone()
+
+    def reduce(self, grads):
+        torch.cat([g.reshape(-1) for g in grads], out=self.part_g)
+        self._twoshot(self._g_bufs, self._g_res, self.kg, self.SLOTS_GRADS, self.state_g)
+        torch._foreach_copy_(grads, [v.view_as(g) for v, g in zip(self.res_g.split([g.numel() for g in grads]), grads)])
+
+
+class GnnRowShard:
+    """Row-sharded GNN across the ranks of a process group: this rank runs the message passing and the MLP head on its target
+    rows ``block = (g0, g1)`` only (``graph.row_block(g0, g1)``, blocks from :func:`gnn_blocks`), and two exchanges keep every rank
+    consistent:
+
+    * :meth:`gather_coords` (autograd): the block's ``[g1 - g0, 3]`` coordinates -> all ``[n, 3]``; its backward hands the block's
+      rows of the coordinate gradient back (no communication);
+    * :meth:`reduce_grads`: sums the parameter gradients -- each rank's are partial sums over its rows -- over the ranks, in place,
+      bit-identical on every rank, so that the replicated parameters stay in lock step.
+
+    ``transport``: ``"p2p"`` (two-shot kernel over NVLink peer memory, capturable), ``"nccl"`` (one f64 ``all_reduce`` per
+    exchange; with a gloo group on CPU tensors too; eager only) or ``"auto"`` (p2p on CUDA with an initialised multi-rank group
+    when the symmetric-memory rendezvous succeeds, else nccl -- the rule of :func:`make_sharded_pair_loss`).  Without a multi-rank
+    process group both exchanges are local no-ops around the one block."""
+
+    def __init__(self, n: int, block: tuple[int, int], params, device, group=None, transport: str = "auto"):
+        if transport not in ("auto", "p2p", "nccl"):
+            raise ValueError(f"GnnRowShard: transport must be 'auto', 'p2p' or 'nccl', got {transport!r}")
+        g0, g1 = int(block[0]), int(block[1])
+        if not 0 <= g0 <= g1 <= n:
+            raise ValueError(f"GnnRowShard: need 0 <= g0 <= g1 <= n = {n}, got [{g0}, {g1})")
+        self.n, self.g0, self.g1, self.group = n, g0, g1, group
+        self.params = list(params)
+        numel = sum(p.numel() for p in self.params)
+        multi = dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
+        self._x = None
+        if transport == "p2p" or (transport == "auto" and multi and torch.device(device).type == "cuda"):
+            try:
+                self._x = _P2PExchange(n, numel, device, group)
+            except Exception as e:  # no symmetric memory on this system: the collective exchange is equivalent
+                if transport == "p2p":
+                    raise
+                import warnings
+
+                warnings.warn(f"symmetric-memory exchange unavailable ({e!r}); using the NCCL all-reduce")
+        if self._x is None:
+            self._x = _CollectiveExchange(n, numel, device, group)
+        self.transport = "p2p" if isinstance(self._x, _P2PExchange) else "nccl"
+        # a single rank has nothing to exchange: its (local) collective exchange launches no collective and can be captured
+        self.capturable = self._x.capturable or not multi
+
+    @classmethod
+    def for_rank(cls, graph, params, device, group=None, transport: str = "auto", rank: int | None = None, world: int | None = None):
+        """The shard of this rank (or of ``rank`` of ``world``) with the edge-balanced blocks of :func:`gnn_blocks`."""
+        multi = dist.is_available() and dist.is_initialized()
+        world = world if world is not None else (dist.get_world_size(group) if multi else 1)
+        rank = rank if rank is not None else (dist.get_rank(group) if multi else 0)
+        return cls(graph.n, gnn_blocks(graph.rowptr, world)[rank], params, device, group, transport)
+
+    def graph(self, graph):
+        """This rank's row-block view of ``graph``."""
+        return graph.row_block(self.g0, self.g1)
+
+    def gather_coords(self, local: torch.Tensor) -> torch.Tensor:
+        if local.shape != (self.g1 - self.g0, 3):
+            raise ValueError(f"GnnRowShard.gather_coords: expected [{self.g1 - self.g0}, 3] block coordinates, got {list(local.shape)}")
+        return _GatherCoords.apply(local, self)
+
+    def reduce_grads(self, params=None) -> None:
+        """Sum ``p.grad`` over the ranks for the shard's parameters (a missing gradient counts as zero and is created)."""
+        params = self.params if params is None else list(params)
+        if [p.numel() for p in params] != [p.numel() for p in self.params]:
+            raise ValueError("GnnRowShard.reduce_grads: the parameters differ from those the shard was built for")
+        for p in params:
+            if p.grad is None:
+                p.grad = torch.zeros_like(p)
+        self._x.reduce([p.grad for p in params])

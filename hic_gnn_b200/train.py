@@ -65,10 +65,15 @@ class TrainStep:
     ``track_dscc=True`` also evaluates the dSCC of every step's forward coordinates -- the structure before that step's update, whose
     ``spearmanr`` the reference records every iteration (HiC_GAT_generalize_directly.py:242) -- with a :class:`metrics.DsccMeter`, on
     the device and inside the graph.  The value is ``step.dscc`` (0-d f64, overwritten by the next step).  Needs the full target:
-    refused with a sharded ``reducer``."""
+    refused with a sharded ``reducer``.
+
+    ``gnn_shard`` (:class:`sharding.GnnRowShard`): the GNN runs on this rank's target rows only.  A step is: forward on the
+    row-block view of ``graph`` -> ``gnn_shard.gather_coords`` (all N coordinates) -> the fused loss (sharded with ``reducer`` or
+    not) -> backward -> ``gnn_shard.reduce_grads`` -> Adam; every rank ends the step with identical parameters.  With
+    ``use_cuda_graph`` the exchange must be capturable (the p2p transport)."""
 
     def __init__(self, model, x, graph, target: WishTarget, mode: str = "mse", lr: float = 1e-3, use_cuda_graph: bool = False, reducer=None,
-                 alpha: float = 1.0, track_dscc: bool = False):
+                 alpha: float = 1.0, track_dscc: bool = False, gnn_shard=None):
         if mode not in _KERNEL_MODE:
             raise ValueError(mode)
         if track_dscc and reducer is not None:
@@ -80,6 +85,15 @@ class TrainStep:
             # one-shot p2p kernel) or runs a NCCL collective outside torch's graph support would reuse one epoch forever
             raise ValueError("use_cuda_graph needs a capturable sharded reducer (the default two-shot p2p exchange); "
                              f"{type(reducer).__name__} takes per-step host arguments")
+        if use_cuda_graph and gnn_shard is not None and not gnn_shard.capturable:
+            # the NCCL exchange of the sharded GNN runs collectives outside torch's graph support
+            raise ValueError("use_cuda_graph needs a capturable GNN row shard (the two-shot p2p exchange); "
+                             f"the {gnn_shard.transport!r} exchange of {type(gnn_shard).__name__} is eager only")
+        self.gnn_shard = gnn_shard
+        if gnn_shard is not None:
+            from .graph import as_graph
+
+            graph = gnn_shard.graph(as_graph(graph, None, x.shape[0]))
         self.model, self.x, self.graph, self.target, self.mode, self.reducer, self.alpha = model, x, graph, target, mode, reducer, alpha
         self.optimizer = Adam(model.parameters(), lr=lr, capturable=use_cuda_graph)
         self.total = None
@@ -97,10 +111,14 @@ class TrainStep:
     def _eager(self):
         self.optimizer.zero_grad(set_to_none=True)
         coords = self.model.get_model(self.x, self.graph)
+        if self.gnn_shard is not None:
+            coords = self.gnn_shard.gather_coords(coords)
         if self._meter is not None:
             self.dscc = self._meter(coords.detach().contiguous())
         loss, total, moments = _loss_of_coords(coords, self.target, self.mode, self.reducer, self.alpha)
         loss.backward()
+        if self.gnn_shard is not None:
+            self.gnn_shard.reduce_grads(self.model.parameters())
         self.optimizer.step()
         return total, moments
 
@@ -136,7 +154,7 @@ class TrainStep:
 
 
 def fit(model, x, graph, target: WishTarget, mode: str = "mse", lr: float = 1e-3, thresh: float = 1e-8, max_steps: int | None = None,
-        check_every: int = 1, use_cuda_graph: bool = False, reducer=None, alpha: float = 1.0, dscc_out: list | None = None):
+        check_every: int = 1, use_cuda_graph: bool = False, reducer=None, alpha: float = 1.0, dscc_out: list | None = None, gnn_shard=None):
     """Reference loop.  Returns the list of per-step total losses (floats).
 
     ``check_every=1`` evaluates the stop rule every step exactly like the reference (one host
@@ -144,9 +162,11 @@ def fit(model, x, graph, target: WishTarget, mode: str = "mse", lr: float = 1e-3
     loop may overrun the reference's stopping step by up to ``check_every-1`` iterations.
 
     ``dscc_out``: a list to which the dSCC of every step's (pre-update) structure is appended, like the reference's ``SpRho``
-    history (``TrainStep(track_dscc=True)``); read back in the same batched reads as the losses."""
+    history (``TrainStep(track_dscc=True)``); read back in the same batched reads as the losses.
+
+    ``gnn_shard``: row-sharded GNN (:class:`TrainStep`)."""
     track = dscc_out is not None
-    step = TrainStep(model, x, graph, target, mode, lr, use_cuda_graph, reducer, alpha, track_dscc=track)
+    step = TrainStep(model, x, graph, target, mode, lr, use_cuda_graph, reducer, alpha, track_dscc=track, gnn_shard=gnn_shard)
     hist: list[float] = []
     pending: list[torch.Tensor] = []
     pending_dscc: list[torch.Tensor] = []

@@ -401,6 +401,12 @@ HICGAT_API int hicgat_sage_norm_values(const int32_t* rowptr, const int32_t* col
 HICGAT_API int hicgat_spmm_csr_f32(const int32_t* rowptr, const int32_t* col, const float* w,
                         const float* x, int64_t n, int64_t f, float* out,
                         hicgat_stream_t stream);
+/* Row block [g0, g1) of the same aggregation (0 <= g0 <= g1 <= n): x holds all n rows, out [g1 - g0, f] the block's rows,
+ * bit-identical to rows g0..g1-1 of hicgat_spmm_csr_f32 (which is this call with the block (0, n)).  out may be NULL for an
+ * empty block. */
+HICGAT_API int hicgat_spmm_csr_rows_f32(const int32_t* rowptr, const int32_t* col, const float* w,
+                             const float* x, int64_t n, int64_t g0, int64_t g1, int64_t f, float* out,
+                             hicgat_stream_t stream);
 /* perm[k] = position of the transposed entry (col[k], row(k)) ; w_t = w[perm]. */
 HICGAT_API int hicgat_csr_transpose_perm(const int32_t* rowptr, const int32_t* col, int64_t n,
                               int32_t* perm, hicgat_stream_t stream);
@@ -443,6 +449,26 @@ HICGAT_API int hicgat_gat_bwd_fused(const int32_t* rowptr, const int32_t* col, c
                          const float* a_dst, const float* alpha, const float* out, const float* gout,
                          float* dxl, float* datt_l, float* datt_r, float* dbias, void* workspace,
                          size_t workspace_bytes, hicgat_stream_t stream);
+/* Row block [g0, g1) of the CSR GATConv (0 <= g0 <= g1 <= n), for a GNN whose rows are sharded across GPUs.  The call with the
+ * block (0, n) is hicgat_gat_fwd / hicgat_gat_bwd_fused, bit for bit.  e0 must equal rowptr[g0] (the caller reads it once per block;
+ * the kernels index the block's arrays from it without a host read) and e1 = rowptr[g1] (self-loop pattern).
+ *   fwd_rows : xl [n,H*C] is the projection of ALL rows; a_src / a_dst [n,H] are computed for all rows; alpha [e1-e0,H] holds the
+ *              block's entries (entry k at k - e0) and out [g1-g0,H*C] the block's rows, bit-identical to the full call's.
+ *   bwd_fused_rows : g = dL/dout and out, alpha of the block (as fwd_rows wrote them); outputs are PARTIAL sums over the block's
+ *              target rows: dxl [n,H*C] (every row; zero where no neighbour lies in the block), datt_l / datt_r / dbias [H*C].
+ *              Summed over a partition of [0, n) they equal the full backward up to f32 summation order.  The columns of every row
+ *              must be ascending.  Source row j visits only its neighbours inside the block (two binary searches), so the edge work
+ *              is the block's own.  Same workspace as hicgat_gat_bwd (sized for the whole graph); deterministic, no atomics.
+ * alpha / out / g may be NULL for an empty block.  The two-pass hicgat_gat_bwd and the dense-tile path (1d) have no row-block form. */
+HICGAT_API int hicgat_gat_fwd_rows(const int32_t* rowptr, const int32_t* col, int64_t n, int64_t g0, int64_t g1, int64_t e0, int heads,
+                        int channels, const float* xl, const float* att_l, const float* att_r, const float* bias,
+                        float slope, float* a_src, float* a_dst, float* alpha, float* out, hicgat_stream_t stream);
+HICGAT_API int hicgat_gat_bwd_fused_rows(const int32_t* rowptr, const int32_t* col, const int32_t* perm, int64_t n,
+                              int64_t nnz, int64_t g0, int64_t g1, int64_t e0, int heads, int channels, const float* xl,
+                              const float* att_l, const float* att_r, const float* bias, float slope, const float* a_src,
+                              const float* a_dst, const float* alpha, const float* out, const float* gout,
+                              float* dxl, float* datt_l, float* datt_r, float* dbias, void* workspace,
+                              size_t workspace_bytes, hicgat_stream_t stream);
 
 /* ------------------------------------------------------------------------------------
  * (1d) Dense-tile path of the same GATConv for near-dense graphs (1 Mb / 100 kb maps): per head the
