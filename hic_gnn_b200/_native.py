@@ -41,6 +41,7 @@ SIGNATURES = {
     "hicgat_pairloss_rowside_add": (C.c_int, [_p, _p, _i64, _i64, _i64, _i64, _f32, _p, _p]),
     "hicgat_allreduce_partials_p2p": (C.c_int, [_p, _p, _i32, _i32, _i64, _i64, _i32, _u32, _p, _p, _p, _p]),
     "hicgat_allreduce_partials_twoshot": (C.c_int, [_p, _p, _p, _i32, _i32, _i64, _i32, _p, _p, _p, _p]),
+    "hicgat_allreduce_u64_twoshot": (C.c_int, [_p, _p, _p, _i32, _i32, _i64, _i32, _p, _p]),
     "hicgat_rank_histograms": (C.c_int, [_p, _p, _i64, _i64, _i64, _i64, _f32, _f32, _i32, _p, _p, _p]),
     "hicgat_rank_cross_sum": (C.c_int, [_p, _p, _i64, _i64, _i64, _i64, _f32, _f32, _i32, _p, _p, _p, _p]),
     "hicgat_dist_histogram": (C.c_int, [_p, _i64, _i64, _i64, _f32, _i32, _p, _p]),
@@ -49,6 +50,12 @@ SIGNATURES = {
     "hicgat_dscc_target_ranks": (C.c_int, [_p, _i64, _i64, _f32, _i32, _p, _p, _p, _sz, _p]),
     "hicgat_dscc_dense": (C.c_int, [_p, _p, _i64, _i64, _f32, _i32, _p, _p, _p, _p, _sz, _p]),
     "hicgat_dscc_implicit": (C.c_int, [_p, _p, _p, _p, _i64, _p, _p, _i32, _p, _p, _sz, _p]),
+    "hicgat_dscc_dist_hist_rows": (C.c_int, [_p, _i64, _i64, _i64, _i32, _p, _p, _sz, _p]),
+    "hicgat_dscc_target_hist_rows": (C.c_int, [_p, _i64, _i64, _i64, _i64, _f32, _i32, _p, _p]),
+    "hicgat_dscc_hist_ranks": (C.c_int, [_p, _i64, _i32, _p, _p, _p, _sz, _p]),
+    "hicgat_dscc_cross_dense_rows": (C.c_int, [_p, _p, _i64, _i64, _i64, _i64, _f32, _i32, _p, _p, _p, _p, _sz, _p]),
+    "hicgat_dscc_cross_implicit_rows": (C.c_int, [_p, _p, _p, _p, _i64, _i64, _i64, _i32, _p, _p, _p, _sz, _p]),
+    "hicgat_dscc_finish": (C.c_int, [_p, _i64, _i32, _i32, _p, _p, _p, _p, _sz, _p]),
     "hicgat_pairdist_fwd": (C.c_int, [_p, _i64, _p, _i64, _p]),
     "hicgat_pairdist_bwd": (C.c_int, [_p, _i64, _p, _i64, _p, _p]),
     "hicgat_cont2dist_max_f64": (C.c_int, [_p, _i64, _i64, _i64, _i64, _f64, _p, _p, _sz, _p]),

@@ -115,18 +115,22 @@ __device__ __forceinline__ uint32_t ld_relaxed_gpu_u32(const uint32_t* p) {
     return v;
 }
 
-template <int WORLD>  // 0 = run-time world
-__global__ void __launch_bounds__(256) allreduce_twoshot_kernel(const PeerTable2 T, int rank, int world_rt, int slot_base, uint32_t* __restrict__ state,
-                                                                int64_t total_quads, int64_t slice_quads, const double* __restrict__ moment_const,
-                                                                double* __restrict__ out_moments) {
-    const int world = WORLD ? WORLD : world_rt;
-    __shared__ unsigned s_ticket;
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // the next loss kernel may set itself up behind this one
-    asm volatile("griddepcontrol.wait;" ::: "memory");  // the producer of the local partial has completed and flushed
+__device__ __forceinline__ ulonglong2 ld_relaxed_sys_u64x2(const void* p) {
+    ulonglong2 v;
+    asm volatile("ld.relaxed.sys.global.v2.u64 {%0,%1}, [%2];" : "=l"(v.x), "=l"(v.y) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ void st_relaxed_sys_u64x2(void* p, ulonglong2 v) {
+    asm volatile("st.relaxed.sys.global.v2.u64 [%0], {%1,%2};" ::"l"(p), "l"(v.x), "l"(v.y) : "memory");
+}
+
+// The two barriers of a two-shot kernel (every block of the grid calls both, in order).  Entry: wait for the producer grid (programmatic
+// stream serialization), take this launch's epoch from `state`, and barrier A -- every rank's source is complete.
+__device__ __forceinline__ uint32_t twoshot_enter(const PeerTable2& T, int rank, int world, int slot_base, const uint32_t* state) {
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // the next kernel may set itself up behind this one
+    asm volatile("griddepcontrol.wait;" ::: "memory");  // the producer of the local source has completed and flushed
     const uint32_t epoch = ld_relaxed_gpu_u32(state) + 1u;
-    uint32_t* const sig_a = T.pad[rank] + slot_base;             // "partial of epoch e is complete", one slot per source rank
-    uint32_t* const sig_b = T.pad[rank] + slot_base + kMaxWorld; // "my reduced slice of epoch e has landed everywhere"
-    // ---- barrier A
+    uint32_t* const sig_a = T.pad[rank] + slot_base;             // "source of epoch e is complete", one slot per source rank
     if (blockIdx.x == 0 && threadIdx.x < world) {
         __threadfence_system();
         st_release_sys(T.pad[threadIdx.x] + slot_base + rank, epoch);
@@ -135,6 +139,43 @@ __global__ void __launch_bounds__(256) allreduce_twoshot_kernel(const PeerTable2
         while ((int32_t)(ld_acquire_sys(sig_a + threadIdx.x) - epoch) < 0) { __nanosleep(20); }
     }
     __syncthreads();
+    return epoch;
+}
+
+// Barrier B -- the last block of this rank to finish its stores signals every peer, all wait for every peer's signal -- then the last
+// block to leave publishes the epoch and clears the tickets (every block has read state[0] by now).
+__device__ __forceinline__ void twoshot_leave(const PeerTable2& T, int rank, int world, int slot_base, uint32_t* state, uint32_t epoch) {
+    __shared__ unsigned s_ticket;
+    uint32_t* const sig_b = T.pad[rank] + slot_base + kMaxWorld; // "my reduced slice of epoch e has landed everywhere"
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        __threadfence_system();
+        s_ticket = atomicAdd(state + 1, 1u);
+        __threadfence_system();
+    }
+    __syncthreads();
+    if (s_ticket == gridDim.x - 1 && threadIdx.x < world) st_release_sys(T.pad[threadIdx.x] + slot_base + kMaxWorld + rank, epoch);
+    if (threadIdx.x < world) {
+        while ((int32_t)(ld_acquire_sys(sig_b + threadIdx.x) - epoch) < 0) { __nanosleep(20); }
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const unsigned t2 = atomicAdd(state + 2, 1u);
+        if (t2 == gridDim.x - 1) {
+            state[1] = 0u;
+            state[2] = 0u;
+            __threadfence();
+            state[0] = epoch;
+        }
+    }
+}
+
+template <int WORLD>  // 0 = run-time world
+__global__ void __launch_bounds__(256) allreduce_twoshot_kernel(const PeerTable2 T, int rank, int world_rt, int slot_base, uint32_t* __restrict__ state,
+                                                                int64_t total_quads, int64_t slice_quads, const double* __restrict__ moment_const,
+                                                                double* __restrict__ out_moments) {
+    const int world = WORLD ? WORLD : world_rt;
+    const uint32_t epoch = twoshot_enter(T, rank, world, slot_base, state);
     // ---- moments: 8 doubles per rank, every rank sums all of them in rank order
     if (blockIdx.x == 0 && threadIdx.x < HICGAT_PAIR_NMOM) {
         double s = 0.0;
@@ -162,29 +203,42 @@ __global__ void __launch_bounds__(256) allreduce_twoshot_kernel(const PeerTable2
             if (r < world) st_relaxed_sys_f32x4(T.res[r] + off, o);
         }
     }
-    // ---- barrier B: the last block of this rank to finish its stores signals every peer
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        __threadfence_system();
-        s_ticket = atomicAdd(state + 1, 1u);
-        __threadfence_system();
-    }
-    __syncthreads();
-    if (s_ticket == gridDim.x - 1 && threadIdx.x < world) st_release_sys(T.pad[threadIdx.x] + slot_base + kMaxWorld + rank, epoch);
-    if (threadIdx.x < world) {
-        while ((int32_t)(ld_acquire_sys(sig_b + threadIdx.x) - epoch) < 0) { __nanosleep(20); }
-    }
-    __syncthreads();
-    // ---- the last block to leave publishes the epoch and clears the tickets (every block has read state[0] by now)
-    if (threadIdx.x == 0) {
-        const unsigned t2 = atomicAdd(state + 2, 1u);
-        if (t2 == gridDim.x - 1) {
-            state[1] = 0u;
-            state[2] = 0u;
-            __threadfence();
-            state[0] = epoch;
+    twoshot_leave(T, rank, world, slot_base, state, epoch);
+}
+
+// u64 sums: slice `rank` of the 16-byte pairs (and, on the last rank's slice owner, an odd trailing element), every load of an element in
+// flight together, stored into every rank's result.  Integer adds: the result does not depend on the order.
+__global__ void __launch_bounds__(256) allreduce_u64_twoshot_kernel(const PeerTable2 T, int rank, int world, int slot_base, uint32_t* __restrict__ state,
+                                                                    int64_t count, int64_t slice_pairs) {
+    const uint32_t epoch = twoshot_enter(T, rank, world, slot_base, state);
+    const int64_t pairs = count >> 1;
+    const int64_t base = (int64_t)rank * slice_pairs;
+    int64_t cnt = pairs - base;
+    cnt = cnt < 0 ? 0 : (cnt > slice_pairs ? slice_pairs : cnt);
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < cnt; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t off = 16 * (base + i);
+        ulonglong2 v[kMaxWorld];
+#pragma unroll
+        for (int r = 0; r < kMaxWorld; ++r) v[r] = r < world ? ld_relaxed_sys_u64x2(T.part[r] + off) : make_ulonglong2(0ull, 0ull);
+        ulonglong2 o = make_ulonglong2(0ull, 0ull);
+#pragma unroll
+        for (int r = 0; r < kMaxWorld; ++r) { o.x += v[r].x; o.y += v[r].y; }
+#pragma unroll
+        for (int r = 0; r < kMaxWorld; ++r) {
+            if (r < world) st_relaxed_sys_u64x2(T.res[r] + off, o);
         }
     }
+    if ((count & 1) && rank == world - 1 && blockIdx.x == 0 && threadIdx.x == 0) {
+        const int64_t off = 8 * (count - 1);
+        unsigned long long o = 0ull;
+        for (int r = 0; r < world; ++r) {
+            unsigned long long v;
+            asm volatile("ld.relaxed.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(T.part[r] + off) : "memory");
+            o += v;
+        }
+        for (int r = 0; r < world; ++r) asm volatile("st.relaxed.sys.global.u64 [%0], %1;" ::"l"(T.res[r] + off), "l"(o) : "memory");
+    }
+    twoshot_leave(T, rank, world, slot_base, state, epoch);
 }
 
 }  // namespace
@@ -255,6 +309,42 @@ extern "C" int hicgat_allreduce_partials_twoshot(const uint64_t* peer_partials_h
     }
     if (e != cudaSuccess) {
         set_error("allreduce_twoshot_kernel: launch failed: %s", cudaGetErrorString(e));
+        return HICGAT_ERR_CUDA;
+    }
+    count_launch();
+    return HICGAT_OK;
+}
+
+extern "C" int hicgat_allreduce_u64_twoshot(const uint64_t* peer_src_host, const uint64_t* peer_dst_host, const uint64_t* signal_pads_host, int rank,
+                                            int world, int64_t count, int slot_base, uint32_t* state, hicgat_stream_t stream_) {
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    HICGAT_REQUIRE(peer_src_host && peer_dst_host && signal_pads_host && state, "hicgat_allreduce_u64_twoshot: null pointer");
+    HICGAT_REQUIRE(world >= 1 && world <= kMaxWorld && rank >= 0 && rank < world, "hicgat_allreduce_u64_twoshot: bad rank/world (%d/%d)", rank, world);
+    HICGAT_REQUIRE(count > 0 && slot_base >= 0, "hicgat_allreduce_u64_twoshot: bad count/slot_base");
+    PeerTable2 T;
+    for (int r = 0; r < world; ++r) {
+        HICGAT_REQUIRE(peer_src_host[r] && peer_dst_host[r] && signal_pads_host[r], "hicgat_allreduce_u64_twoshot: null peer pointer for rank %d", r);
+        HICGAT_REQUIRE((peer_src_host[r] % 16) == 0 && (peer_dst_host[r] % 16) == 0, "hicgat_allreduce_u64_twoshot: peer buffer %d not 16-byte aligned", r);
+        T.part[r] = reinterpret_cast<const unsigned char*>(peer_src_host[r]);
+        T.res[r] = reinterpret_cast<unsigned char*>(peer_dst_host[r]);
+        T.pad[r] = reinterpret_cast<uint32_t*>(signal_pads_host[r]);
+    }
+    const int64_t slice_pairs = (count / 2 + world - 1) / world;
+    int grid = (int)((slice_pairs + 255) / 256);
+    if (grid > 64) grid = 64;  // all blocks are co-resident (every block takes part in the barriers)
+    if (grid < 1) grid = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(256);
+    cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, allreduce_u64_twoshot_kernel, T, rank, world, slot_base, state, count, slice_pairs);
+    if (e != cudaSuccess) {
+        set_error("allreduce_u64_twoshot_kernel: launch failed: %s", cudaGetErrorString(e));
         return HICGAT_ERR_CUDA;
     }
     count_launch();

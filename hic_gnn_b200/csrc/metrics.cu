@@ -196,15 +196,16 @@ __global__ void __launch_bounds__(kFinishThreads) dscc_scale_kernel(const float*
     }
 }
 
-// Histogram of every pair i < j of an n x n map: of the reconstructed distance (TARGET = false, scale read from the device) or of
-// the dense target (TARGET = true).  Same tiles as rank_pass_kernel; a warp whose pairs all share a bin (the t == 1.0 group of a wish
-// matrix, a collapsed structure) adds once instead of serialising 32 atomics on one address.
+// Histogram of the pairs i < j with i in rows [r0, r1) of an n x n map: of the reconstructed distance (TARGET = false, scale read from
+// the device) or of the dense target (TARGET = true; row i at target + (i - r0) pitch).  Same tiles as rank_pass_kernel; a warp whose
+// pairs all share a bin (the t == 1.0 group of a wish matrix, a collapsed structure) adds once instead of serialising 32 atomics on one
+// address.
 template <bool TARGET>
 __global__ void __launch_bounds__(kThreadsM) dscc_hist_kernel(const float* __restrict__ coords, const float* __restrict__ target, int64_t pitch, int n,
-                                                              const float* __restrict__ d_scale_p, float t_scale, int nbins,
+                                                              int r0, int r1, const float* __restrict__ d_scale_p, float t_scale, int nbins,
                                                               unsigned long long* __restrict__ hist) {
     __shared__ float s_x[kRows][3];
-    const int i0 = blockIdx.y * kRows;
+    const int i0 = r0 + blockIdx.y * kRows;
     const int j = blockIdx.x * kThreadsM + threadIdx.x;
     if (tile_below_diagonal(i0)) return;
     if (!TARGET) load_tile_rows(s_x, coords, i0, n);
@@ -215,12 +216,12 @@ __global__ void __launch_bounds__(kThreadsM) dscc_hist_kernel(const float* __res
         d_scale = *d_scale_p;
         if (col_ok) xj = coords[(size_t)j * 3], yj = coords[(size_t)j * 3 + 1], zj = coords[(size_t)j * 3 + 2];
     }
-    const int rows = min(kRows, n - i0);
+    const int rows = min(kRows, r1 - i0);
     for (int u = 0; u < rows; ++u) {  // warp-uniform trip count: every lane takes part in the match
         const int i = i0 + u;
         int b = -1;
         if (col_ok && i < j) {
-            b = TARGET ? bin_of(__ldg(target + (size_t)i * pitch + j), t_scale, nbins)
+            b = TARGET ? bin_of(__ldg(target + (size_t)(i - r0) * pitch + j), t_scale, nbins)
                        : bin_of(pair_dist(xj, yj, zj, s_x[u][0], s_x[u][1], s_x[u][2]), d_scale, nbins);
         }
         hist_add_warp(hist, b);
@@ -299,14 +300,15 @@ __global__ void __launch_bounds__(kScanThreads) dscc_midrank_kernel(const unsign
     }
 }
 
-// Dense target: partial[tile] = sum over the tile's pairs i < j of rank_d[bin(d_ij)] * rank_t[bin(t_ij)]; every tile writes its slot.
+// Dense target, rows [r0, r1) (row i at target + (i - r0) pitch): partial[tile] = sum over the tile's pairs i < j of
+// rank_d[bin(d_ij)] * rank_t[bin(t_ij)]; every tile of the block writes its slot.
 __global__ void __launch_bounds__(kThreadsM) dscc_cross_dense_kernel(const float* __restrict__ coords, const float* __restrict__ target, int64_t pitch, int n,
-                                                                     const float* __restrict__ d_scale_p, float t_scale, int nbins,
+                                                                     int r0, int r1, const float* __restrict__ d_scale_p, float t_scale, int nbins,
                                                                      const double* __restrict__ rank_d, const double* __restrict__ rank_t,
                                                                      double* __restrict__ partials) {
     __shared__ float s_x[kRows][3];
     __shared__ double s_red[kThreadsM / 32];
-    const int i0 = blockIdx.y * kRows;
+    const int i0 = r0 + blockIdx.y * kRows;
     const int j = blockIdx.x * kThreadsM + threadIdx.x;
     const size_t slot = (size_t)blockIdx.y * gridDim.x + blockIdx.x;
     if (tile_below_diagonal(i0)) {
@@ -319,12 +321,12 @@ __global__ void __launch_bounds__(kThreadsM) dscc_cross_dense_kernel(const float
     if (j < n) {
         const float d_scale = *d_scale_p;
         const float xj = coords[(size_t)j * 3], yj = coords[(size_t)j * 3 + 1], zj = coords[(size_t)j * 3 + 2];
-        const int rows = min(kRows, n - i0);
+        const int rows = min(kRows, r1 - i0);
         for (int u = 0; u < rows; ++u) {
             const int i = i0 + u;
             if (i >= j) break;
             const float d = pair_dist(xj, yj, zj, s_x[u][0], s_x[u][1], s_x[u][2]);
-            const float t = __ldg(target + (size_t)i * pitch + j);
+            const float t = __ldg(target + (size_t)(i - r0) * pitch + j);
             acc += rank_d[bin_of(d, d_scale, nbins)] * rank_t[bin_of(t, t_scale, nbins)];
         }
     }
@@ -332,16 +334,17 @@ __global__ void __launch_bounds__(kThreadsM) dscc_cross_dense_kernel(const float
     if (threadIdx.x == 0) partials[slot] = s;
 }
 
-// Implicit target: over the stored CSR entries k = (i, j), j > i (one warp per row), partial[0][blk] = sum rank_t_csr[k] rank_d[bin(d_ij)]
-// and partial[1][blk] = sum rank_d[bin(d_ij)]; the fill group's share follows from them (dscc_finish_kernel).
+// Implicit target: over the stored CSR entries k = (i, j), j > i, of rows [r0, r1) (one warp per row), partial[0][blk] =
+// sum rank_t_csr[k] rank_d[bin(d_ij)] and partial[1][blk] = sum rank_d[bin(d_ij)]; the fill group's share follows from them
+// (dscc_finish_kernel).
 __global__ void __launch_bounds__(kCsrRowsPerBlock * 32) dscc_cross_csr_kernel(const float* __restrict__ coords, const int32_t* __restrict__ rowptr,
                                                                                const int32_t* __restrict__ col, const double* __restrict__ rank_t_csr,
-                                                                               int n, const float* __restrict__ d_scale_p, int nbins,
+                                                                               int r0, int r1, const float* __restrict__ d_scale_p, int nbins,
                                                                                const double* __restrict__ rank_d, double* __restrict__ partials) {
     __shared__ double s_red[kCsrRowsPerBlock];
-    const int i = blockIdx.x * kCsrRowsPerBlock + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    const int i = r0 + blockIdx.x * kCsrRowsPerBlock + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     double sx = 0.0, sd = 0.0;
-    if (i < n) {
+    if (i < r1) {
         const float d_scale = *d_scale_p;
         const float xi = coords[(size_t)i * 3], yi = coords[(size_t)i * 3 + 1], zi = coords[(size_t)i * 3 + 2];
         for (int k = rowptr[i] + lane; k < rowptr[i + 1]; k += 32) {
@@ -366,26 +369,28 @@ __device__ double block_sum_strided(const double* __restrict__ v, int64_t count,
     return block_sum_fixed<kFinishThreads>(a, s_red);
 }
 
-// out = sum of v[0..count) in a fixed order.  One block.
-__global__ void __launch_bounds__(kFinishThreads) dscc_sum_kernel(const double* __restrict__ v, int64_t count, double* __restrict__ out) {
+// out[q] = sum of v[q count .. (q + 1) count) in a fixed order for q < nsums, out[q] = 0 for nsums <= q < nout.  One block.
+__global__ void __launch_bounds__(kFinishThreads) dscc_sum_kernel(const double* __restrict__ v, int64_t count, int nsums, int nout, double* __restrict__ out) {
     __shared__ double s_red[kFinishThreads / 32];
-    const double s = block_sum_strided(v, count, s_red);
-    if (threadIdx.x == 0) *out = s;
+    for (int q = 0; q < nout; ++q) {
+        const double s = q < nsums ? block_sum_strided(v + q * count, count, s_red) : 0.0;
+        if (threadIdx.x == 0) out[q] = s;
+    }
 }
 
-// rho = (cross - P mean^2) / sqrt(var_d var_t), NaN unless var_d var_t is finite and > 0.  Implicit target (csr_partials != 0):
-// cross = sum_stored rank_t rank_d + rank_fill (sum_all h rank_d - sum_stored rank_d).  One block.
+// rho = (cross - P mean^2) / sqrt(var_d var_t), NaN unless var_d var_t is finite and > 0; cross_sum = the rank-summed f64[2] of the block
+// cross sums.  Implicit target: cross = cross_sum[0] + rank_fill (sum_all h rank_d - cross_sum[1]), cross_sum[1] = sum_stored rank_d.
+// One block.
 __global__ void __launch_bounds__(kFinishThreads) dscc_finish_kernel(const double* __restrict__ scan_partials, int nscan,
-                                                                     const double* __restrict__ cross_partials, int64_t ncross, int implicit,
+                                                                     const double* __restrict__ cross_sum, int implicit,
                                                                      const double* __restrict__ var_t, const double* __restrict__ rank_fill,
                                                                      double npairs, double* __restrict__ rho) {
     __shared__ double s_red[kFinishThreads / 32];
     const double var_d = block_sum_strided(scan_partials, nscan, s_red);
-    double cross = block_sum_strided(cross_partials, ncross, s_red);
+    double cross = cross_sum[0];
     if (implicit) {
         const double sum_hr = block_sum_strided(scan_partials + nscan, nscan, s_red);
-        const double sum_rd = block_sum_strided(cross_partials + ncross, ncross, s_red);
-        if (threadIdx.x == 0) cross += *rank_fill * (sum_hr - sum_rd);
+        if (threadIdx.x == 0) cross += *rank_fill * (sum_hr - cross_sum[1]);
     }
     if (threadIdx.x == 0) {
         const double mean = (npairs + 1.0) / 2.0;
@@ -458,6 +463,7 @@ struct DsccWorkspace {
     unsigned long long* block_sums;
     double* scan_partials;   // [2][nscan]
     double* cross_partials;  // [2][ncross]
+    double* cross_sum;       // [2]: the block cross sum of the (0, n) entry points
     int nscan;
     int64_t ncross;
     size_t bytes;
@@ -481,70 +487,151 @@ DsccWorkspace dscc_layout(int64_t n, int nbins, void* base) {
     w.block_sums = reinterpret_cast<unsigned long long*>(take((size_t)w.nscan * 8));
     w.scan_partials = reinterpret_cast<double*>(take((size_t)w.nscan * 16));
     w.cross_partials = reinterpret_cast<double*>(take((size_t)w.ncross * 16));
+    w.cross_sum = reinterpret_cast<double*>(take(16));
     w.bytes = off;
     return w;
 }
 
 bool dscc_sizes_ok(int64_t n, int nbins) { return n > 0 && n <= kDsccMaxN && nbins > 0; }
+bool dscc_rows_ok(int64_t n, int64_t r0, int64_t r1, int nbins) { return dscc_sizes_ok(n, nbins) && r0 >= 0 && r0 <= r1 && r1 <= n; }
 
-// histogram of the pairs (distances from the device scale, or the dense target) -> mid-rank table + per-scan-block partials
-int dscc_ranks(bool of_target, const float* coords, const float* target, int64_t pitch, int64_t n, float t_scale, int nbins, double* rank,
-               const DsccWorkspace& w, cudaStream_t stream) {
-    HICGAT_CUDA(cudaMemsetAsync(w.hist, 0, (size_t)nbins * 8, stream));
-    const dim3 grid((unsigned)((n + kThreadsM - 1) / kThreadsM), (unsigned)((n + kRows - 1) / kRows));
-    if (of_target) dscc_hist_kernel<true><<<grid, kThreadsM, 0, stream>>>(nullptr, target, pitch, (int)n, nullptr, t_scale, nbins, w.hist);
-    else dscc_hist_kernel<false><<<grid, kThreadsM, 0, stream>>>(coords, nullptr, 0, (int)n, w.d_scale, 0.f, nbins, w.hist);
+// zero hist, then add the pairs i < j of rows [r0, r1): distances (of_target = false, scale from the workspace) or the dense block
+int dscc_block_hist(bool of_target, const float* coords, const float* target, int64_t pitch, int64_t n, int64_t r0, int64_t r1, const float* d_scale,
+                    float t_scale, int nbins, unsigned long long* hist, cudaStream_t stream) {
+    HICGAT_CUDA(cudaMemsetAsync(hist, 0, (size_t)nbins * 8, stream));
+    if (r1 == r0) return HICGAT_OK;
+    const dim3 grid((unsigned)((n + kThreadsM - 1) / kThreadsM), (unsigned)((r1 - r0 + kRows - 1) / kRows));
+    if (of_target) dscc_hist_kernel<true><<<grid, kThreadsM, 0, stream>>>(nullptr, target, pitch, (int)n, (int)r0, (int)r1, nullptr, t_scale, nbins, hist);
+    else dscc_hist_kernel<false><<<grid, kThreadsM, 0, stream>>>(coords, nullptr, 0, (int)n, (int)r0, (int)r1, d_scale, 0.f, nbins, hist);
     HICGAT_CHECK_LAUNCH("dscc_hist_kernel");
-    dscc_bin_block_sums_kernel<<<w.nscan, kScanThreads, 0, stream>>>(w.hist, nbins, w.block_sums);
+    return HICGAT_OK;
+}
+
+// mid-rank table of a (summed) histogram of all P = n (n - 1) / 2 pairs + per-scan-block partials of var and sum h rank (w.scan_partials)
+int dscc_hist_midranks(const unsigned long long* hist, int64_t n, int nbins, double* rank, const DsccWorkspace& w, cudaStream_t stream) {
+    dscc_bin_block_sums_kernel<<<w.nscan, kScanThreads, 0, stream>>>(hist, nbins, w.block_sums);
     HICGAT_CHECK_LAUNCH("dscc_bin_block_sums_kernel");
     const double npairs = (double)n * (double)(n - 1) / 2.0;
-    dscc_midrank_kernel<<<w.nscan, kScanThreads, 0, stream>>>(w.hist, nbins, w.block_sums, (npairs + 1.0) / 2.0, rank, w.scan_partials);
+    dscc_midrank_kernel<<<w.nscan, kScanThreads, 0, stream>>>(hist, nbins, w.block_sums, (npairs + 1.0) / 2.0, rank, w.scan_partials);
     HICGAT_CHECK_LAUNCH("dscc_midrank_kernel");
     return HICGAT_OK;
 }
 
-int dscc_distance_side(const float* coords, int64_t n, int nbins, const DsccWorkspace& w, cudaStream_t stream) {
-    dscc_scale_kernel<<<1, kFinishThreads, 0, stream>>>(coords, (int)n, nbins, w.d_scale);
-    HICGAT_CHECK_LAUNCH("dscc_scale_kernel");
-    return dscc_ranks(false, coords, nullptr, 0, n, 0.f, nbins, w.rank_d, w, stream);
+// the block's per-tile (per-CSR-block) partials [2][count] -> cross f64[2] (cross[1] = 0 for a dense target)
+int dscc_cross_total(int64_t count, bool implicit, double* cross, const DsccWorkspace& w, cudaStream_t stream) {
+    dscc_sum_kernel<<<1, kFinishThreads, 0, stream>>>(w.cross_partials, count, implicit ? 2 : 1, 2, cross);
+    HICGAT_CHECK_LAUNCH("dscc_sum_kernel");
+    return HICGAT_OK;
 }
 }  // namespace
+
+#define DSCC_WORKSPACE(name)                                                                                                   \
+    const DsccWorkspace w = dscc_layout(n, nbins, workspace);                                                                  \
+    HICGAT_REQUIRE(workspace_bytes >= w.bytes, name ": workspace of %zu bytes, %zu needed", workspace_bytes, w.bytes);         \
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_)
 
 extern "C" size_t hicgat_dscc_workspace_bytes(int64_t n, int nbins) {
     if (!dscc_sizes_ok(n, nbins)) return 0;
     return dscc_layout(n, nbins, nullptr).bytes;
 }
 
+// ---- the phases of one evaluation over target rows [r0, r1)
+extern "C" int hicgat_dscc_dist_hist_rows(const float* coords, int64_t n, int64_t r0, int64_t r1, int nbins, uint64_t* hist_d, void* workspace,
+                                          size_t workspace_bytes, hicgat_stream_t stream_) {
+    HICGAT_REQUIRE(dscc_rows_ok(n, r0, r1, nbins), "hicgat_dscc_dist_hist_rows: bad n/r0/r1/nbins (need 0 <= r0 <= r1 <= n <= %lld, nbins > 0)", (long long)kDsccMaxN);
+    HICGAT_REQUIRE(coords && hist_d && workspace, "hicgat_dscc_dist_hist_rows: null pointer");
+    DSCC_WORKSPACE("hicgat_dscc_dist_hist_rows");
+    dscc_scale_kernel<<<1, kFinishThreads, 0, stream>>>(coords, (int)n, nbins, w.d_scale);  // from all n loci: the same bins on every rank
+    HICGAT_CHECK_LAUNCH("dscc_scale_kernel");
+    return dscc_block_hist(false, coords, nullptr, 0, n, r0, r1, w.d_scale, 0.f, nbins, reinterpret_cast<unsigned long long*>(hist_d), stream);
+}
+
+extern "C" int hicgat_dscc_target_hist_rows(const float* target, int64_t pitch, int64_t n, int64_t r0, int64_t r1, float t_scale, int nbins,
+                                            uint64_t* hist_t, hicgat_stream_t stream_) {
+    HICGAT_REQUIRE(dscc_rows_ok(n, r0, r1, nbins), "hicgat_dscc_target_hist_rows: bad n/r0/r1/nbins (need 0 <= r0 <= r1 <= n <= %lld, nbins > 0)", (long long)kDsccMaxN);
+    HICGAT_REQUIRE(target && hist_t && pitch >= n, "hicgat_dscc_target_hist_rows: null pointer / bad pitch");
+    return dscc_block_hist(true, nullptr, target, pitch, n, r0, r1, nullptr, t_scale, nbins, reinterpret_cast<unsigned long long*>(hist_t),
+                           static_cast<cudaStream_t>(stream_));
+}
+
+extern "C" int hicgat_dscc_hist_ranks(const uint64_t* hist, int64_t n, int nbins, double* rank, double* var, void* workspace, size_t workspace_bytes,
+                                      hicgat_stream_t stream_) {
+    HICGAT_REQUIRE(dscc_sizes_ok(n, nbins), "hicgat_dscc_hist_ranks: bad n/nbins (need 0 < n <= %lld, nbins > 0)", (long long)kDsccMaxN);
+    HICGAT_REQUIRE(hist && rank && var && workspace, "hicgat_dscc_hist_ranks: null pointer");
+    DSCC_WORKSPACE("hicgat_dscc_hist_ranks");
+    const int rc = dscc_hist_midranks(reinterpret_cast<const unsigned long long*>(hist), n, nbins, rank, w, stream);
+    if (rc != HICGAT_OK) return rc;
+    dscc_sum_kernel<<<1, kFinishThreads, 0, stream>>>(w.scan_partials, w.nscan, 1, 1, var);
+    HICGAT_CHECK_LAUNCH("dscc_sum_kernel");
+    return HICGAT_OK;
+}
+
+extern "C" int hicgat_dscc_cross_dense_rows(const float* coords, const float* target, int64_t pitch, int64_t n, int64_t r0, int64_t r1, float t_scale,
+                                            int nbins, const uint64_t* hist_d, const double* rank_t, double* cross, void* workspace,
+                                            size_t workspace_bytes, hicgat_stream_t stream_) {
+    HICGAT_REQUIRE(dscc_rows_ok(n, r0, r1, nbins), "hicgat_dscc_cross_dense_rows: bad n/r0/r1/nbins (need 0 <= r0 <= r1 <= n <= %lld, nbins > 0)", (long long)kDsccMaxN);
+    HICGAT_REQUIRE(coords && target && hist_d && rank_t && cross && workspace && pitch >= n, "hicgat_dscc_cross_dense_rows: null pointer / bad pitch");
+    DSCC_WORKSPACE("hicgat_dscc_cross_dense_rows");
+    int rc = dscc_hist_midranks(reinterpret_cast<const unsigned long long*>(hist_d), n, nbins, w.rank_d, w, stream);
+    if (rc != HICGAT_OK) return rc;
+    const dim3 grid((unsigned)((n + kThreadsM - 1) / kThreadsM), (unsigned)((r1 - r0 + kRows - 1) / kRows));
+    if (r1 > r0) {
+        dscc_cross_dense_kernel<<<grid, kThreadsM, 0, stream>>>(coords, target, pitch, (int)n, (int)r0, (int)r1, w.d_scale, t_scale, nbins, w.rank_d, rank_t,
+                                                                w.cross_partials);
+        HICGAT_CHECK_LAUNCH("dscc_cross_dense_kernel");
+    }
+    return dscc_cross_total((int64_t)grid.x * grid.y, false, cross, w, stream);
+}
+
+extern "C" int hicgat_dscc_cross_implicit_rows(const float* coords, const int32_t* rowptr, const int32_t* col, const double* rank_t_csr, int64_t n,
+                                               int64_t r0, int64_t r1, int nbins, const uint64_t* hist_d, double* cross, void* workspace,
+                                               size_t workspace_bytes, hicgat_stream_t stream_) {
+    HICGAT_REQUIRE(dscc_rows_ok(n, r0, r1, nbins), "hicgat_dscc_cross_implicit_rows: bad n/r0/r1/nbins (need 0 <= r0 <= r1 <= n <= %lld, nbins > 0)", (long long)kDsccMaxN);
+    HICGAT_REQUIRE(coords && rowptr && col && rank_t_csr && hist_d && cross && workspace, "hicgat_dscc_cross_implicit_rows: null pointer");
+    DSCC_WORKSPACE("hicgat_dscc_cross_implicit_rows");
+    int rc = dscc_hist_midranks(reinterpret_cast<const unsigned long long*>(hist_d), n, nbins, w.rank_d, w, stream);
+    if (rc != HICGAT_OK) return rc;
+    const int blocks = (int)((r1 - r0 + kCsrRowsPerBlock - 1) / kCsrRowsPerBlock);
+    if (blocks > 0) {
+        dscc_cross_csr_kernel<<<blocks, kCsrRowsPerBlock * 32, 0, stream>>>(coords, rowptr, col, rank_t_csr, (int)r0, (int)r1, w.d_scale, nbins, w.rank_d,
+                                                                            w.cross_partials);
+        HICGAT_CHECK_LAUNCH("dscc_cross_csr_kernel");
+    }
+    return dscc_cross_total(blocks, true, cross, w, stream);
+}
+
+extern "C" int hicgat_dscc_finish(const double* cross_sum, int64_t n, int nbins, int implicit, const double* rank_fill, const double* var_t, double* rho,
+                                  void* workspace, size_t workspace_bytes, hicgat_stream_t stream_) {
+    HICGAT_REQUIRE(dscc_sizes_ok(n, nbins), "hicgat_dscc_finish: bad n/nbins (need 0 < n <= %lld, nbins > 0)", (long long)kDsccMaxN);
+    HICGAT_REQUIRE(cross_sum && var_t && rho && workspace && (rank_fill || !implicit), "hicgat_dscc_finish: null pointer");
+    DSCC_WORKSPACE("hicgat_dscc_finish");
+    dscc_finish_kernel<<<1, kFinishThreads, 0, stream>>>(w.scan_partials, w.nscan, cross_sum, implicit ? 1 : 0, var_t, rank_fill,
+                                                         (double)n * (double)(n - 1) / 2.0, rho);
+    HICGAT_CHECK_LAUNCH("dscc_finish_kernel");
+    return HICGAT_OK;
+}
+
+// ---- the full target: the phases over rows (0, n) with the workspace's own histogram and cross sum
 extern "C" int hicgat_dscc_target_ranks(const float* target, int64_t pitch, int64_t n, float t_scale, int nbins, double* rank_t, double* var_t,
                                         void* workspace, size_t workspace_bytes, hicgat_stream_t stream_) {
     HICGAT_REQUIRE(dscc_sizes_ok(n, nbins), "hicgat_dscc_target_ranks: bad n/nbins (need 0 < n <= %lld, nbins > 0)", (long long)kDsccMaxN);
     HICGAT_REQUIRE(target && rank_t && var_t && workspace && pitch >= n, "hicgat_dscc_target_ranks: null pointer / bad pitch");
-    const DsccWorkspace w = dscc_layout(n, nbins, workspace);
-    HICGAT_REQUIRE(workspace_bytes >= w.bytes, "hicgat_dscc_target_ranks: workspace of %zu bytes, %zu needed", workspace_bytes, w.bytes);
-    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-    const int rc = dscc_ranks(true, nullptr, target, pitch, n, t_scale, nbins, rank_t, w, stream);
+    DSCC_WORKSPACE("hicgat_dscc_target_ranks");
+    const int rc = hicgat_dscc_target_hist_rows(target, pitch, n, 0, n, t_scale, nbins, reinterpret_cast<uint64_t*>(w.hist), stream);
     if (rc != HICGAT_OK) return rc;
-    dscc_sum_kernel<<<1, kFinishThreads, 0, stream>>>(w.scan_partials, w.nscan, var_t);
-    HICGAT_CHECK_LAUNCH("dscc_sum_kernel");
-    return HICGAT_OK;
+    return hicgat_dscc_hist_ranks(reinterpret_cast<const uint64_t*>(w.hist), n, nbins, rank_t, var_t, workspace, workspace_bytes, stream);
 }
 
 extern "C" int hicgat_dscc_dense(const float* coords, const float* target, int64_t pitch, int64_t n, float t_scale, int nbins, const double* rank_t,
                                  const double* var_t, double* rho, void* workspace, size_t workspace_bytes, hicgat_stream_t stream_) {
     HICGAT_REQUIRE(dscc_sizes_ok(n, nbins), "hicgat_dscc_dense: bad n/nbins (need 0 < n <= %lld, nbins > 0)", (long long)kDsccMaxN);
     HICGAT_REQUIRE(coords && target && rank_t && var_t && rho && workspace && pitch >= n, "hicgat_dscc_dense: null pointer / bad pitch");
-    const DsccWorkspace w = dscc_layout(n, nbins, workspace);
-    HICGAT_REQUIRE(workspace_bytes >= w.bytes, "hicgat_dscc_dense: workspace of %zu bytes, %zu needed", workspace_bytes, w.bytes);
-    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-    int rc = dscc_distance_side(coords, n, nbins, w, stream);
-    if (rc != HICGAT_OK) return rc;
-    const dim3 grid((unsigned)((n + kThreadsM - 1) / kThreadsM), (unsigned)((n + kRows - 1) / kRows));
-    dscc_cross_dense_kernel<<<grid, kThreadsM, 0, stream>>>(coords, target, pitch, (int)n, w.d_scale, t_scale, nbins, w.rank_d, rank_t, w.cross_partials);
-    HICGAT_CHECK_LAUNCH("dscc_cross_dense_kernel");
-    const int64_t ncross = (int64_t)grid.x * grid.y;
-    dscc_finish_kernel<<<1, kFinishThreads, 0, stream>>>(w.scan_partials, w.nscan, w.cross_partials, ncross, 0, var_t, nullptr, (double)n * (double)(n - 1) / 2.0, rho);
-    HICGAT_CHECK_LAUNCH("dscc_finish_kernel");
-    return HICGAT_OK;
+    DSCC_WORKSPACE("hicgat_dscc_dense");
+    uint64_t* hist = reinterpret_cast<uint64_t*>(w.hist);
+    int rc = hicgat_dscc_dist_hist_rows(coords, n, 0, n, nbins, hist, workspace, workspace_bytes, stream);
+    if (rc == HICGAT_OK) rc = hicgat_dscc_cross_dense_rows(coords, target, pitch, n, 0, n, t_scale, nbins, hist, rank_t, w.cross_sum, workspace, workspace_bytes, stream);
+    if (rc == HICGAT_OK) rc = hicgat_dscc_finish(w.cross_sum, n, nbins, 0, nullptr, var_t, rho, workspace, workspace_bytes, stream);
+    return rc;
 }
 
 extern "C" int hicgat_dscc_implicit(const float* coords, const int32_t* rowptr, const int32_t* col, const double* rank_t_csr, int64_t n,
@@ -552,15 +639,10 @@ extern "C" int hicgat_dscc_implicit(const float* coords, const int32_t* rowptr, 
                                     hicgat_stream_t stream_) {
     HICGAT_REQUIRE(dscc_sizes_ok(n, nbins), "hicgat_dscc_implicit: bad n/nbins (need 0 < n <= %lld, nbins > 0)", (long long)kDsccMaxN);
     HICGAT_REQUIRE(coords && rowptr && col && rank_t_csr && rank_fill && var_t && rho && workspace, "hicgat_dscc_implicit: null pointer");
-    const DsccWorkspace w = dscc_layout(n, nbins, workspace);
-    HICGAT_REQUIRE(workspace_bytes >= w.bytes, "hicgat_dscc_implicit: workspace of %zu bytes, %zu needed", workspace_bytes, w.bytes);
-    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-    int rc = dscc_distance_side(coords, n, nbins, w, stream);
-    if (rc != HICGAT_OK) return rc;
-    const int blocks = (int)((n + kCsrRowsPerBlock - 1) / kCsrRowsPerBlock);
-    dscc_cross_csr_kernel<<<blocks, kCsrRowsPerBlock * 32, 0, stream>>>(coords, rowptr, col, rank_t_csr, (int)n, w.d_scale, nbins, w.rank_d, w.cross_partials);
-    HICGAT_CHECK_LAUNCH("dscc_cross_csr_kernel");
-    dscc_finish_kernel<<<1, kFinishThreads, 0, stream>>>(w.scan_partials, w.nscan, w.cross_partials, blocks, 1, var_t, rank_fill, (double)n * (double)(n - 1) / 2.0, rho);
-    HICGAT_CHECK_LAUNCH("dscc_finish_kernel");
-    return HICGAT_OK;
+    DSCC_WORKSPACE("hicgat_dscc_implicit");
+    uint64_t* hist = reinterpret_cast<uint64_t*>(w.hist);
+    int rc = hicgat_dscc_dist_hist_rows(coords, n, 0, n, nbins, hist, workspace, workspace_bytes, stream);
+    if (rc == HICGAT_OK) rc = hicgat_dscc_cross_implicit_rows(coords, rowptr, col, rank_t_csr, n, 0, n, nbins, hist, w.cross_sum, workspace, workspace_bytes, stream);
+    if (rc == HICGAT_OK) rc = hicgat_dscc_finish(w.cross_sum, n, nbins, 1, rank_fill, var_t, rho, workspace, workspace_bytes, stream);
+    return rc;
 }

@@ -7,7 +7,8 @@ AVERAGE ranks for ties -- every zero-contact pair has wish distance exactly 1.0,
 rule, not the exception.  The distances come from the library's pair-distance kernel; the rank
 transform is sort-based torch glue (evaluation runs once per model, not per step).
 :class:`DsccMeter` is the per-step form (the reference also evaluates ``spearmanr`` every iteration,
-HiC_GAT_generalize_directly.py:242): histogram mid-ranks entirely on the device, graph-capturable.
+HiC_GAT_generalize_directly.py:242): histogram mid-ranks entirely on the device, graph-capturable; :class:`ShardedDsccMeter` is the
+same for a target row-sharded over the GPUs of one box.
 """
 from __future__ import annotations
 
@@ -147,6 +148,29 @@ def dscc_streamed(coords: torch.Tensor, target, nbins: int = NBINS, reduce=None)
     return _spearman_from_tables(hist_d, hist_t, cross, npairs)
 
 
+def _t_scale(tmax: float, nbins: int) -> float:
+    """Bin scale of a dense target whose largest value is ``tmax``: the rule of :func:`dscc_streamed`."""
+    return nbins / (max(tmax, 1e-30) * (1.0 + 1e-6))
+
+
+def _implicit_rank_table(target):
+    """Target side of the per-step dSCC of an implicit target (all of its CSR): (rank of the stored value of every entry (i, j) with
+    j > i -- 0 elsewhere --, rank of the fill group, var_t), the last two as 0-d device tensors."""
+    n, dev = target.n, target.tval.device
+    row = torch.repeat_interleave(torch.arange(n, device=dev), target.rowptr[1:].long() - target.rowptr[:-1].long())
+    up = target.col.long() > row
+    rt, r_fill, var_t = _implicit_target_ranks(target.tval[up].double(), target.fill, n * (n - 1) / 2.0)
+    rank_t = torch.zeros(max(target.col.numel(), 1), dtype=torch.float64, device=dev)
+    rank_t[: target.col.numel()][up] = rt
+    return rank_t, r_fill.reshape(()).clone(), var_t.reshape(()).clone()
+
+
+def _check_coords(coords: torch.Tensor, n: int) -> None:
+    ops._cuda(coords)
+    if coords.dtype != torch.float32 or coords.dim() != 2 or tuple(coords.shape) != (n, 3) or not coords.is_contiguous():
+        raise RuntimeError(f"coords must be contiguous float32 [n,3] with n={n}, got {coords.dtype} {tuple(coords.shape)}")
+
+
 class DsccMeter:
     """dSCC of a full target at every training step (``spearmanr`` per iteration, HiC_GAT_generalize_directly.py:242), on the device.
 
@@ -175,29 +199,21 @@ class DsccMeter:
             raise ValueError(f"DsccMeter: unsupported size n={n}, nbins={nbins}")
         self._ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         self.rho = torch.full((), float("nan"), dtype=torch.float64, device=dev)
-        npairs = n * (n - 1) / 2.0
         if isinstance(target, ops.WishTarget):
             tmax = float(target.data.max()) if target.data.numel() else 1.0
-            self._t_scale = nbins / (max(tmax, 1e-30) * (1.0 + 1e-6))          # the rule of dscc_streamed
+            self._t_scale = _t_scale(tmax, nbins)
             self._rank_t = torch.empty(nbins, dtype=torch.float64, device=dev)
             self._var_t = torch.empty((), dtype=torch.float64, device=dev)
             N.check(lib.hicgat_dscc_target_ranks(target.data.data_ptr(), target.pitch, n, self._t_scale, nbins, self._rank_t.data_ptr(),
                                                  self._var_t.data_ptr(), self._ws.data_ptr(), ws_bytes, ops._stream()), "hicgat_dscc_target_ranks")
         else:
-            row = torch.repeat_interleave(torch.arange(n, device=dev), target.rowptr[1:].long() - target.rowptr[:-1].long())
-            up = target.col.long() > row
-            rt, r_fill, var_t = _implicit_target_ranks(target.tval[up].double(), target.fill, npairs)
-            self._rank_t = torch.zeros(max(target.col.numel(), 1), dtype=torch.float64, device=dev)
-            self._rank_t[: target.col.numel()][up] = rt
-            self._rank_fill, self._var_t = r_fill.reshape(()).clone(), var_t.reshape(()).clone()
+            self._rank_t, self._rank_fill, self._var_t = _implicit_rank_table(target)
         self._ws_bytes = ws_bytes
 
     def __call__(self, coords: torch.Tensor) -> torch.Tensor:
         from . import _native as N
 
-        ops._cuda(coords)
-        if coords.dtype != torch.float32 or coords.dim() != 2 or tuple(coords.shape) != (self.n, 3) or not coords.is_contiguous():
-            raise RuntimeError(f"coords must be contiguous float32 [n,3] with n={self.n}, got {coords.dtype} {tuple(coords.shape)}")
+        _check_coords(coords, self.n)
         lib, t = N.lib(), self.target
         if isinstance(t, ops.WishTarget):
             rc = lib.hicgat_dscc_dense(coords.data_ptr(), t.data.data_ptr(), t.pitch, self.n, self._t_scale, self.nbins, self._rank_t.data_ptr(),
@@ -208,6 +224,92 @@ class DsccMeter:
                                           self._rank_fill.data_ptr(), self._var_t.data_ptr(), self.nbins, self.rho.data_ptr(), self._ws.data_ptr(),
                                           self._ws_bytes, ops._stream())
             N.check(rc, "hicgat_dscc_implicit")
+        return self.rho
+
+
+class ShardedDsccMeter:
+    """:class:`DsccMeter` of a target row-sharded over the ranks of a process group: ``target`` is this rank's row block ``[r0, r1)``
+    of a dense :class:`ops.WishTarget` or of an implicit :class:`ops.SparseWishTarget` (which holds the whole CSR on every rank).
+
+    The target side runs once, here: dense -- ``t_scale`` from the all-reduced max of every block (so it equals the full meter's), the
+    block's target histogram summed over the ranks, its mid-ranks and ``var_t``; implicit -- the rank table of :class:`DsccMeter`, with
+    no communication.  Every buffer is allocated here.  ``meter(coords)`` takes the full ``[n, 3]`` coordinates (identical on every
+    rank) and runs: the block's distance histogram -> sum over the ranks -> the block's cross sum -> sum over the ranks, in rank order
+    -> rho (``hicgat_dscc_*_rows``, ``hicgat_dscc_finish``).  It returns the same 0-d f64 CUDA tensor every call, with no host read and
+    no allocation; rho is bit-identical on every rank, and within 1e-12 of :class:`DsccMeter` (only the grouping of the cross sum
+    differs; the summed histograms are the full ones bit for bit).  Every rank must call it, as for any collective.
+
+    ``transport``: the exchange of :class:`sharding.DsccExchange` (``"p2p"`` / ``"nccl"`` / ``"auto"``); ``capturable`` says whether a
+    call can be captured in a CUDA graph (the p2p exchange, or a single rank).  The p2p exchange holds two symmetric buffers of
+    8 ``nbins`` bytes per rank.  Without a multi-rank process group the target must be the full one, and the meter equals
+    :class:`DsccMeter` bit for bit."""
+
+    def __init__(self, target, group=None, transport: str = "auto", nbins: int = NBINS):
+        import torch.distributed as dist
+
+        from . import _native as N
+        from . import sharding
+
+        if not isinstance(target, (ops.WishTarget, ops.SparseWishTarget)):
+            raise TypeError("ShardedDsccMeter expects a WishTarget or a SparseWishTarget row block")
+        nbins = int(nbins)
+        if nbins <= 0:
+            raise ValueError(f"nbins must be positive, got {nbins}")
+        if transport not in ("auto", "p2p", "nccl"):
+            raise ValueError(f"ShardedDsccMeter: transport must be 'auto', 'p2p' or 'nccl', got {transport!r}")
+        multi = dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
+        if not multi and (target.r0 != 0 or target.r1 != target.n):
+            raise ValueError(f"ShardedDsccMeter: rows [{target.r0}, {target.r1}) of {target.n} without a multi-rank process group; "
+                             "one rank needs the full target")
+        self.target, self.n, self.nbins = target, target.n, nbins
+        self.r0, self.r1 = target.r0, target.r1
+        lib, n = N.lib(), target.n
+        dense = isinstance(target, ops.WishTarget)
+        dev = target.data.device if dense else target.tval.device
+        ws_bytes = lib.hicgat_dscc_workspace_bytes(n, nbins)
+        if ws_bytes == 0:
+            raise ValueError(f"ShardedDsccMeter: unsupported size n={n}, nbins={nbins}")
+        self._ws, self._ws_bytes = torch.empty(ws_bytes, dtype=torch.uint8, device=dev), ws_bytes
+        self.rho = torch.full((), float("nan"), dtype=torch.float64, device=dev)
+        self._x = sharding.DsccExchange(nbins, dev, group, transport)
+        self.transport, self.capturable = self._x.transport, self._x.capturable
+        if dense:
+            tmax = target.data.max().reshape(1).double() if target.data.numel() else torch.full((1,), -float("inf"), dtype=torch.float64, device=dev)
+            tmax = float(sharding.allreduce_max_(tmax, group))
+            self._t_scale = _t_scale(tmax if tmax != -float("inf") else 1.0, nbins)
+            self._rank_t = torch.empty(nbins, dtype=torch.float64, device=dev)
+            self._var_t = torch.empty((), dtype=torch.float64, device=dev)
+            st = ops._stream()
+            N.check(lib.hicgat_dscc_target_hist_rows(target.data.data_ptr(), target.pitch, n, self.r0, self.r1, self._t_scale, nbins,
+                                                     self._x.hist.data_ptr(), st), "hicgat_dscc_target_hist_rows")
+            hist_t = self._x.sum_hist()
+            N.check(lib.hicgat_dscc_hist_ranks(hist_t.data_ptr(), n, nbins, self._rank_t.data_ptr(), self._var_t.data_ptr(), self._ws.data_ptr(),
+                                               ws_bytes, ops._stream()), "hicgat_dscc_hist_ranks")
+            self._rank_fill = None
+        else:
+            self._rank_t, self._rank_fill, self._var_t = _implicit_rank_table(target)
+
+    def __call__(self, coords: torch.Tensor) -> torch.Tensor:
+        from . import _native as N
+
+        _check_coords(coords, self.n)
+        lib, t, x, st = N.lib(), self.target, self._x, ops._stream()
+        ws, wb = self._ws.data_ptr(), self._ws_bytes
+        N.check(lib.hicgat_dscc_dist_hist_rows(coords.data_ptr(), self.n, self.r0, self.r1, self.nbins, x.hist.data_ptr(), ws, wb, st),
+                "hicgat_dscc_dist_hist_rows")
+        hist_d = x.sum_hist()
+        if isinstance(t, ops.WishTarget):
+            N.check(lib.hicgat_dscc_cross_dense_rows(coords.data_ptr(), t.data.data_ptr(), t.pitch, self.n, self.r0, self.r1, self._t_scale,
+                                                     self.nbins, hist_d.data_ptr(), self._rank_t.data_ptr(), x.cross.data_ptr(), ws, wb, st),
+                    "hicgat_dscc_cross_dense_rows")
+        else:
+            N.check(lib.hicgat_dscc_cross_implicit_rows(coords.data_ptr(), t.rowptr.data_ptr(), ops._addr(t.col), self._rank_t.data_ptr(), self.n,
+                                                        self.r0, self.r1, self.nbins, hist_d.data_ptr(), x.cross.data_ptr(), ws, wb, st),
+                    "hicgat_dscc_cross_implicit_rows")
+        cross = x.sum_cross()
+        implicit = self._rank_fill is not None
+        N.check(lib.hicgat_dscc_finish(cross.data_ptr(), self.n, self.nbins, int(implicit), self._rank_fill.data_ptr() if implicit else None,
+                                       self._var_t.data_ptr(), self.rho.data_ptr(), ws, wb, st), "hicgat_dscc_finish")
         return self.rho
 
 

@@ -531,3 +531,105 @@ class GnnRowShard:
             if p.grad is None:
                 p.grad = torch.zeros_like(p)
         self._x.reduce([p.grad for p in params])
+
+
+# ------------------------------------------------------------------------------ row-sharded per-step dSCC
+class DsccExchange:
+    """The two exchanges of a row-sharded dSCC evaluation (:class:`metrics.ShardedDsccMeter`):
+
+    * :meth:`sum_hist`: ``hist_sum = sum over the ranks of hist`` (u64[nbins] distance or target histograms; integer counts, so exact
+      and independent of the order);
+    * :meth:`sum_cross`: ``cross_sum = sum over the ranks of cross`` (f64[2] block cross sums), added in rank order starting from 0.0,
+      so the result is bit-identical on every rank and between the transports.
+
+    The local buffers ``hist`` / ``cross`` are where this rank's block phases write; ``hist_sum`` / ``cross_sum`` hold the results.
+    ``transport``: ``"p2p"`` (``hicgat_allreduce_u64_twoshot`` for the histogram; the two-shot partials kernel for the cross sums, which
+    ride in its moment slot with a zero gradient part; both capturable), ``"nccl"`` (an int64 ``all_reduce`` of the histogram, and
+    ``allreduce_packed`` of a ``[world, 2]`` buffer that is zero outside this rank's row, summed over the rows in rank order; with gloo
+    on CPU tensors too; eager only) or ``"auto"`` (the rule of :class:`GnnRowShard`).  Without a multi-rank process group both steps
+    are no-ops and the sums are the local buffers."""
+
+    SLOTS_HIST = P2PShardedPairLoss.SLOT_BASE + 192   # the loss exchanges use SLOT_BASE + 0 .. + 127, the GNN exchanges + 128 .. + 191
+    SLOTS_CROSS = P2PShardedPairLoss.SLOT_BASE + 224
+
+    def __init__(self, nbins: int, device, group=None, transport: str = "auto"):
+        if transport not in ("auto", "p2p", "nccl"):
+            raise ValueError(f"DsccExchange: transport must be 'auto', 'p2p' or 'nccl', got {transport!r}")
+        self.nbins, self.group = int(nbins), group
+        multi = dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
+        self.world = dist.get_world_size(group) if multi else 1
+        self.rank = dist.get_rank(group) if multi else 0
+        self._p2p = False
+        if transport == "p2p" or (transport == "auto" and multi and torch.device(device).type == "cuda"):
+            try:
+                self._init_p2p(device, group)
+                self._p2p = True
+            except Exception as e:  # no symmetric memory on this system: the collective exchange is equivalent
+                if transport == "p2p":
+                    raise
+                import warnings
+
+                warnings.warn(f"symmetric-memory exchange unavailable ({e!r}); using the NCCL all-reduce")
+        if not self._p2p:
+            self.hist = torch.zeros(self.nbins, dtype=torch.int64, device=device)
+            self.cross = torch.zeros(2, dtype=torch.float64, device=device)
+            self.hist_sum, self.cross_sum = self.hist, (self.cross if not multi else torch.zeros(2, dtype=torch.float64, device=device))
+            self._rows = torch.zeros(self.world, 2, dtype=torch.float64, device=device) if multi else None
+        self.multi = multi
+        self.transport = "p2p" if self._p2p else "nccl"
+        self.capturable = self._p2p or not multi
+
+    def _init_p2p(self, device, group):
+        import ctypes as C
+
+        import torch.distributed._symmetric_memory as symm
+
+        group = group if group is not None else dist.group.WORLD
+        hbytes = (8 * self.nbins + 15) // 16 * 16
+        # layout: [hist: hbytes | hist_sum: hbytes | cross partial: 64 moments + 16 zero gradient | cross result: 16]
+        h_part, h_res, c_part = 0, hbytes, 2 * hbytes
+        c_res = c_part + 80
+        self.buf = symm.empty(c_res + 16, dtype=torch.uint8, device=device)
+        self.buf.zero_()
+        self.hdl = symm.rendezvous(self.buf, group)
+        self.world, self.rank = self.hdl.world_size, self.hdl.rank
+        if self.hdl.signal_pad_size < 4 * (self.SLOTS_CROSS + 32):
+            raise RuntimeError("symmetric-memory signal pad too small")
+        ptrs = [int(p) for p in self.hdl.buffer_ptrs]
+        table = lambda off: (C.c_uint64 * self.world)(*[p + off for p in ptrs])
+        self._h_part, self._h_res = table(h_part), table(h_res)
+        self._c_part, self._c_res = table(c_part), table(c_res)
+        self._pads = (C.c_uint64 * self.world)(*[int(p) for p in self.hdl.signal_pad_ptrs])
+        self.hist = self.buf[h_part: h_part + 8 * self.nbins].view(torch.int64)
+        self.hist_sum = self.buf[h_res: h_res + 8 * self.nbins].view(torch.int64)
+        self.cross = self.buf[c_part: c_part + 16].view(torch.float64)    # moments 0, 1 of the partial; moments 2..7 stay zero
+        self._moments = torch.zeros(N.PAIR_NMOM, dtype=torch.float64, device=device)
+        self.cross_sum = self._moments[:2]
+        self.state_h = torch.zeros(4, dtype=torch.int32, device=device)
+        self.state_c = torch.zeros(4, dtype=torch.int32, device=device)
+        torch.cuda.synchronize(device)
+        dist.barrier(group)  # every rank's buffer is zeroed and mapped before the first signal
+
+    def sum_hist(self) -> torch.Tensor:
+        if self._p2p:
+            N.check(N.lib().hicgat_allreduce_u64_twoshot(self._h_part, self._h_res, self._pads, self.rank, self.world, self.nbins, self.SLOTS_HIST,
+                                                         self.state_h.data_ptr(), torch.cuda.current_stream().cuda_stream),
+                    "hicgat_allreduce_u64_twoshot")
+        elif self.multi:
+            dist.all_reduce(self.hist, op=dist.ReduceOp.SUM, group=self.group)
+        return self.hist_sum
+
+    def sum_cross(self) -> torch.Tensor:
+        if self._p2p:
+            N.check(N.lib().hicgat_allreduce_partials_twoshot(self._c_part, self._c_res, self._pads, self.rank, self.world, 1, self.SLOTS_CROSS,
+                                                              self.state_c.data_ptr(), None, self._moments.data_ptr(),
+                                                              torch.cuda.current_stream().cuda_stream),
+                    "hicgat_allreduce_partials_twoshot")
+        elif self.multi:
+            self._rows.zero_()
+            self._rows[self.rank] = self.cross
+            allreduce_packed(self._rows, self.group)   # x + 0 + ... + 0 = x: each row arrives exactly
+            self.cross_sum.zero_()
+            for r in range(self.world):                # rank order, from 0.0: the sum of the p2p kernel
+                self.cross_sum += self._rows[r]
+        return self.cross_sum

@@ -16,7 +16,8 @@ loss+gradient launch over the f32 target, backward through the conv kernels, Ada
   ``"contrastive"``  total = 0.1 mean_{i<j} |t - d|                    (train_and_test_same_res_GAT_node2vec.py:131-134)
   ``"mse_spearman"`` total = MSE + alpha (1 - dSCC), fixed alpha       (combined_loss_training.py:119-142; the Spearman
                      term is a scipy value in the reference, i.e. a constant for autograd: the gradient is MSE's.  The
-                     rank transform runs on the GPU (metrics.dscc) but costs a host read per step: no CUDA graph)
+                     rank transform runs on the GPU (metrics.dscc) but costs a host read per step: no CUDA graph.  With a
+                     sharded ``reducer`` the dSCC comes from a ``dscc_meter`` (metrics.ShardedDsccMeter), identical on every rank)
 """
 from __future__ import annotations
 
@@ -39,13 +40,18 @@ def step_loss(model, x, graph, target: WishTarget, mode: str, reducer=None, alph
     return _loss_of_coords(model.get_model(x, graph), target, mode, reducer, alpha)
 
 
-def _loss_of_coords(coords, target, mode: str, reducer, alpha: float):
+def _loss_of_coords(coords, target, mode: str, reducer, alpha: float, rho=None):
+    """``rho``: the dSCC of ``coords`` from a meter (0-d tensor), for ``mse_spearman``; needed with a sharded ``reducer``, whose ``target``
+    is a row block: a block-local rank correlation would differ from rank to rank, and so would the totals the stop rule compares."""
+    if mode == "mse_spearman" and rho is None and reducer is not None:
+        raise ValueError("mse_spearman with a sharded reducer needs dscc_meter= (metrics.ShardedDsccMeter): "
+                         "the dSCC of a row block differs from rank to rank")
     loss, moments = pairwise_loss(coords, target, _KERNEL_MODE[mode], reducer)
     total = loss.detach()  # mse_pearson_grad: the f64 total from the same moments as the gradient
     if mode == "mse_spearman":
         from . import metrics
 
-        rho = metrics.dscc(coords.detach(), target)          # spearmanr of the i<j distances (:137)
+        rho = metrics.dscc(coords.detach(), target) if rho is None else float(rho)   # spearmanr of the i<j distances (:137)
         if rho != rho:                                        # NaN -> 0 (:138-140)
             rho = 0.0
         total = total.double() + alpha * (1.0 - rho)
@@ -67,17 +73,31 @@ class TrainStep:
     the device and inside the graph.  The value is ``step.dscc`` (0-d f64, overwritten by the next step).  Needs the full target:
     refused with a sharded ``reducer``.
 
+    ``dscc_meter``: a caller-built :class:`metrics.DsccMeter` or :class:`metrics.ShardedDsccMeter` in place of ``track_dscc``; it is
+    evaluated on the same (gathered, pre-update) coordinates every step into ``step.dscc``, inside the graph when the step is graphed
+    (which needs ``dscc_meter.capturable``).  With a sharded ``reducer`` it is what gives per-step dSCC, and ``mode="mse_spearman"``
+    takes its rho from it (without a meter that combination is refused; without a reducer ``mse_spearman`` keeps ``metrics.dscc``).
+
     ``gnn_shard`` (:class:`sharding.GnnRowShard`): the GNN runs on this rank's target rows only.  A step is: forward on the
     row-block view of ``graph`` -> ``gnn_shard.gather_coords`` (all N coordinates) -> the fused loss (sharded with ``reducer`` or
     not) -> backward -> ``gnn_shard.reduce_grads`` -> Adam; every rank ends the step with identical parameters.  With
     ``use_cuda_graph`` the exchange must be capturable (the p2p transport)."""
 
     def __init__(self, model, x, graph, target: WishTarget, mode: str = "mse", lr: float = 1e-3, use_cuda_graph: bool = False, reducer=None,
-                 alpha: float = 1.0, track_dscc: bool = False, gnn_shard=None):
+                 alpha: float = 1.0, track_dscc: bool = False, gnn_shard=None, dscc_meter=None):
         if mode not in _KERNEL_MODE:
             raise ValueError(mode)
+        if track_dscc and dscc_meter is not None:
+            raise ValueError("track_dscc and dscc_meter both ask for a per-step dSCC: pass one of them")
         if track_dscc and reducer is not None:
-            raise ValueError("track_dscc needs the full target on one GPU: per-step dSCC of a row-sharded target is not supported")
+            raise ValueError("track_dscc needs the full target on one GPU: for a row-sharded target pass "
+                             "dscc_meter=metrics.ShardedDsccMeter(target) instead")
+        if mode == "mse_spearman" and reducer is not None and dscc_meter is None:
+            raise ValueError("mse_spearman with a sharded reducer needs dscc_meter= (metrics.ShardedDsccMeter): "
+                             "the dSCC of a row block differs from rank to rank")
+        if use_cuda_graph and dscc_meter is not None and not getattr(dscc_meter, "capturable", True):
+            raise ValueError("use_cuda_graph needs a capturable dSCC meter (the two-shot p2p exchange); "
+                             f"the {getattr(dscc_meter, 'transport', '?')!r} exchange of {type(dscc_meter).__name__} is eager only")
         if mode == "mse_spearman" and use_cuda_graph:
             raise ValueError("mse_spearman reads the rank correlation back every step: it cannot be captured in a CUDA graph")
         if use_cuda_graph and reducer is not None and not getattr(reducer, "capturable", False):
@@ -99,7 +119,7 @@ class TrainStep:
         self.total = None
         self.moments = None
         self.dscc = None
-        self._meter = None
+        self._meter = dscc_meter
         if track_dscc:
             from .metrics import DsccMeter
 
@@ -115,7 +135,8 @@ class TrainStep:
             coords = self.gnn_shard.gather_coords(coords)
         if self._meter is not None:
             self.dscc = self._meter(coords.detach().contiguous())
-        loss, total, moments = _loss_of_coords(coords, self.target, self.mode, self.reducer, self.alpha)
+        rho = self.dscc if self.reducer is not None and self.mode == "mse_spearman" else None  # one GPU: metrics.dscc, exact up to 4 096 loci
+        loss, total, moments = _loss_of_coords(coords, self.target, self.mode, self.reducer, self.alpha, rho)
         loss.backward()
         if self.gnn_shard is not None:
             self.gnn_shard.reduce_grads(self.model.parameters())
@@ -154,7 +175,8 @@ class TrainStep:
 
 
 def fit(model, x, graph, target: WishTarget, mode: str = "mse", lr: float = 1e-3, thresh: float = 1e-8, max_steps: int | None = None,
-        check_every: int = 1, use_cuda_graph: bool = False, reducer=None, alpha: float = 1.0, dscc_out: list | None = None, gnn_shard=None):
+        check_every: int = 1, use_cuda_graph: bool = False, reducer=None, alpha: float = 1.0, dscc_out: list | None = None, gnn_shard=None,
+        dscc_meter=None):
     """Reference loop.  Returns the list of per-step total losses (floats).
 
     ``check_every=1`` evaluates the stop rule every step exactly like the reference (one host
@@ -164,9 +186,13 @@ def fit(model, x, graph, target: WishTarget, mode: str = "mse", lr: float = 1e-3
     ``dscc_out``: a list to which the dSCC of every step's (pre-update) structure is appended, like the reference's ``SpRho``
     history (``TrainStep(track_dscc=True)``); read back in the same batched reads as the losses.
 
-    ``gnn_shard``: row-sharded GNN (:class:`TrainStep`)."""
+    ``gnn_shard``: row-sharded GNN (:class:`TrainStep`).
+
+    ``dscc_meter``: the meter that fills ``dscc_out`` (and gives ``mse_spearman`` its rho) instead of a :class:`metrics.DsccMeter` built
+    here; with a sharded ``reducer`` a :class:`metrics.ShardedDsccMeter` of the same row block (:class:`TrainStep`)."""
     track = dscc_out is not None
-    step = TrainStep(model, x, graph, target, mode, lr, use_cuda_graph, reducer, alpha, track_dscc=track, gnn_shard=gnn_shard)
+    step = TrainStep(model, x, graph, target, mode, lr, use_cuda_graph, reducer, alpha, track_dscc=track and dscc_meter is None, gnn_shard=gnn_shard,
+                     dscc_meter=dscc_meter)
     hist: list[float] = []
     pending: list[torch.Tensor] = []
     pending_dscc: list[torch.Tensor] = []

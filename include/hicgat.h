@@ -246,6 +246,14 @@ HICGAT_API int hicgat_allreduce_partials_twoshot(const uint64_t* peer_partials_h
                                       uint32_t* state, const double* moment_const, double* out_moments,
                                       hicgat_stream_t stream);
 
+/* Two-shot all-reduce of a u64 array (count elements; integer sums, exact and order-free) over NVLink peer memory, with the
+ * barrier, state and epoch protocol of hicgat_allreduce_partials_twoshot: rank r's source array at peer_src_host[r], its result
+ * at peer_dst_host[r] (both symmetric, 16-byte aligned), `state` uint32[4] local and zero-initialised once, signal slots
+ * slot_base .. slot_base + 31 of every pad.  Rank r sums slice r and stores it into every rank's result.  Capturable in a CUDA
+ * graph; programmatic stream serialization.  Sums the per-rank dSCC distance histograms (hicgat_dscc_dist_hist_rows). */
+HICGAT_API int hicgat_allreduce_u64_twoshot(const uint64_t* peer_src_host, const uint64_t* peer_dst_host, const uint64_t* signal_pads_host,
+                                 int rank, int world, int64_t count, int slot_base, uint32_t* state, hicgat_stream_t stream);
+
 /* ------------------------------------------------------------------------------------
  * (next row f-3) dSCC at scale: Spearman correlation of the i<j wish distances and reconstructed distances
  * (scipy.stats.spearmanr on triu_indices gathers: HiC-GNN_main.py:135-139, HiC_GAT_generalize_directly.py:210-242) without the
@@ -298,6 +306,39 @@ HICGAT_API int hicgat_dscc_dense(const float* coords, const float* target, int64
 HICGAT_API int hicgat_dscc_implicit(const float* coords, const int32_t* rowptr, const int32_t* col, const double* rank_t_csr, int64_t n,
                          const double* rank_fill, const double* var_t, int nbins, double* rho, void* workspace,
                          size_t workspace_bytes, hicgat_stream_t stream);
+
+/* The same evaluation in phases over target rows [r0, r1) (0 <= r0 <= r1 <= n), for a target row-sharded over the ranks of a process
+ * group: each rank runs the block phases on its rows, and the caller sums the distance histogram and the cross sums over the ranks
+ * between them.  hicgat_dscc_target_ranks / _dense / _implicit are these phases over (0, n), with the workspace's own hist and cross
+ * buffers; their results are bit-identical to the phases called over (0, n).  One workspace (hicgat_dscc_workspace_bytes of the FULL n)
+ * carries d_scale, rank_d and the scan partials from phase to phase: use one per evaluation, in this order, on one stream.
+ *   hicgat_dscc_dist_hist_rows      d_scale from ALL n coordinates (the same bins on every rank) into the workspace, then hist_d (u64[nbins],
+ *                                   caller-owned, zeroed first) = the histogram of d_ij over the pairs i < j with i in [r0, r1)
+ *   hicgat_dscc_target_hist_rows    once per dense target: hist_t (u64[nbins], zeroed first) of t_ij over the same pairs; `target` points at
+ *                                   the block's first row, row i is read at target + (i - r0) pitch (pitch >= n)
+ *   hicgat_dscc_hist_ranks          once per dense target: rank f64[nbins] and var (f64 scalar) of the rank-summed hist_t
+ *   hicgat_dscc_cross_dense_rows    rank_d and its scan partials of the rank-summed hist_d into the workspace, then the block cross sum
+ *                                   cross f64[2] = [sum rank_d rank_t over the block's pairs, 0]
+ *   hicgat_dscc_cross_implicit_rows the same for an implicit target (rank_t_csr as for hicgat_dscc_implicit):
+ *                                   cross = [sum rank_t_csr rank_d, sum rank_d] over the block's stored entries (i, j) with j > i
+ *   hicgat_dscc_finish              rho from the rank-summed cross f64[2] and the workspace's var_d and sum h rank_d (implicit != 0:
+ *                                   rank_fill is read, cross as in hicgat_dscc_implicit); NaN under the same conditions
+ * The block cross sum reduces the block's per-tile partials in the fixed order of one block; summed over the ranks in rank order, rho is
+ * bit-identical on every rank.  The histograms are integer counts: their rank sum equals the (0, n) histogram bit for bit. */
+HICGAT_API int hicgat_dscc_dist_hist_rows(const float* coords, int64_t n, int64_t r0, int64_t r1, int nbins, uint64_t* hist_d,
+                               void* workspace, size_t workspace_bytes, hicgat_stream_t stream);
+HICGAT_API int hicgat_dscc_target_hist_rows(const float* target, int64_t pitch, int64_t n, int64_t r0, int64_t r1, float t_scale,
+                                 int nbins, uint64_t* hist_t, hicgat_stream_t stream);
+HICGAT_API int hicgat_dscc_hist_ranks(const uint64_t* hist, int64_t n, int nbins, double* rank, double* var, void* workspace,
+                           size_t workspace_bytes, hicgat_stream_t stream);
+HICGAT_API int hicgat_dscc_cross_dense_rows(const float* coords, const float* target, int64_t pitch, int64_t n, int64_t r0, int64_t r1,
+                                 float t_scale, int nbins, const uint64_t* hist_d, const double* rank_t, double* cross,
+                                 void* workspace, size_t workspace_bytes, hicgat_stream_t stream);
+HICGAT_API int hicgat_dscc_cross_implicit_rows(const float* coords, const int32_t* rowptr, const int32_t* col, const double* rank_t_csr,
+                                    int64_t n, int64_t r0, int64_t r1, int nbins, const uint64_t* hist_d, double* cross,
+                                    void* workspace, size_t workspace_bytes, hicgat_stream_t stream);
+HICGAT_API int hicgat_dscc_finish(const double* cross, int64_t n, int nbins, int implicit, const double* rank_fill, const double* var_t,
+                       double* rho, void* workspace, size_t workspace_bytes, hicgat_stream_t stream);
 
 /* Materialising variant kept for API parity of model.forward() (returns the N x N matrix,
  * models.py:39): dist[i,j] = |x_i - x_j|, and its backward
